@@ -2,7 +2,7 @@
 """bench.py -- HPGMG-FV fv4 FMG DOF/s on B200 (BASELINE.json metric) + roofline + CPU baseline.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log2-box-dim 7] [--boxes-per-rank 8]
-                  [--smoother gsrb|cheby] [--scaling weak|strong --global-dim 512]
+                  [--smoother gsrb|cheby] [--scaling weak|strong --global-dim 512] [--dump-outputs DIR]
 
 A step is what the reference's bench_hpgmg times (hpgmg-fv.c:78-80): zero_vector(U); FMGSolve(...)
 on the finest level.  Workload at N=1: `hpgmg-fv 7 8` = 256^3 as 2^3 boxes of 128^3 (configs[1]);
@@ -252,6 +252,8 @@ def ours(args):
     ms_per_step = dev_ms / args.steps
     value = dof / (1e-3 * ms_per_step)
 
+    if args.dump_outputs:            # before the check below: outputs that differ are the ones worth comparing
+        dump_outputs(args.dump_outputs, api, lvl, norm_r, rel, rank, world)
     # the work must be the reference's work: the F-cycle residual norm has to be the one the reference prints for this grid
     gold = golden_norm(log2, total_boxes, args.smoother)
     if gold is not None and norm_r != gold:
@@ -379,6 +381,26 @@ def ours(args):
         dist.destroy_process_group()
 
 
+DUMP_SAMPLE_CELLS = 1 << 22             # 32 MB of float64 over all ranks: a fixed sample of u where the grid has more cells
+
+
+def dump_outputs(out_dir, api, lvl, norm_r, rel, rank, world):
+    """What the last timed FMGSolve gave its caller: u on the cells of this rank's level-0 boxes (box by box, [k][j][i],
+    a sample at fixed seeded positions when there are more than this rank's share of DUMP_SAMPLE_CELLS) and the F-cycle
+    residual norm."""
+    import numpy as np
+    Lc = lvl.contents
+    u = np.concatenate([np.ascontiguousarray(api.interior(lvl, api.download(lvl, b, api.VECTOR_U))).reshape(-1)
+                        for b in range(Lc.num_my_boxes)])
+    share = DUMP_SAMPLE_CELLS // world
+    if u.size > share:
+        u = u[np.sort(np.random.default_rng(rank).choice(u.size, share, replace=False))]
+    suffix = f"_rank{rank}" if world > 1 else ""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"u{suffix}.npy"), u.astype(np.float64))
+    np.save(os.path.join(out_dir, f"f_cycle_norm{suffix}.npy"), np.array([norm_r, rel], dtype=np.float64))
+
+
 _REAL_STDOUT = None
 
 
@@ -411,6 +433,8 @@ def main():
     ap.add_argument("--ref-build", default="", choices=["", "O2", "Ofast-native", "Ofast-v3"], help="--impl reference: which build of the reference (default: the fastest that runs here)")
     ap.add_argument("--no-graphs", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write u of the last one (a fixed sample on large grids) and its residual norm to DIR/*.npy")
     ap.add_argument("--ncu", default="", choices=["", "solve", "sweep", "ops"], help="bracket one solve / two smoother sweeps / residual+restriction+interpolations of level 0 with cudaProfilerStart/Stop and exit")
     args = ap.parse_args()
     if args.impl == "reference":

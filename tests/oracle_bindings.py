@@ -12,6 +12,7 @@ import json
 import os
 import subprocess
 import sys
+import zlib
 
 import numpy as np
 
@@ -30,6 +31,82 @@ GOLDEN = os.path.join(ROOT, "tests", "golden", "goldens.json")
 def goldens():
     with open(GOLDEN) as f:
         return json.load(f)
+
+
+# ---------------------------------------------------------------------------------------------- pins
+# The reference library is built only where its sources are present.  What a reference comparison compares against is
+# also stored in tests/golden/pins.json, recorded from the reference itself, so that the comparison holds on a machine
+# without the reference too.  HPGMG_B200_RECORD_PINS=<file> records the reference's values into <file>; recording
+# refuses to run without the reference build.
+PINS = os.path.join(ROOT, "tests", "golden", "pins.json")
+PIN_SAMPLES = 8                 # values stored beside an array's hash, at evenly spaced positions, for the failure message
+_recorded = {}
+
+
+@functools.lru_cache(None)
+def pins():
+    with open(PINS) as f:
+        return json.load(f)
+
+
+def seed(*parts):
+    """A seed for np.random.default_rng that is the same in every process (hash() of a str is not)."""
+    return zlib.crc32(" ".join(map(str, parts)).encode())
+
+
+def fingerprint(value):
+    """Exact fingerprint: a float as float.hex, an int as itself, a str as its sha1; an array or a list of arrays as a sha1
+    of their float64 bytes, their size and PIN_SAMPLES of their values."""
+    if isinstance(value, (int, np.integer)) and not isinstance(value, bool):
+        return int(value)
+    if isinstance(value, (float, np.floating)):
+        return float(value).hex()
+    h = hashlib.sha1()
+    if isinstance(value, str):
+        h.update(value.encode())
+        return h.hexdigest()[:24]
+    flat = np.concatenate([np.ascontiguousarray(a, dtype=np.float64).reshape(-1) for a in (value if isinstance(value, list) else [value])])
+    h.update(flat.tobytes())
+    at = np.linspace(0, flat.size - 1, min(PIN_SAMPLES, flat.size)).astype(np.int64) if flat.size else []
+    return {"sha1": h.hexdigest()[:24], "size": int(flat.size), "sample": {str(int(i)): float(flat[i]).hex() for i in at}}
+
+
+def _mismatch(fp, want):
+    if not isinstance(want, dict) or not isinstance(fp, dict):
+        return f"{fp!r} differs from the reference's {want!r}"
+    if fp["size"] != want["size"]:
+        return f"{fp['size']} values, the reference has {want['size']}"
+    diffs = {i: (float.fromhex(fp["sample"][i]), float.fromhex(v)) for i, v in want["sample"].items() if fp["sample"][i] != v}
+    return (f"cells differ from the reference's (hash {fp['sha1']} vs {want['sha1']}); at the sampled positions "
+            + (", ".join(f"[{i}] {a!r} vs {b!r}" for i, (a, b) in diffs.items()) if diffs else "all values agree"))
+
+
+def pin(key, ours, theirs):
+    """Assert that ours equals the reference's value stored under key.  theirs is the reference's value computed in this
+    process, or None where the reference is not built; recording stores theirs."""
+    out = os.environ.get("HPGMG_B200_RECORD_PINS")
+    if out:
+        assert theirs is not None, f"{key}: HPGMG_B200_RECORD_PINS records the reference's values; build it first (make -C oracle ref)"
+        _recorded[key] = fingerprint(theirs)
+        with open(out, "w") as f:
+            json.dump(_recorded, f, indent=0, sort_keys=True)
+        return                  # the test itself compares ours with theirs
+    stored = pins()
+    assert key in stored, f"{key}: nothing recorded in tests/golden/pins.json"
+    fp = fingerprint(ours)
+    assert fp == stored[key], f"{key}: {_mismatch(fp, stored[key])}"
+
+
+class NoReference:
+    """Stands in for the reference's hierarchy or library where the reference is not built: every call does nothing and
+    returns None, so that a test runs its own side and checks it against the pins alone."""
+    mg = None
+
+    def level(self, l):
+        return None
+
+    def __getattr__(self, name):
+        return lambda *args: None
 
 
 # ---------------------------------------------------------------------------------------------- oracle
@@ -99,7 +176,31 @@ def ref(cheby=False):
     """The reference compiled as a shared library, bound with the same signatures as ours."""
     path = os.path.join(REF_DIR, "libhpgmg_ref_cheby.so" if cheby else "libhpgmg_ref.so")
     L = C.CDLL(path)           # RTLD_LOCAL: its symbols (smooth, norm, ...) must not clash with ours
-    return api.bind(L, {k: api.SIGNATURES[k] for k in _REF_SYMBOLS})
+    if hasattr(L, "create_level"):
+        return api.bind(L, {k: api.SIGNATURES[k] for k in _REF_SYMBOLS})
+    return _bind_by_symbol_table(L, path)
+
+
+def _bind_by_symbol_table(L, path):
+    """A reference build that does not export its functions (its hpgmg-fv executable, made loadable by clearing the PIE
+    flag of its dynamic section): the functions at the load address plus their symbol-table values."""
+    value = {}
+    for line in subprocess.run(["nm", "--defined-only", path], capture_output=True, text=True, check=True).stdout.splitlines():
+        f = line.split()
+        if len(f) == 3 and f[1] in "Tt":
+            value[f[2]] = int(f[0], 16)
+    link_map = C.c_void_p()
+    assert C.CDLL(None).dlinfo(C.c_void_p(L._handle), 2, C.byref(link_map)) == 0       # RTLD_DI_LINKMAP
+    base = C.cast(link_map, C.POINTER(C.c_size_t))[0]                                   # link_map.l_addr
+
+    class Functions:
+        pass
+    out = Functions()
+    for k in _REF_SYMBOLS:
+        res, args = api.SIGNATURES[k]
+        setattr(out, k, C.CFUNCTYPE(res, *args)(base + value[k]))
+    out._keep = L
+    return out
 
 
 @contextlib.contextmanager

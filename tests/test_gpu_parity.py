@@ -186,23 +186,35 @@ def test_pipelined_host_solves_equal_the_serial_call(gpu_lib):
 
 # ------------------------------------------------------------------------------ operator by operator
 def mirror_random(H, R, rng, levels, ids):
-    """Identical seeded data (ghost zones included) in our device level and the reference's host level."""
+    """Identical seeded data (ghost zones included) in our device level and, when R is not None, the reference's host level."""
     for l in levels:
-        nb = R.level(l).contents.num_my_boxes
-        for b in range(nb):
+        Lc = H.level(l).contents
+        n = Lc.box_dim + 2 * Lc.box_ghosts
+        for b in range(Lc.num_my_boxes):
             for vid in ids:
-                a = rng.standard_normal(R.array(l, b, vid).shape)
-                R.array(l, b, vid)[...] = a
+                a = rng.standard_normal((n, n, Lc.box_jStride))
+                if R is not None:
+                    R.array(l, b, vid)[...] = a
                 api.upload(H.level(l), b, vid, a)
 
 
 def assert_level_equal(H, R, l, vid, where, what):
-    Lc = R.level(l).contents
+    """Our vector vid on level l, cell by cell: against the reference's when R is not None, and against the reference's
+    recorded under `what` (ob.pin)."""
+    Lc = H.level(l).contents
     n = Lc.box_dim
-    for b in range(Lc.num_my_boxes):
-        ours, ref = api.download(H.level(l), b, vid), R.array(l, b, vid)
-        s = slice(2, 2 + n) if where == "in" else slice(0, n + 4)
-        np.testing.assert_array_equal(ours[s, s, s], ref[s, s, s], err_msg=f"{what}: level {l} box {b} vec {vid} ({where})")
+    s = slice(2, 2 + n) if where == "in" else slice(0, n + 4)
+    ours = [api.download(H.level(l), b, vid)[s, s, s] for b in range(Lc.num_my_boxes)]
+    theirs = None if R is None else [R.array(l, b, vid)[s, s, s] for b in range(Lc.num_my_boxes)]
+    if R is not None:
+        for b in range(Lc.num_my_boxes):
+            np.testing.assert_array_equal(ours[b], theirs[b], err_msg=f"{what}: level {l} box {b} vec {vid} ({where})")
+    ob.pin(f"{what}: level {l} vec {vid} ({where})", ours, theirs)
+
+
+def reference(*args, **kw):
+    """The reference library's hierarchy, or None where the reference is not built (the pins stand in for it)."""
+    return ob.RefHierarchy(*args, **kw) if ob.have_ref(kw.get("cheby", False)) else None
 
 
 OPS = ["exchange_box", "exchange_star", "exchange_nocorners", "bc_v4_box", "bc_v4_nocorners", "bc_v2_box", "bc_v1_box",
@@ -211,7 +223,6 @@ OPS = ["exchange_box", "exchange_star", "exchange_nocorners", "bc_v4_box", "bc_v
        "color", "random", "dot_norm_mean", "extrapolate_betas", "rebuild_blackbox", "iterative_solver", "vcycle"]
 
 
-@pytest.mark.skipif(not ob.have_ref(), reason="oracle/_ref (prebuilt reference library) not shipped")
 @pytest.mark.parametrize("cfg", ["4 8", "4 27", "4 1", "5 8", "6 1"])
 @pytest.mark.parametrize("op", OPS)
 def test_operator_equals_reference(gpu_lib, cfg, op):
@@ -220,90 +231,99 @@ def test_operator_equals_reference(gpu_lib, cfg, op):
     U, E, Rr, T, F, DINV = api.VECTOR_U, api.VECTOR_E, api.VECTOR_R, api.VECTOR_TEMP, api.VECTOR_F, api.VECTOR_DINV
     BI, BJ, BK = api.VECTOR_BETA_I, api.VECTOR_BETA_J, api.VECTOR_BETA_K
     with api.Hierarchy(log2, boxes, use_graphs=False) as H:
-        R = ob.RefHierarchy(log2, boxes)
-        rng = np.random.default_rng(hash((cfg, op)) % (2 ** 32))
+        R = reference(log2, boxes)
+        rng = np.random.default_rng(ob.seed(cfg, op))
         mirror_random(H, R, rng, (0, 1), (U, E, Rr, T))
-        l0, l1, r0, r1 = H.level(0), H.level(1), R.level(0), R.level(1)
+        Rc = R or ob.NoReference()
+        l0, l1, r0, r1 = H.level(0), H.level(1), Rc.level(0), Rc.level(1)
         a, b = 0.0, 1.0
         checks = []
+        key = f"operator {cfg} {op}"
+
+        def same(what, ours, theirs):
+            if R is not None:
+                assert ours == theirs, (what, ours, theirs)
+            ob.pin(f"{key}: {what}", ours, theirs)
 
         if op.startswith("exchange_"):
             shape = {"box": 0, "star": 1, "nocorners": 2}[op.split("_")[1]]
-            L.exchange_boundary(l0, U, shape); R.call("exchange_boundary", r0, U, shape); checks = [(0, U, "all")]
+            L.exchange_boundary(l0, U, shape); Rc.call("exchange_boundary", r0, U, shape); checks = [(0, U, "all")]
         elif op.startswith("bc_"):
             v, shp = op.split("_")[1], {"box": 0, "nocorners": 2}[op.split("_")[2]]
-            L.exchange_boundary(l0, U, shp); R.call("exchange_boundary", r0, U, shp)
+            L.exchange_boundary(l0, U, shp); Rc.call("exchange_boundary", r0, U, shp)
             getattr(L, f"apply_BCs_{v}")(l0, U, shp)
             with ob.ref_threads(1):
-                R.call(f"apply_BCs_{v}", r0, U, shp)
+                Rc.call(f"apply_BCs_{v}", r0, U, shp)
             checks = [(0, U, "all")]
         elif op == "apply_op":
-            L.apply_op(l0, T, U, a, b); R.call("apply_op", r0, T, U, a, b); checks = [(0, T, "in"), (0, U, "all")]
+            L.apply_op(l0, T, U, a, b); Rc.call("apply_op", r0, T, U, a, b); checks = [(0, T, "in"), (0, U, "all")]
         elif op == "residual":
-            L.residual(l0, T, U, Rr, a, b); R.call("residual", r0, T, U, Rr, a, b); checks = [(0, T, "in"), (0, U, "all")]
+            L.residual(l0, T, U, Rr, a, b); Rc.call("residual", r0, T, U, Rr, a, b); checks = [(0, T, "in"), (0, U, "all")]
         elif op == "smooth_gsrb":
-            L.smooth(l0, U, Rr, a, b); R.call("smooth", r0, U, Rr, a, b); checks = [(0, U, "in"), (0, T, "in")]
+            L.smooth(l0, U, Rr, a, b); Rc.call("smooth", r0, U, Rr, a, b); checks = [(0, U, "in"), (0, T, "in")]
         elif op.startswith("restrict_"):
             t = {"cell": 0, "face_i": 1, "face_j": 2, "face_k": 3}[op[len("restrict_"):]]
-            L.restriction(l1, Rr, l0, T, t); R.call("restriction", r1, Rr, r0, T, t); checks = [(1, Rr, "all")]
+            L.restriction(l1, Rr, l0, T, t); Rc.call("restriction", r1, Rr, r0, T, t); checks = [(1, Rr, "all")]
         elif op == "interp_v2":
-            L.interpolation_v2(l0, U, 1.0, l1, E); R.call("interpolation_v2", r0, U, 1.0, r1, E); checks = [(0, U, "in"), (1, E, "all")]
+            L.interpolation_v2(l0, U, 1.0, l1, E); Rc.call("interpolation_v2", r0, U, 1.0, r1, E); checks = [(0, U, "in"), (1, E, "all")]
         elif op.startswith("interp_v4"):
             ps = float(op[-1])
-            L.interpolation_v4(l0, U, ps, l1, E); R.call("interpolation_v4", r0, U, ps, r1, E); checks = [(0, U, "in"), (1, E, "all")]
+            L.interpolation_v4(l0, U, ps, l1, E); Rc.call("interpolation_v4", r0, U, ps, r1, E); checks = [(0, U, "in"), (1, E, "all")]
         elif op == "zero":
-            L.zero_vector(l0, U); R.call("zero_vector", r0, U); checks = [(0, U, "all")]
+            L.zero_vector(l0, U); Rc.call("zero_vector", r0, U); checks = [(0, U, "all")]
         elif op == "init":
-            L.init_vector(l0, U, 3.25); R.call("init_vector", r0, U, 3.25); checks = [(0, U, "all")]
+            L.init_vector(l0, U, 3.25); Rc.call("init_vector", r0, U, 3.25); checks = [(0, U, "all")]
         elif op == "scale":
-            L.scale_vector(l0, T, -1.7, U); R.call("scale_vector", r0, T, -1.7, U); checks = [(0, T, "all")]
+            L.scale_vector(l0, T, -1.7, U); Rc.call("scale_vector", r0, T, -1.7, U); checks = [(0, T, "all")]
         elif op == "add":
-            L.add_vectors(l0, T, 0.3, U, -2.1, E); R.call("add_vectors", r0, T, 0.3, U, -2.1, E); checks = [(0, T, "all")]
+            L.add_vectors(l0, T, 0.3, U, -2.1, E); Rc.call("add_vectors", r0, T, 0.3, U, -2.1, E); checks = [(0, T, "all")]
         elif op == "mul":
-            L.mul_vectors(l0, T, 1.3, U, E); R.call("mul_vectors", r0, T, 1.3, U, E); checks = [(0, T, "all")]
+            L.mul_vectors(l0, T, 1.3, U, E); Rc.call("mul_vectors", r0, T, 1.3, U, E); checks = [(0, T, "all")]
         elif op == "invert":
-            L.invert_vector(l0, T, 2.0, U); R.call("invert_vector", r0, T, 2.0, U); checks = [(0, T, "all")]
+            L.invert_vector(l0, T, 2.0, U); Rc.call("invert_vector", r0, T, 2.0, U); checks = [(0, T, "all")]
         elif op == "shift":
-            L.shift_vector(l0, T, U, 0.125); R.call("shift_vector", r0, T, U, 0.125); checks = [(0, T, "all")]
+            L.shift_vector(l0, T, U, 0.125); Rc.call("shift_vector", r0, T, U, 0.125); checks = [(0, T, "all")]
         elif op == "color":
-            L.color_vector(l0, T, 4, 1, 2, 3); R.call("color_vector", r0, T, 4, 1, 2, 3); checks = [(0, T, "all")]
+            L.color_vector(l0, T, 4, 1, 2, 3); Rc.call("color_vector", r0, T, 4, 1, 2, 3); checks = [(0, T, "all")]
         elif op == "random":
-            L.random_vector(l0, T); R.call("random_vector", r0, T); checks = [(0, T, "all")]
+            L.random_vector(l0, T); Rc.call("random_vector", r0, T); checks = [(0, T, "all")]
         elif op == "dot_norm_mean":
             # the reference's OpenMP reduction order over tiles is only defined for one thread; norm is order-free
-            assert L.norm(l0, U) == R.call("norm", r0, U)
+            same("norm", L.norm(l0, U), Rc.call("norm", r0, U))
             with ob.ref_threads(1):
-                assert L.dot(l0, U, E) == R.call("dot", r0, U, E)
-                assert L.mean(l0, U) == R.call("mean", r0, U)
-            assert L.error(l0, U, E) == R.call("error", r0, U, E)
+                same("dot", L.dot(l0, U, E), Rc.call("dot", r0, U, E))
+                same("mean", L.mean(l0, U), Rc.call("mean", r0, U))
+            same("error", L.error(l0, U, E), Rc.call("error", r0, U, E))
         elif op == "extrapolate_betas":
             mirror_random(H, R, rng, (0,), (BI, BJ, BK))
-            L.extrapolate_betas(l0); R.call("extrapolate_betas", r0)
-            Lc = R.level(0).contents
+            L.extrapolate_betas(l0); Rc.call("extrapolate_betas", r0)
+            Lc = l0.contents
             n = Lc.box_dim
             ring = slice(1, n + 3)       # only the first ghost layer is ever read (and is order-independent)
-            for bx in range(Lc.num_my_boxes):
-                for vid in (BI, BJ, BK):
-                    np.testing.assert_array_equal(api.download(l0, bx, vid)[ring, ring, ring], R.array(0, bx, vid)[ring, ring, ring])
+            for vid in (BI, BJ, BK):
+                ours = [api.download(l0, bx, vid)[ring, ring, ring] for bx in range(Lc.num_my_boxes)]
+                if R is not None:
+                    for bx in range(Lc.num_my_boxes):
+                        np.testing.assert_array_equal(ours[bx], R.array(0, bx, vid)[ring, ring, ring])
+                ob.pin(f"{key}: vec {vid} (ring)", ours, [R.array(0, bx, vid)[ring, ring, ring] for bx in range(Lc.num_my_boxes)] if R else None)
         elif op == "rebuild_blackbox":
-            L.rebuild_operator_blackbox(l0, a, b, 4); R.call("rebuild_operator_blackbox", r0, a, b, 4)
-            assert l0.contents.dominant_eigenvalue_of_DinvA == r0.contents.dominant_eigenvalue_of_DinvA
+            L.rebuild_operator_blackbox(l0, a, b, 4); Rc.call("rebuild_operator_blackbox", r0, a, b, 4)
+            same("eig", l0.contents.dominant_eigenvalue_of_DinvA, r0.contents.dominant_eigenvalue_of_DinvA if R else None)
             checks = [(0, DINV, "in"), (0, E, "in")]
         elif op == "iterative_solver":
-            lb, rb = H.level(H.num_levels - 1), R.level(R.num_levels - 1)
+            lb, rb = H.level(H.num_levels - 1), R.level(R.num_levels - 1) if R else None
             mirror_random(H, R, rng, (H.num_levels - 1,), (U, Rr))
-            L.IterativeSolver(lb, U, Rr, a, b, 1e-3); R.call("IterativeSolver", rb, U, Rr, a, b, 1e-3)
+            L.IterativeSolver(lb, U, Rr, a, b, 1e-3); Rc.call("IterativeSolver", rb, U, Rr, a, b, 1e-3)
             checks = [(H.num_levels - 1, U, "in")]
         elif op == "vcycle":
-            L.MGVCycle(H.mg, E, Rr, a, b, 0); R.call("MGVCycle", R.mg, E, Rr, a, b, 0)
+            L.MGVCycle(H.mg, E, Rr, a, b, 0); Rc.call("MGVCycle", Rc.mg, E, Rr, a, b, 0)
             checks = [(l, E, "in") for l in range(H.num_levels)]
         else:
             raise AssertionError(op)
         for l, vid, where in checks:
-            assert_level_equal(H, R, l, vid, where, op)
+            assert_level_equal(H, R, l, vid, where, key)
 
 
-@pytest.mark.skipif(not ob.have_ref(), reason="oracle/_ref (prebuilt reference library) not shipped")
 @pytest.mark.parametrize("log2", [7, 8])
 def test_large_single_box_operators_equal_reference(gpu_lib, log2):
     """One 128^3 box (`7 1`: the box size behind the headline number) and one 256^3 box (`8 1`: BASELINE config 4):
@@ -312,26 +332,29 @@ def test_large_single_box_operators_equal_reference(gpu_lib, log2):
     L = gpu_lib
     U, E, Rr, T = api.VECTOR_U, api.VECTOR_E, api.VECTOR_R, api.VECTOR_TEMP
     with api.Hierarchy(log2, 1, use_graphs=False) as H:
-        R = ob.RefHierarchy(log2, 1)
+        R = reference(log2, 1)
+        Rc = R or ob.NoReference()
         rng = np.random.default_rng(log2)
         mirror_random(H, R, rng, (0,), (U, Rr, T))
         mirror_random(H, R, rng, (1,), (E,))
-        l0, l1, r0, r1 = H.level(0), H.level(1), R.level(0), R.level(1)
-        L.smooth(l0, U, Rr, 0.0, 1.0); R.call("smooth", r0, U, Rr, 0.0, 1.0)
-        assert_level_equal(H, R, 0, U, "in", "smooth")
-        assert_level_equal(H, R, 0, T, "in", "smooth (TEMP)")
-        L.residual(l0, T, U, Rr, 0.0, 1.0); R.call("residual", r0, T, U, Rr, 0.0, 1.0)
-        assert_level_equal(H, R, 0, T, "in", "residual")
-        assert L.norm(l0, T) == R.call("norm", r0, T)
-        L.restriction(l1, Rr, l0, T, api.RESTRICT_CELL); R.call("restriction", r1, Rr, r0, T, api.RESTRICT_CELL)
-        assert_level_equal(H, R, 1, Rr, "in", "restriction")
-        L.interpolation_v2(l0, U, 1.0, l1, E); R.call("interpolation_v2", r0, U, 1.0, r1, E)
-        assert_level_equal(H, R, 0, U, "in", "interpolation_v2")
-        L.interpolation_v4(l0, T, 0.0, l1, E); R.call("interpolation_v4", r0, T, 0.0, r1, E)
-        assert_level_equal(H, R, 0, T, "in", "interpolation_v4")
+        l0, l1, r0, r1 = H.level(0), H.level(1), Rc.level(0), Rc.level(1)
+        key = f"large box {log2} 1"
+        L.smooth(l0, U, Rr, 0.0, 1.0); Rc.call("smooth", r0, U, Rr, 0.0, 1.0)
+        assert_level_equal(H, R, 0, U, "in", f"{key} smooth")
+        assert_level_equal(H, R, 0, T, "in", f"{key} smooth (TEMP)")
+        L.residual(l0, T, U, Rr, 0.0, 1.0); Rc.call("residual", r0, T, U, Rr, 0.0, 1.0)
+        assert_level_equal(H, R, 0, T, "in", f"{key} residual")
+        norm, ref_norm = L.norm(l0, T), Rc.call("norm", r0, T)
+        assert R is None or norm == ref_norm
+        ob.pin(f"{key} norm", norm, ref_norm)
+        L.restriction(l1, Rr, l0, T, api.RESTRICT_CELL); Rc.call("restriction", r1, Rr, r0, T, api.RESTRICT_CELL)
+        assert_level_equal(H, R, 1, Rr, "in", f"{key} restriction")
+        L.interpolation_v2(l0, U, 1.0, l1, E); Rc.call("interpolation_v2", r0, U, 1.0, r1, E)
+        assert_level_equal(H, R, 0, U, "in", f"{key} interpolation_v2")
+        L.interpolation_v4(l0, T, 0.0, l1, E); Rc.call("interpolation_v4", r0, T, 0.0, r1, E)
+        assert_level_equal(H, R, 0, T, "in", f"{key} interpolation_v4")
 
 
-@pytest.mark.skipif(not ob.have_ref(), reason="oracle/_ref (prebuilt reference library) not shipped")
 def test_overwritten_diagonal_is_read_not_recomputed(gpu_lib):
     """The TMA GSRB kernel forms Dinv = 1/Aii in registers only while VECTOR_DINV is known to come from
     rebuild_operator_blackbox: once ANY operator of the API writes vector 5 the kernel must read it again."""
@@ -339,20 +362,21 @@ def test_overwritten_diagonal_is_read_not_recomputed(gpu_lib):
     U, Rr, DINV, E = api.VECTOR_U, api.VECTOR_R, api.VECTOR_DINV, api.VECTOR_E
     for writer in ("scale", "mul", "add", "restriction"):
         with api.Hierarchy(6, 1, use_graphs=False) as H:             # one 64^3 box: the TMA kernel, tiles away from the boundary
-            R = ob.RefHierarchy(6, 1)
+            R = reference(6, 1)
             rng = np.random.default_rng(11)
             mirror_random(H, R, rng, (0, 1), (U, Rr, E))
             lv, rl = (1, 1) if writer == "restriction" else (0, 0)
-            l, r = H.level(lv), R.level(rl)
+            Rc = R or ob.NoReference()
+            l, r = H.level(lv), Rc.level(rl)
             if writer == "scale":
-                L.scale_vector(l, DINV, 0.5, DINV); R.call("scale_vector", r, DINV, 0.5, DINV)
+                L.scale_vector(l, DINV, 0.5, DINV); Rc.call("scale_vector", r, DINV, 0.5, DINV)
             elif writer == "mul":
-                L.mul_vectors(l, DINV, 1.25, DINV, DINV); R.call("mul_vectors", r, DINV, 1.25, DINV, DINV)
+                L.mul_vectors(l, DINV, 1.25, DINV, DINV); Rc.call("mul_vectors", r, DINV, 1.25, DINV, DINV)
             elif writer == "add":
-                L.add_vectors(l, DINV, 0.75, DINV, 0.0, E); R.call("add_vectors", r, DINV, 0.75, DINV, 0.0, E)
+                L.add_vectors(l, DINV, 0.75, DINV, 0.0, E); Rc.call("add_vectors", r, DINV, 0.75, DINV, 0.0, E)
             else:                                                    # level 1 (32^3): Dinv <- restriction of the fine Dinv
-                L.restriction(l, DINV, H.level(0), DINV, api.RESTRICT_CELL); R.call("restriction", r, DINV, R.level(0), DINV, api.RESTRICT_CELL)
-            L.smooth(l, U, Rr, 0.0, 1.0); R.call("smooth", r, U, Rr, 0.0, 1.0)
+                L.restriction(l, DINV, H.level(0), DINV, api.RESTRICT_CELL); Rc.call("restriction", r, DINV, Rc.level(0), DINV, api.RESTRICT_CELL)
+            L.smooth(l, U, Rr, 0.0, 1.0); Rc.call("smooth", r, U, Rr, 0.0, 1.0)
             assert_level_equal(H, R, lv, U, "in", f"smooth after {writer} wrote Dinv")
 
 
@@ -387,27 +411,28 @@ def test_last_norms_are_kept_per_hierarchy(gpu_lib):
         assert gpu_lib.hpgmg_last_norm_of_F(A.mg) == ga["norm_of_F"] and gpu_lib.hpgmg_last_norm_of_F(B.mg) == gb["norm_of_F"]
 
 
-@pytest.mark.skipif(not ob.have_ref(), reason="oracle/_ref (prebuilt reference library) not shipped")
 def test_multibox_bottom_level_solves_without_recording(gpu_lib):
     """MGBuild(minCoarseGridDim=16) on `4 8` stops at a 16^3 bottom level of 8 boxes: the bottom solve is the
     host-driven BiCGStab (dots and norms read back every iteration), which must not be stream-captured."""
     U, F = api.VECTOR_U, api.VECTOR_F
     H = api.Hierarchy(4, 8, build_operator=False, use_graphs=True)
-    R = ob.RefHierarchy(4, 8, build_operator=False)
+    R = reference(4, 8, build_operator=False)
     try:
         gpu_lib.initialize_problem(H.level_h, H.h, 0.0, 1.0)
         gpu_lib.rebuild_operator(H.level_h, None, 0.0, 1.0)
         gpu_lib.MGBuild(H.mg, H.level_h, 0.0, 1.0, 16)
         H.built = True
-        with ob.quiet():
-            R.L.initialize_problem(R.level_h, R.h, 0.0, 1.0)
-            R.L.rebuild_operator(R.level_h, None, 0.0, 1.0)
-            R.L.MGBuild(R.mg, R.level_h, 0.0, 1.0, 16)
-        R.built = True
-        assert H.num_levels == R.num_levels == 2
-        with ob.ref_threads(1):                  # the reference's dots are sums over tiles: order defined on one thread
-            R.call("zero_vector", R.level(0), U)
-            R.call("FMGSolve", R.mg, 0, U, F, 0.0, 1.0, 1e-10)
+        assert H.num_levels == 2
+        if R is not None:
+            with ob.quiet():
+                R.L.initialize_problem(R.level_h, R.h, 0.0, 1.0)
+                R.L.rebuild_operator(R.level_h, None, 0.0, 1.0)
+                R.L.MGBuild(R.mg, R.level_h, 0.0, 1.0, 16)
+            R.built = True
+            assert R.num_levels == 2
+            with ob.ref_threads(1):              # the reference's dots are sums over tiles: order defined on one thread
+                R.call("zero_vector", R.level(0), U)
+                R.call("FMGSolve", R.mg, 0, U, F, 0.0, 1.0, 1e-10)
         for _ in range(2):                       # twice: a recorded graph would be replayed the second time
             gpu_lib.zero_vector(H.level(0), U)
             gpu_lib.FMGSolve(H.mg, 0, U, F, 0.0, 1.0, 1e-10)
@@ -417,15 +442,18 @@ def test_multibox_bottom_level_solves_without_recording(gpu_lib):
         H.close()
 
 
-@pytest.mark.skipif(not ob.have_ref(True), reason="oracle/_ref (prebuilt Chebyshev reference library) not shipped")
 def test_chebyshev_smoother_equals_reference(gpu_lib):
     with api.Hierarchy(4, 8, smoother=api.SMOOTHER_CHEBY, use_graphs=False) as H:
-        R = ob.RefHierarchy(4, 8, cheby=True)
+        R = reference(4, 8, cheby=True)
         rng = np.random.default_rng(7)
         mirror_random(H, R, rng, (0,), (api.VECTOR_U, api.VECTOR_R, api.VECTOR_TEMP))
-        assert H.level(0).contents.dominant_eigenvalue_of_DinvA == R.level(0).contents.dominant_eigenvalue_of_DinvA
+        eig = H.level(0).contents.dominant_eigenvalue_of_DinvA
+        ref_eig = R.level(0).contents.dominant_eigenvalue_of_DinvA if R else None
+        assert R is None or eig == ref_eig
+        ob.pin("chebyshev eig", eig, ref_eig)
         gpu_lib.smooth(H.level(0), api.VECTOR_U, api.VECTOR_R, 0.0, 1.0)
-        R.call("smooth", R.level(0), api.VECTOR_U, api.VECTOR_R, 0.0, 1.0)
+        if R is not None:
+            R.call("smooth", R.level(0), api.VECTOR_U, api.VECTOR_R, 0.0, 1.0)
         assert_level_equal(H, R, 0, api.VECTOR_U, "in", "chebyshev")
         assert_level_equal(H, R, 0, api.VECTOR_TEMP, "in", "chebyshev")
     gpu_lib.hpgmg_b200_set_smoother(api.SMOOTHER_GSRB)
@@ -557,17 +585,17 @@ def test_multi_gpu_fmg_equals_single_process_reference(gpu_lib, ranks):
 
 
 # ------------------------------------------------------------------------- the other solve drivers of mg.c
-@pytest.mark.skipif(not ob.have_ref(), reason="oracle/_ref (prebuilt reference library) not shipped")
 @pytest.mark.parametrize("driver", ["MGSolve", "FMGSolve2", "MGPCG"])
 def test_other_solve_drivers_equal_reference(gpu_lib, driver):
     """MGSolve (V-cycles to rtol, mg.c:1168-1233), FMGSolve2 (mg.c:1348-1495) and MGPCG (mg.c:1500-1607) are part of the
     API surface of the path (SURVEY.md 8a20): same solution as the reference library, cell by cell.  The reference
     runs on one OpenMP thread: MGPCG's dots are sums over tiles whose order is only defined there."""
     with api.Hierarchy(5, 8, verbose=False) as H:
-        R = ob.RefHierarchy(5, 8)
-        with ob.ref_threads(1):
-            R.call("zero_vector", R.level(0), api.VECTOR_U)
-            R.call(driver, R.mg, 0, api.VECTOR_U, api.VECTOR_F, 0.0, 1.0, 1e-10)
+        R = reference(5, 8)
+        if R is not None:
+            with ob.ref_threads(1):
+                R.call("zero_vector", R.level(0), api.VECTOR_U)
+                R.call(driver, R.mg, 0, api.VECTOR_U, api.VECTOR_F, 0.0, 1.0, 1e-10)
         gpu_lib.zero_vector(H.level(0), api.VECTOR_U)
         getattr(gpu_lib, driver)(H.mg, 0, api.VECTOR_U, api.VECTOR_F, 0.0, 1.0, 1e-10)
         gpu_lib.hpgmg_b200_sync()
