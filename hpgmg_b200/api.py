@@ -25,7 +25,7 @@ VECTORS_RESERVED = 9
 BC_PERIODIC, BC_DIRICHLET = 0, 1
 STENCIL_SHAPE_BOX, STENCIL_SHAPE_STAR, STENCIL_SHAPE_NO_CORNERS = 0, 1, 2
 RESTRICT_CELL, RESTRICT_FACE_I, RESTRICT_FACE_J, RESTRICT_FACE_K = 0, 1, 2, 3
-SMOOTHER_GSRB, SMOOTHER_CHEBY = 0, 1
+SMOOTHER_GSRB, SMOOTHER_CHEBY, SMOOTHER_JACOBI, SMOOTHER_L1JACOBI = 0, 1, 2, 3    # include/hpgmg_b200.h
 
 ALLGATHER_FN = C.CFUNCTYPE(None, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p)
 BARRIER_FN = C.CFUNCTYPE(None, C.c_void_p)
@@ -46,6 +46,7 @@ SIGNATURES = {
     "hpgmg_b200_profile_operators": (_V, [_I]), "hpgmg_b200_use_coarse_kernel": (_V, [_I]), "hpgmg_b200_coarse_profile": (_V, [_I, C.c_void_p]), "hpgmg_b200_coarse_levels_in_smem": (_V, [_I]), "hpgmg_b200_set_layout_only": (_V, [_I]),
     "hpgmg_download_box_vector": (_V, [_LP, _I, _I, C.c_void_p]),
     "hpgmg_upload_box_vector": (_V, [_LP, _I, _I, C.c_void_p]),
+    "hpgmg_download_l1inv": (_V, [_LP, _I, C.c_void_p]),
     "hpgmg_b200_host_alloc_pinned": (C.c_void_p, [C.c_size_t]), "hpgmg_b200_host_free_pinned": (_V, [C.c_void_p]),
     "hpgmg_fmg_solve_host": (_D, [_MP, _I, _I, _I, _D, _D, _D, C.c_void_p, C.c_void_p]),
     "hpgmg_fmg_solve_host_bytes": (C.c_ulonglong, [_MP, _I]),

@@ -13,9 +13,9 @@
  * with __syncthreads() where the stream version has kernel boundaries.
  *
  * Residency.  A single-box level keeps the vectors the cycle touches (TEMP, e, R, Dinv, beta_i/j/k; on the
- * bottom level also the 8 Krylov vectors) in shared memory for the duration of the kernel: 160 KB for
- * 8^3 + 4^3 + 2^3.  They arrive and leave as bulk asynchronous copies (cp.async.bulk, one per vector, issued
- * by one thread and counted by an mbarrier).  The phase program addresses vectors by SLOT, so the same
+ * bottom level also the 8 Krylov vectors; under L1-Jacobi the level's L1 row inverse, which is not in the slab)
+ * in shared memory for the duration of the kernel: 160 KB for 8^3 + 4^3 + 2^3.  They arrive and leave as bulk
+ * asynchronous copies (cp.async.bulk, one per vector, issued by one thread and counted by an mbarrier).  The phase program addresses vectors by SLOT, so the same
  * operator bodies run on a level that stays in global memory (slot == vector id there).
  *
  * Speed.  A phase is latency-bound: one warp issuing the instructions of one fv4 stencil.  The resident
@@ -54,6 +54,10 @@ struct CoarseLevel {
   int restr_cells, interp_cells;                  /* cells of the largest entry of each list */
   double h2inv;
   double c1[6], c2[6];                            /* Chebyshev coefficients of this level */
+  double jw;                                      /* Jacobi weight (jacobi.c): 2/3 with lambda = Dinv, 1 with the L1 row inverse */
+  const double *l1;                               /* L1-Jacobi: the level's L1 row inverse in global memory ([box][volume]) */
+  int s_lam;                                      /* slot of lambda; -1: read it from l1.  == nslots on a resident level under L1-Jacobi:
+                                                     the resident copy of l1, right after the slots */
   int smem_offset;                                /* >=0: resident, doubles from the start of the pool */
   int nslots;
   int fast;                                       /* 8, 4, 2: resident single box of that size, specialised bodies; 0: generic */
@@ -122,7 +126,7 @@ __device__ static void c_fill_ghosts(const CoarseLevel &V, const int slot, const
   }
 }
 
-/* one sweep / residual over every cell of every box.  mode: 0 GSRB sweep s, 1 Chebyshev sweep s, 2 residual.
+/* one sweep / residual over every cell of every box.  mode: 0 GSRB sweep s, 1 Chebyshev sweep s, 2 residual, 3 Jacobi sweep.
  * GSRB on even boxes: a thread owns an i-pair (exactly one active cell per pair, so no lane idles). */
 __device__ static void c_stencil(const CoarseLevel &V, const int mode, const int src, const int dst, const int rhs_slot, const int s, const double b)
 {
@@ -160,6 +164,11 @@ __device__ static void c_stencil(const CoarseLevel &V, const int mode, const int
     const double Ax = fv4_apply_op(x, L.vec(box, V.s_bi) + ijk, L.vec(box, V.s_bj) + ijk, L.vec(box, V.s_bk) + ijk, jS, kS, b, V.h2inv);
     const double rhs = L.vec(box, rhs_slot)[ijk];
     if (mode == 2) { out[0] = rhs - Ax; continue; }
+    if (mode == 3) {                                                /* jacobi.c: x_n + weight*lambda*(rhs - Ax_n) */
+      const double lam = V.s_lam >= 0 ? L.vec(box, V.s_lam)[ijk] : V.l1[(size_t)box * L.volume + L.origin + ijk];
+      out[0] = x[0] + (V.jw * lam) * (rhs - Ax);
+      continue;
+    }
     const double dinv = L.vec(box, V.s_dinv)[ijk];
     if (mode == 0) out[0] = x[0] + dinv * (rhs - Ax);
     else { const double xn = x[0]; out[0] = xn + V.c1[s] * (xn - out[0]) + V.c2[s] * dinv * (rhs - Ax); }
@@ -294,14 +303,15 @@ __device__ static void c_fill_fast(double *v, const bool box_shape, const bool f
 }
 
 /* one sweep / residual of ONE box of N^3 cells whose low corner is the domain's; `base` points at cell (0,0,0) of slot 0,
- * strides Geo<N>.  GSRB: one thread per i-pair = per updated cell; Chebyshev / residual: one thread per cell. */
+ * strides Geo<N>.  GSRB: one thread per i-pair = per updated cell; Chebyshev / Jacobi / residual: one thread per cell.
+ * Resident levels only: lambda of a Jacobi sweep is always in a slot there. */
 template <int N>
 __device__ static void c_stencil_fast(const CoarseLevel &V, double *base, const int mode, const int src, const int dst, const int rhs_slot, const int s, const double b)
 {
   typedef Geo<N> G;
   constexpr int LG = N == 8 ? 3 : (N == 4 ? 2 : 1);
   const double *x = base + src * G::VOL, *bi = base + V.s_bi * G::VOL, *bj = base + V.s_bj * G::VOL, *bk = base + V.s_bk * G::VOL;
-  const double *rhs = base + rhs_slot * G::VOL, *dinv = base + V.s_dinv * G::VOL;
+  const double *rhs = base + rhs_slot * G::VOL, *dinv = base + V.s_dinv * G::VOL, *lam = base + V.s_lam * G::VOL;
   double *out = base + dst * G::VOL;
   const double h2inv = V.h2inv;
   const int work = mode == 0 ? N * N * N / 2 : N * N * N;
@@ -329,6 +339,8 @@ __device__ static void c_stencil_fast(const CoarseLevel &V, double *base, const 
       out[ijk] = xnew;
     } else if (mode == 2) {
       out[ijk] = rhs[ijk] - Ax;
+    } else if (mode == 3) {
+      out[ijk] = x[ijk] + (V.jw * lam[ijk]) * (rhs[ijk] - Ax);     /* jacobi.c */
     } else {
       const double xn = x[ijk];
       out[ijk] = xn + V.c1[s] * (xn - out[ijk]) + V.c2[s] * dinv[ijk] * (rhs[ijk] - Ax);     /* x_{n-1} aliases x_{n+1} (chebyshev.c:75-80) */
@@ -388,6 +400,7 @@ __global__ void __launch_bounds__(COARSE_THREADS, 1) coarse_cycle_kernel(const _
       if (G.smem_offset < 0) continue;
       A.lv[l].L.base = pool + G.smem_offset;
       for (int sl = 0; sl < G.nslots; sl++) if (G.slot_io[sl] & 1) total += (unsigned)G.L.volume * 8u;
+      if (G.s_lam == G.nslots) total += (unsigned)G.L.volume * 8u;
     }
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(total) : "memory");
     for (int l = 0; l < Ain.nlevels; l++) {
@@ -395,6 +408,7 @@ __global__ void __launch_bounds__(COARSE_THREADS, 1) coarse_cycle_kernel(const _
       if (G.smem_offset < 0) continue;
       for (int sl = 0; sl < G.nslots; sl++)
         if (G.slot_io[sl] & 1) bulk_load(pool + G.smem_offset + (size_t)sl * G.L.volume, G.gbase + (size_t)G.slot_id[sl] * G.L.volume, (unsigned)G.L.volume * 8u, bar);
+      if (G.s_lam == G.nslots) bulk_load(pool + G.smem_offset + (size_t)G.nslots * G.L.volume, G.l1, (unsigned)G.L.volume * 8u, bar);     /* read-only */
     }
   }
   asm volatile(
@@ -547,12 +561,13 @@ static void p_add(CoarseArgs &A, int op, int lv, int a = 0, int b = 0, int c = 0
   Phase P = { (unsigned char)op, (unsigned char)lv, (unsigned char)a, (unsigned char)b, (unsigned char)c, (unsigned char)d, (unsigned char)e, 0 };
   A.prog[A.nphases++] = P;
 }
-static void p_smooth(CoarseArgs &A, const Slots *S, int l)                  /* smooth(): gsrb.c:24-132 / chebyshev.c:8-100 */
+static void p_smooth(CoarseArgs &A, const Slots *S, int l)                  /* smooth(): gsrb.c:24-132 / chebyshev.c:8-100 / jacobi.c */
 {
+  const int mode = A.smoother == HPGMG_SMOOTHER_CHEBY ? 1 : (A.smoother == HPGMG_SMOOTHER_JACOBI || A.smoother == HPGMG_SMOOTHER_L1JACOBI) ? 3 : 0;
   for (int s = 0; s < 6; s++) {
     const int src = (s & 1) ? S[l].temp : S[l].e, dst = (s & 1) ? S[l].e : S[l].temp;
     p_add(A, PH_FILL, l, src, 0, 0);
-    p_add(A, PH_STENCIL, l, A.smoother == HPGMG_SMOOTHER_CHEBY ? 1 : 0, src, dst, S[l].R, s);
+    p_add(A, PH_STENCIL, l, mode, src, dst, S[l].R, s);
   }
 }
 static void p_vcycle(CoarseArgs &A, const Slots *S, int c)                  /* MGVCycle: mg.c:1135-1164 */
@@ -620,6 +635,9 @@ extern "C" void hpgmg_coarse_cycle(mg_type *MG, int from, int mode_ftail, int ze
     double theta = 0.5 * (beta + alpha), delta = 0.5 * (beta - alpha), sigma = theta / delta, rho_n = 1 / sigma;
     V.c1[0] = 0.0;  V.c2[0] = 1 / theta;
     for (int s = 1; s < 6; s++) { double rho_nm1 = rho_n; rho_n = 1.0 / (2.0 * sigma - rho_nm1); V.c1[s] = rho_n * rho_nm1; V.c2[s] = rho_n * 2.0 / delta; }
+    const bool l1jacobi = A.smoother == HPGMG_SMOOTHER_L1JACOBI;
+    V.jw = l1jacobi ? 1.0 : 2.0 / 3.0;                               /* jacobi.c */
+    V.l1 = l1jacobi ? hpgmg_l1inv_array(level) : NULL;
 
     /* slots: the vectors a cycle touches; identity (slot == vector id) when the level stays in global memory */
     int ids[COARSE_MAX_SLOTS], io[COARSE_MAX_SLOTS], n = 0;
@@ -628,7 +646,7 @@ extern "C" void hpgmg_coarse_cycle(mg_type *MG, int from, int mode_ftail, int ze
     const int s_dinv = add(VECTOR_DINV, 1), s_bi = add(VECTOR_BETA_I, 1), s_bj = add(VECTOR_BETA_J, 1), s_bk = add(VECTOR_BETA_K, 1);
     int kry[8] = { 0 };
     if (l == bottom) for (int q = 0; q < 8; q++) kry[q] = add(VECTORS_RESERVED + q, 0);     /* scratch of the solver: every one is written before it is read */
-    const size_t doubles = (size_t)n * V.L.volume;
+    const size_t doubles = (size_t)(n + (l1jacobi ? 1 : 0)) * V.L.volume;     /* + the resident copy of the L1 row inverse */
     const box_type *box0 = &level->my_boxes[0];
     const bool single = V.L.nboxes == 1 && box0->low.i == 0 && box0->low.j == 0 && box0->low.k == 0;
     V.smem_offset = -1;
@@ -638,6 +656,7 @@ extern "C" void hpgmg_coarse_cycle(mg_type *MG, int from, int mode_ftail, int ze
       V.nslots = n;  V.L.nvec = n;
       for (int q = 0; q < n; q++) { V.slot_id[q] = (unsigned char)ids[q]; V.slot_io[q] = (unsigned char)io[q]; }
       V.s_dinv = s_dinv;  V.s_bi = s_bi;  V.s_bj = s_bj;  V.s_bk = s_bk;
+      V.s_lam = l1jacobi ? n : s_dinv;
       S[l - from].temp = s_temp;  S[l - from].e = s_e;  S[l - from].R = s_R;
       if (l == bottom) {
         BottomIds I = { kry[0], kry[1], kry[2], kry[3], kry[4], kry[5], kry[6], kry[7], s_dinv, s_temp, s_bi, s_bj, s_bk };
@@ -649,6 +668,7 @@ extern "C" void hpgmg_coarse_cycle(mg_type *MG, int from, int mode_ftail, int ze
       stop = true;                                                    /* keep the resident set contiguous from the bottom */
       V.nslots = 0;
       V.s_dinv = VECTOR_DINV;  V.s_bi = VECTOR_BETA_I;  V.s_bj = VECTOR_BETA_J;  V.s_bk = VECTOR_BETA_K;
+      V.s_lam = l1jacobi ? -1 : VECTOR_DINV;
       S[l - from].temp = VECTOR_TEMP;  S[l - from].e = e_id;  S[l - from].R = R_id;
       if (l == bottom) A.bottom_ids = bottom_ids_identity();
       V.fast = 0;

@@ -175,6 +175,8 @@ struct hpgmg_device_level {
                                                    (hpgmg_note_vector_written: BLAS1, transfers, smoothers, uploads). */
   int   *restrict_map;                          /* device [nboxes][4]: coarse box and coarse cell of cell (0,0,0) of every box (smooth.cu: residual fused with restriction) */
   int    restrict_map_state;                    /* 0 not looked at yet, 1 available, -1 the level's restriction is not box-to-box on this GPU */
+  double *l1inv;                                /* default build, L1-Jacobi only: the L1 row inverse, [box][k][j][i] with the geometry of one
+                                                   slab vector (the vector map has no room for it); written by rebuild_operator_blackbox */
   double *tile_partials;                        /* scratch for dot/mean: one double per compute tile */
   blockCopy_type *tiles;                        /* device copy of level->my_blocks                  */
   int     ntiles;

@@ -310,6 +310,7 @@ extern "C" void hpgmg_device_level_destroy(level_type *level)
   free_fill_tables(D);
   if (D->low) CUDA_CHECK(cudaFree(D->low));
   if (D->restrict_map) CUDA_CHECK(cudaFree(D->restrict_map));
+  if (D->l1inv) hpgmg_rt_free(D->l1inv);
   if (D->tiles) CUDA_CHECK(cudaFree(D->tiles));
   if (D->tile_partials) CUDA_CHECK(cudaFree(D->tile_partials));
   free(D);

@@ -128,7 +128,14 @@ extern "C" const char *hpgmg_b200_backend(void) { return "cuda-sm_100a"; }
 extern "C" void *hpgmg_b200_stream(void) { require_init("stream"); return (void *)g_stream; }
 extern "C" int hpgmg_b200_device(void) { return g_device; }
 
-extern "C" void hpgmg_b200_set_smoother(int which) { g_smoother = which; }
+extern "C" void hpgmg_b200_set_smoother(int which)
+{
+  if (which != HPGMG_SMOOTHER_GSRB && which != HPGMG_SMOOTHER_CHEBY && which != HPGMG_SMOOTHER_JACOBI && which != HPGMG_SMOOTHER_L1JACOBI) {
+    fprintf(stderr, "hpgmg_b200_set_smoother: %d is not a smoother (0 GSRB, 1 Chebyshev, 2 Jacobi, 3 L1-Jacobi); keeping %d\n", which, g_smoother);
+    return;
+  }
+  g_smoother = which;
+}
 extern "C" int  hpgmg_b200_get_smoother(void) { return g_smoother; }
 extern "C" void hpgmg_b200_set_verbose(int on) { g_verbose = on; }
 extern "C" void hpgmg_b200_use_graphs(int on) { g_use_graphs = on; }

@@ -1,7 +1,8 @@
 /*
- * smooth.cu -- the operator-applying kernels: GSRB and Chebyshev smoothers, residual, apply_op and
- * the black-box diagonal rebuild.  Entry points mirror the reference one for one:
- *   smooth            operators/gsrb.c:24-132 (GSRB_OOP + GSRB_STRIDE2) | operators/chebyshev.c:8-100
+ * smooth.cu -- the operator-applying kernels: GSRB, Chebyshev, weighted Jacobi and L1-Jacobi smoothers, residual,
+ * apply_op and the black-box diagonal rebuild.  Entry points mirror the reference one for one:
+ *   smooth            operators/gsrb.c:24-132 (GSRB_OOP + GSRB_STRIDE2) | operators/chebyshev.c:8-100 |
+ *                     operators/jacobi.c (USE_JACOBI: w = 2/3, lambda = D^-1; USE_L1JACOBI: w = 1, lambda = L1 row inverse)
  *   residual          operators/residual.c:9-51
  *   apply_op          operators/apply_op.c:9-50
  *   rebuild_operator  operators.fv4.c:145-173, rebuild_operator_blackbox operators/rebuild.c:47-208
@@ -14,7 +15,8 @@
 #include "stencil.cuh"
 
 enum { OP_APPLY = 0, OP_RESIDUAL = 1, OP_GSRB = 2, OP_CHEBY = 3, OP_REBUILD = 4,
-       OP_RESRES = 5 };   /* residual fused with the cell restriction that follows it in MGVCycle (k-marching kernel only) */
+       OP_RESRES = 5,     /* residual fused with the cell restriction that follows it in MGVCycle (k-marching kernel only) */
+       OP_JACOBI = 6 };   /* one Jacobi sweep: x + (weight*lambda)*(rhs - A x) */
 
 /* The Helmholtz build (-DUSE_HELMHOLTZ, as in the reference: operators.fv4.c:56-85): A x = a*alpha*x - b*h2inv*(...).  The
  * reference subtracts (b*h2inv)*(...) from a*alpha*x; fv4_apply_op returns (-b*h2inv)*(...), the exact negation, and
@@ -34,6 +36,9 @@ struct StencilArgs {
   int x_id, rhs_id, out_id, xm1_id;
   double a, b, h2inv;
   double c1, c2;           /* Chebyshev */
+  double weight;           /* Jacobi: 2/3 (lambda = Dinv) or 1 (lambda = L1 row inverse) */
+  const double *lam;       /* Jacobi: lambda of box b, cell (0,0,0), at lam + b * lam_bstride */
+  size_t lam_bstride;
   int sweep;               /* GSRB sweep number s (colour) */
   int reverse;             /* march k downwards (TMA kernel only; same result) */
   int diag;                /* TMA GSRB kernel: form Dinv = 1/Aii in registers from the face coefficients wherever the stencil
@@ -91,6 +96,10 @@ __global__ void __launch_bounds__(256) stencil_generic_kernel(const StencilArgs 
     const double dinv = L.vec(box, VECTOR_DINV)[ijk];
     const double rhs = L.vec(box, A.rhs_id)[ijk];
     L.vec(box, A.out_id)[ijk] = xn + A.c1 * (xn - xm1) + A.c2 * dinv * (rhs - Ax);
+  } else if (OP == OP_JACOBI) {                          /* jacobi.c: x_n + weight*lambda*(rhs - Ax_n), left to right */
+    const double lam = A.lam[(size_t)box * A.lam_bstride + ijk];
+    const double rhs = L.vec(box, A.rhs_id)[ijk];
+    L.vec(box, A.out_id)[ijk] = x[0] + (A.weight * lam) * (rhs - Ax);
   } else if (OP == OP_REBUILD) {
     /* rebuild.c:127-133: x is a 0/1 colouring; Aii += x*Ax, sumAbsAij += |(1-x)*Ax| */
     double *Aii = L.vec(box, A.out_id) + ijk;
@@ -243,6 +252,11 @@ __global__ void __launch_bounds__(256) stencil_pair_kernel(const StencilArgs A)
   if (OP == OP_APPLY) { *out = make_double2(Ax0, Ax1); return; }
   const double2 rhs2 = *reinterpret_cast<const double2 *>(L.vec(box, A.rhs_id) + ijk);
   if (OP == OP_RESIDUAL) { *out = make_double2(rhs2.x - Ax0, rhs2.y - Ax1); return; }
+  if (OP == OP_JACOBI) {
+    const double2 lam2 = *reinterpret_cast<const double2 *>(A.lam + (size_t)box * A.lam_bstride + ijk);
+    *out = make_double2(x[0] + (A.weight * lam2.x) * (rhs2.x - Ax0), x[1] + (A.weight * lam2.y) * (rhs2.y - Ax1));
+    return;
+  }
   const double2 dinv2 = *reinterpret_cast<const double2 *>(L.vec(box, VECTOR_DINV) + ijk);   /* OP_CHEBY */
   const double2 xm = *reinterpret_cast<const double2 *>(L.vec(box, A.xm1_id) + ijk);
   *out = make_double2(x[0] + A.c1 * (x[0] - xm.x) + A.c2 * dinv2.x * (rhs2.x - Ax0),
@@ -306,6 +320,7 @@ static void launch_box(level_type *level, const StencilArgs &S, const int write_
   A.L = D->L;  A.low = D->low;  A.ranges = T.ranges;  A.copies = T.copies;  A.bc = T.bc;
   A.x_id = S.x_id;  A.rhs_id = S.rhs_id;  A.out_id = S.out_id;  A.sweep = S.sweep;  A.write_ghosts = write_ghosts;
   A.b = S.b;  A.h2inv = 1.0 / (level->h * level->h);  A.c1 = S.c1;  A.c2 = S.c2;
+  A.weight = S.weight;  A.lam = S.lam;  A.lam_bstride = S.lam_bstride;
   typedef BoxCfg<N, TI, TJ, TK> C;
   LAUNCH((stencil_box_kernel<OP, N, TI, TJ, TK>), D->L.nboxes * C::TILES, C::NT, 0, A);
 }
@@ -505,6 +520,65 @@ static void smooth_chebyshev(level_type *level, int x_id, int rhs_id, double a, 
   }
 }
 
+/* The L1 row inverse of a level in the default build (rebuild_operator_blackbox stores it only while L1-Jacobi is selected).
+ * The reference fixes its smoother at compile time, so it always has the vector; here a level built for another smoother
+ * cannot be smoothed with L1-Jacobi: recomputing the array here would overwrite VECTOR_TEMP and VECTOR_E, which hold live
+ * data in the middle of a cycle. */
+extern "C" double *hpgmg_l1inv_array(level_type *level)
+{
+  double *p = HPGMG_DEV(level)->l1inv;
+  if (!p && level->num_my_boxes > 0) {
+    fprintf(stderr, "hpgmg_b200: the level of h=%e has no L1 row inverse: L1-Jacobi was not the selected smoother when its operator was "
+                    "built. Select HPGMG_SMOOTHER_L1JACOBI (hpgmg_b200_set_smoother) before rebuild_operator / MGBuild.\n", level->h);
+    fflush(stderr);
+    exit(1);
+  }
+  return p;
+}
+
+extern "C" void hpgmg_download_l1inv(level_type *level, int box, double *host)
+{
+#ifdef VECTOR_L1INV
+  hpgmg_download_box_vector(level, box, VECTOR_L1INV, host);
+#else
+  const double *p = hpgmg_l1inv_array(level);
+  hpgmg_rt_copy_d2h(host, p + (size_t)box * level->box_volume, (size_t)level->box_volume * sizeof(double));
+  hpgmg_rt_sync();
+#endif
+}
+
+/* weight and lambda of the selected Jacobi variant (jacobi.c): USE_JACOBI 2/3 and Dinv, USE_L1JACOBI 1 and the L1 row inverse */
+static void jacobi_operands(level_type *level, StencilArgs &A)
+{
+  const DLevel &L = dl_of(level);
+  if (hpgmg_rt_smoother() == HPGMG_SMOOTHER_L1JACOBI) {
+    A.weight = 1.0;
+#ifdef VECTOR_L1INV
+    A.lam = L.vec(0, VECTOR_L1INV);  A.lam_bstride = (size_t)L.nvec * L.volume;
+#else
+    A.lam = hpgmg_l1inv_array(level) + L.origin;  A.lam_bstride = (size_t)L.volume;
+#endif
+  } else {
+    A.weight = 2.0 / 3.0;
+    A.lam = L.vec(0, VECTOR_DINV);  A.lam_bstride = (size_t)L.nvec * L.volume;
+  }
+}
+
+static void smooth_jacobi(level_type *level, int x_id, int rhs_id, double a, double b)
+{
+  StencilArgs J = {};
+  jacobi_operands(level, J);
+  for (int s = 0; s < 6; s++) {                      /* NUM_SMOOTHS=6 (operators.fv4.c:176-195); x -> TEMP -> x like GSRB */
+    StencilArgs A = J;
+    A.x_id = (s & 1) == 0 ? x_id : VECTOR_TEMP;
+    A.out_id = (s & 1) == 0 ? VECTOR_TEMP : x_id;
+    A.rhs_id = rhs_id;  A.a = a;  A.b = b;
+    fill_and_stencil<OP_JACOBI>(level, A, 0);
+  }
+}
+
+static int is_jacobi(const int smoother) { return smoother == HPGMG_SMOOTHER_JACOBI || smoother == HPGMG_SMOOTHER_L1JACOBI; }
+
 /* one sweep kernel of the current smoother alone (no ghost fill): what bench.py times for the roofline line */
 extern "C" void hpgmg_b200_smoother_sweep(level_type *level, int src_id, int dst_id, int rhs_id, double a, double b, int s)
 {
@@ -512,6 +586,11 @@ extern "C" void hpgmg_b200_smoother_sweep(level_type *level, int src_id, int dst
     double c1[6], c2[6];
     chebyshev_coefficients(level, c1, c2);
     chebyshev_sweep(level, src_id, dst_id, rhs_id, a, b, c1[s % 6], c2[s % 6], 0);
+  } else if (is_jacobi(hpgmg_rt_smoother())) {
+    StencilArgs A = {};
+    jacobi_operands(level, A);
+    A.x_id = src_id;  A.rhs_id = rhs_id;  A.out_id = dst_id;  A.a = a;  A.b = b;
+    launch_stencil<OP_JACOBI>(level, A);
   } else hpgmg_b200_gsrb_sweep(level, src_id, dst_id, rhs_id, a, b, s);
 }
 
@@ -520,12 +599,13 @@ extern "C" void smooth(level_type *level, int x_id, int rhs_id, double a, double
   ProfileScope prof_(&level->timers.smooth);
   hpgmg_note_vector_written(level, x_id);
   if (hpgmg_rt_smoother() == HPGMG_SMOOTHER_CHEBY) smooth_chebyshev(level, x_id, rhs_id, a, b);
+  else if (is_jacobi(hpgmg_rt_smoother())) smooth_jacobi(level, x_id, rhs_id, a, b);
   else smooth_gsrb(level, x_id, rhs_id, a, b);
 }
 
 /* ------------------------------------------------------------------------------------------ */
 /* D^-1 and the Gershgorin bound on lambda_max(D^-1 A) from the operator alone (rebuild.c:47-208) */
-__global__ void rebuild_finish_kernel(const DLevel L, const int *low, int Aii_id, int sum_id, double a, double b, double h2inv, double *eig_slot)
+__global__ void rebuild_finish_kernel(const DLevel L, const int *low, int Aii_id, int sum_id, double a, double b, double h2inv, double *eig_slot, double *l1inv)
 {
   PDL_WAIT();
   const int n = L.dim;
@@ -545,6 +625,7 @@ __global__ void rebuild_finish_kernel(const DLevel L, const int *low, int Aii_id
       if (Di > local) local = Di;
       if (Aii[0] >= 1.5 * sumAbs[0]) sumAbs[0] = 1.0 / (Aii[0]);
       else                           sumAbs[0] = 1.0 / (Aii[0] + 0.5 * sumAbs[0]);
+      if (l1inv) l1inv[(size_t)box * L.volume + L.origin + ijk] = sumAbs[0];    /* the L1-Jacobi lambda, kept (default build) */
       Aii[0] = 1.0 / Aii[0];
     }
   }
@@ -580,10 +661,19 @@ extern "C" void rebuild_operator_blackbox(level_type *level, double a, double b,
   double *slot = hpgmg_rt_scalar_slots() + HPGMG_SLOT_SCRATCH;
   CUDA_CHECK(cudaMemsetAsync(slot, 0, sizeof(double), g_stream));
   const DLevel &L = dl_of(level);
+  double *l1inv = NULL;
+#ifndef VECTOR_L1INV
+  /* the default vector map has no room for the L1 row inverse: an array of the level, made when L1-Jacobi is selected
+   * and refreshed by every later rebuild */
+  hpgmg_device_level *D = HPGMG_DEV(level);
+  if (!D->l1inv && L.nboxes > 0 && hpgmg_rt_smoother() == HPGMG_SMOOTHER_L1JACOBI)
+    D->l1inv = (double *)hpgmg_rt_alloc_zero((size_t)L.nboxes * L.volume * sizeof(double));
+  l1inv = D->l1inv;
+#endif
   if (L.nboxes > 0) {
     const int cells = L.dim * L.dim * L.dim;
     dim3 grid((cells + 255) / 256 > 1024 ? 1024 : (cells + 255) / 256, L.nboxes);
-    LAUNCH(rebuild_finish_kernel, grid, 256, 0, L, HPGMG_DEV(level)->low, Aii_id, sum_id, a, b, 1.0 / (level->h * level->h), slot);
+    LAUNCH(rebuild_finish_kernel, grid, 256, 0, L, HPGMG_DEV(level)->low, Aii_id, sum_id, a, b, 1.0 / (level->h * level->h), slot, l1inv);
   }
   double eig = 0.0;
   hpgmg_rt_read_scalars(&eig, HPGMG_SLOT_SCRATCH, 1);

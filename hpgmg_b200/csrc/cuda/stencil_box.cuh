@@ -13,7 +13,7 @@
  * The values are those the separate fill would have left in the ghost cells (same expressions, same operands), so
  * the result is bit-identical; the ghost cells in HBM are simply not needed any more (residual / apply_op still
  * write them, because callers of the reference API may look at them: residual.c:15-16 fills x in place).
- * gsrb.c:41-129, chebyshev.c:51-97, residual.c:18-49, apply_op.c:18-47; arithmetic = fv4_apply_op_at (stencil.cuh).
+ * gsrb.c:41-129, chebyshev.c:51-97, jacobi.c, residual.c:18-49, apply_op.c:18-47; arithmetic = fv4_apply_op_at (stencil.cuh).
  *
  * Face coefficients, rhs and Dinv are read straight from global memory at compile-time strides (the box size is a
  * template parameter), i.e. as loads at immediate offsets through L1.  Rows of the staged tile are stored as they are
@@ -57,6 +57,9 @@ struct BoxArgs {
   int sweep;                                                       /* GSRB colour */
   int write_ghosts;                                                /* also leave the ghost values in HBM (residual, apply_op) */
   double b, h2inv, c1, c2;
+  double weight;                                                   /* Jacobi: lambda of box b at lam + b * lam_bstride (cell 0,0,0) */
+  const double *lam;
+  size_t lam_bstride;
 };
 
 template <int OP, int N, int TI, int TJ, int TK>
@@ -144,6 +147,9 @@ __global__ void __launch_bounds__((TI / 2) * TJ * TK) stencil_box_kernel(const B
       const double2 rhs2 = *reinterpret_cast<const double2 *>(L.vec(box, A.rhs_id) + cell);
       if constexpr (OP == OP_RESIDUAL) {
         *out = make_double2(rhs2.x - Ax[0], rhs2.y - Ax[1]);
+      } else if constexpr (OP == OP_JACOBI) {                        /* jacobi.c: x_n + weight*lambda*(rhs - Ax_n), left to right */
+        const double2 lam2 = *reinterpret_cast<const double2 *>(A.lam + (size_t)box * A.lam_bstride + cell);
+        *out = make_double2(ts[0] + (A.weight * lam2.x) * (rhs2.x - Ax[0]), ts[1] + (A.weight * lam2.y) * (rhs2.y - Ax[1]));
       } else {                                                       /* OP_CHEBY (chebyshev.c:90) */
         const double2 dinv2 = *reinterpret_cast<const double2 *>(L.vec(box, VECTOR_DINV) + cell);
         const double2 xm = *out;                                     /* x_{n-1} aliases x_{n+1} (chebyshev.c:75-80) */

@@ -2,8 +2,8 @@
  * stencil_tma.cuh -- the operator kernels for boxes >= 32^3, Blackwell version: 2.5-D blocking with the halo
  * tiles staged in shared memory by the TMA engine.
  *
- * GSRB / Chebyshev / residual / apply_op on a TI x TJ column of cells marching along k (gsrb.c:41-129,
- * chebyshev.c:51-97, residual.c:18-49, apply_op.c:18-47 with the macro of operators.fv4.c:87-114); the
+ * GSRB / Chebyshev / Jacobi / residual / apply_op on a TI x TJ column of cells marching along k (gsrb.c:41-129,
+ * chebyshev.c:51-97, jacobi.c, residual.c:18-49, apply_op.c:18-47 with the macro of operators.fv4.c:87-114); the
  * arithmetic is fv4_apply_op_at, shared with every other kernel, hence the same bits.  Around the arithmetic:
  *
  *  - staging: one elected thread issues cp.async.bulk.tensor (TMA) copies of whole (TI+4) x rows tiles
@@ -13,7 +13,7 @@
  *  - layout: rows are stored as they are in memory (TMA cannot split parities).  GSRB: bank conflicts of the stride-2
  *    red-black accesses are avoided by the lane mapping: a thread owns an i-pair (one active cell per sweep), even lanes work
  *    on row r, odd lanes on row r+1 of a row pair; the active cells of the two rows have opposite i-parity, so the 16 lanes of
- *    a half-warp touch 16 distinct 8-byte banks.  Residual / Chebyshev / apply_op: a thread owns the j-pair (i,j), (i,j+1);
+ *    a half-warp touch 16 distinct 8-byte banks.  Residual / Chebyshev / Jacobi / apply_op: a thread owns the j-pair (i,j), (i,j+1);
  *    lanes are consecutive cells of a row (conflict-free), and the two stencils share their common operands (pure loads
  *    merged by the compiler: 85 LDS per cell pair instead of 110).
  *  - addressing: a lane keeps ONE 32-bit shared address per ring slot; every stencil operand is a load at a compile-time
@@ -199,7 +199,9 @@ stencil_tma_kernel(const StencilArgs A, const __grid_constant__ CUtensorMap map_
     const int j = j0 + r;
     const int cell = (i0 + ci_lane) + j * jS;                      /* GSRB: pair (2p, 2p+1) of row j; JP: cells (lane, j), (lane, j+1); plane 0 */
     const double *g_rhs = (OP == OP_APPLY) ? nullptr : L.vec(box, A.rhs_id) + cell;
-    const double *g_dinv = (OP == OP_GSRB || OP == OP_CHEBY) ? L.vec(box, VECTOR_DINV) + cell : nullptr;
+    /* the point-wise inverse: Dinv, or lambda of a Jacobi sweep (Dinv or the L1 row inverse, which need not be in the slab) */
+    const double *g_dinv = (OP == OP_GSRB || OP == OP_CHEBY) ? L.vec(box, VECTOR_DINV) + cell
+                         : (OP == OP_JACOBI) ? A.lam + (size_t)box * A.lam_bstride + cell : nullptr;
     const double *g_xm1 = (OP == OP_CHEBY) ? L.vec(box, A.xm1_id) + cell : nullptr;
     double *g_out = L.vec(box, A.out_id) + cell;
     double *c_out = nullptr;                                         /* OP_RESRES: the coarse cell under (lane, j), plane 0 of the coarse box */
@@ -226,11 +228,11 @@ stencil_tma_kernel(const StencilArgs A, const __grid_constant__ CUtensorMap map_
     const int gk_hi = A.dom[2] - 3;
 #define PLANE_NEEDS_DINV(kk) (!(OP == OP_GSRB) || !tile_inner || gk0 + (kk) < 2 || gk0 + (kk) > gk_hi)
 
-    /* point-wise operands (rhs, Dinv, x_{n-1}) are read one plane ahead into registers */
+    /* point-wise operands (rhs, Dinv or lambda, x_{n-1}) are read one plane ahead into registers */
     double2 rhs_n = make_double2(0.0, 0.0), dinv_n = make_double2(0.0, 0.0), xm_n = make_double2(0.0, 0.0);
 #define LOAD_PAIR(ptr, kk) (JP ? make_double2((ptr)[(kk) * kS], (ptr)[(kk) * kS + jS]) : *reinterpret_cast<const double2 *>((ptr) + (kk) * kS))
     if (OP != OP_APPLY) rhs_n = LOAD_PAIR(g_rhs, kf);
-    if ((OP == OP_GSRB || OP == OP_CHEBY) && PLANE_NEEDS_DINV(kf)) dinv_n = LOAD_PAIR(g_dinv, kf);
+    if ((OP == OP_GSRB || OP == OP_CHEBY || OP == OP_JACOBI) && PLANE_NEEDS_DINV(kf)) dinv_n = LOAD_PAIR(g_dinv, kf);
     if (OP == OP_CHEBY) xm_n = LOAD_PAIR(g_xm1, kf);
 
     mbar_wait(bar0, phasebits & 1u);                               /* step 0's planes */
@@ -257,7 +259,7 @@ stencil_tma_kernel(const StencilArgs A, const __grid_constant__ CUtensorMap map_
       const double2 rhs2 = rhs_n, dinv2 = dinv_n, xm2 = xm_n;
       if (more) {
         if (OP != OP_APPLY) rhs_n = LOAD_PAIR(g_rhs, k + dir);
-        if ((OP == OP_GSRB || OP == OP_CHEBY) && PLANE_NEEDS_DINV(k + dir)) dinv_n = LOAD_PAIR(g_dinv, k + dir);
+        if ((OP == OP_GSRB || OP == OP_CHEBY || OP == OP_JACOBI) && PLANE_NEEDS_DINV(k + dir)) dinv_n = LOAD_PAIR(g_dinv, k + dir);
         if (OP == OP_CHEBY) xm_n = LOAD_PAIR(g_xm1, k + dir);
       }
 
@@ -313,6 +315,10 @@ stencil_tma_kernel(const StencilArgs A, const __grid_constant__ CUtensorMap map_
           if (OP == OP_APPLY) v = Ax;
           else if (OP == OP_RESIDUAL) { v = (c ? rhs2.y : rhs2.x) - Ax; const double f = fabs(v); if (f > vmax) vmax = f; }
           else if (OP == OP_RESRES) v = (c ? rhs2.y : rhs2.x) - Ax;
+          else if (OP == OP_JACOBI) {                                /* jacobi.c: x_n + weight*lambda*(rhs - Ax_n), left to right */
+            const double xn = PX(0, 0, 0);
+            v = xn + (A.weight * (c ? dinv2.y : dinv2.x)) * ((c ? rhs2.y : rhs2.x) - Ax);
+          }
           else {                                                     /* OP_CHEBY, chebyshev.c:90 */
             const double xn = PX(0, 0, 0);
             v = xn + A.c1 * (xn - (c ? xm2.y : xm2.x)) + A.c2 * (c ? dinv2.y : dinv2.x) * ((c ? rhs2.y : rhs2.x) - Ax);

@@ -106,6 +106,9 @@ void   hpgmg_comm_exchange_wait(level_type *level, communicator_type *C);
 void   hpgmg_comm_transfer(level_type *level_send, communicator_type *Cs, level_type *level_recv, communicator_type *Cr, int tag);
 void   hpgmg_comm_transfer_wait(level_type *level_send, communicator_type *Cs, level_type *level_recv, communicator_type *Cr);
 
+/* default build: the L1 row inverse of a level (smooth.cu); a fatal error if the level was built without it */
+double *hpgmg_l1inv_array(level_type *level);
+
 /* coarse end of the cycle as one single-block kernel (coarse.cu): levels from..bottom */
 int  hpgmg_coarse_chain_eligible(mg_type *MG, int from);
 void hpgmg_coarse_cycle(mg_type *MG, int from, int mode_ftail, int zero_bottom, int e_id, int R_id, double a, double b);

@@ -30,10 +30,15 @@ void hpgmg_b200_sync(void);                      /* drain the compute stream    
 const char *hpgmg_b200_backend(void);            /* "cuda-sm_100a": there is no other backend    */
 
 /* ---- variant selection ----------------------------------------------------------------------
- * The reference picks the smoother at compile time (-DUSE_GSRB | -DUSE_CHEBY,
- * operators.fv4.c:176-195, hpgmgconf.py:114-126).  Here it is a runtime switch. */
-#define HPGMG_SMOOTHER_GSRB  0                   /* 3x red-black = 6 sweeps   (NUM_SMOOTHS 3)   */
-#define HPGMG_SMOOTHER_CHEBY 1                   /* one degree-6 polynomial   (CHEBYSHEV_DEGREE) */
+ * The reference picks the smoother at compile time (-DUSE_GSRB | -DUSE_CHEBY | -DUSE_JACOBI | -DUSE_L1JACOBI,
+ * operators.fv4.c:176-195, hpgmgconf.py:114-126).  Here it is a runtime switch.  Any other value is refused
+ * (a message on stderr; the current selection stays).
+ * L1-Jacobi needs the L1 row inverse of every level, which rebuild_operator_blackbox stores only while it is the
+ * selected smoother: select it before rebuild_operator / MGBuild.  Smoothing a level without it is a fatal error. */
+#define HPGMG_SMOOTHER_GSRB     0                /* 3x red-black = 6 sweeps   (NUM_SMOOTHS 3)   */
+#define HPGMG_SMOOTHER_CHEBY    1                /* one degree-6 polynomial   (CHEBYSHEV_DEGREE) */
+#define HPGMG_SMOOTHER_JACOBI   2                /* 6 weighted Jacobi sweeps, w = 2/3, D^-1      (operators/jacobi.c) */
+#define HPGMG_SMOOTHER_L1JACOBI 3                /* 6 L1-Jacobi sweeps, w = 1, 1/(Aii + sum|Aij|/2) (operators/jacobi.c) */
 void hpgmg_b200_set_smoother(int which);
 int  hpgmg_b200_get_smoother(void);
 
@@ -79,6 +84,11 @@ double hpgmg_last_richardson_order(void);
  * compute stream so they are ordered with the operators. */
 void hpgmg_download_box_vector(level_type *level, int box, int id, double *host);
 void hpgmg_upload_box_vector(level_type *level, int box, int id, const double *host);
+/* The L1 row inverse L1-Jacobi smooths with (rebuild.c: 1/Aii or 1/(Aii + sum|Aij|/2)), in the same layout.  The
+ * Helmholtz build reads VECTOR_L1INV; the default build keeps it outside the vector map, in an array of the level
+ * that exists only if L1-Jacobi was selected when the operator was rebuilt (otherwise: a fatal error).  Ghost cells
+ * are not meaningful. */
+void hpgmg_download_l1inv(level_type *level, int box, double *host);
 void *hpgmg_b200_host_alloc_pinned(size_t bytes);
 void  hpgmg_b200_host_free_pinned(void *p);
 
@@ -116,7 +126,8 @@ void   hpgmg_b200_profiler_start(void);
 void   hpgmg_b200_profiler_stop(void);
 /* exactly one GSRB sweep kernel of smooth() (gsrb.c:41-129), without the ghost fill: dst = sweep s of src */
 void   hpgmg_b200_gsrb_sweep(level_type *level, int src_id, int dst_id, int rhs_id, double a, double b, int s);
-/* the same for whichever smoother is selected (Chebyshev: step s of chebyshev.c:51-97, x_{n-1} = dst) */
+/* the same for whichever smoother is selected (Chebyshev: step s of chebyshev.c:51-97, x_{n-1} = dst; Jacobi and
+ * L1-Jacobi: one sweep of jacobi.c, s is ignored) */
 void   hpgmg_b200_smoother_sweep(level_type *level, int src_id, int dst_id, int rhs_id, double a, double b, int s);
 
 /* ---- multi-GPU plumbing -----------------------------------------------------------------------
