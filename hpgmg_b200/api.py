@@ -26,6 +26,7 @@ BC_PERIODIC, BC_DIRICHLET = 0, 1
 STENCIL_SHAPE_BOX, STENCIL_SHAPE_STAR, STENCIL_SHAPE_NO_CORNERS = 0, 1, 2
 RESTRICT_CELL, RESTRICT_FACE_I, RESTRICT_FACE_J, RESTRICT_FACE_K = 0, 1, 2, 3
 SMOOTHER_GSRB, SMOOTHER_CHEBY, SMOOTHER_JACOBI, SMOOTHER_L1JACOBI = 0, 1, 2, 3    # include/hpgmg_b200.h
+BOTTOM_BICGSTAB, BOTTOM_CG = 0, 1                                                 # include/hpgmg_b200.h
 
 ALLGATHER_FN = C.CFUNCTYPE(None, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p)
 BARRIER_FN = C.CFUNCTYPE(None, C.c_void_p)
@@ -42,6 +43,7 @@ SIGNATURES = {
     "hpgmg_b200_init": (_I, [_I]), "hpgmg_b200_finalize": (_V, []), "hpgmg_b200_sync": (_V, []),
     "hpgmg_b200_backend": (C.c_char_p, []),
     "hpgmg_b200_set_smoother": (_V, [_I]), "hpgmg_b200_get_smoother": (_I, []),
+    "hpgmg_b200_set_bottom_solver": (_V, [_I]), "hpgmg_b200_get_bottom_solver": (_I, []),
     "hpgmg_b200_set_verbose": (_V, [_I]), "hpgmg_b200_use_graphs": (_V, [_I]),
     "hpgmg_b200_profile_operators": (_V, [_I]), "hpgmg_b200_use_coarse_kernel": (_V, [_I]), "hpgmg_b200_coarse_profile": (_V, [_I, C.c_void_p]), "hpgmg_b200_coarse_levels_in_smem": (_V, [_I]), "hpgmg_b200_set_layout_only": (_V, [_I]),
     "hpgmg_download_box_vector": (_V, [_LP, _I, _I, C.c_void_p]),
@@ -175,12 +177,13 @@ class Hierarchy:
     """The reference driver's setup sequence (hpgmg-fv.c:280-308) as an object.
 
     level_h -> initialize_problem -> rebuild_operator -> MGBuild, for `hpgmg-fv <log2_box_dim>
-    <target_boxes_per_rank>` on `num_ranks` ranks (this process being `my_rank`).
+    <target_boxes_per_rank>` on `num_ranks` ranks (this process being `my_rank`).  `smoother`, `bottom_solver`, `verbose`
+    and `use_graphs` are process-wide selections of the library; they are set only when `library` is None.
     """
 
     def __init__(self, log2_box_dim, target_boxes_per_rank, my_rank=0, num_ranks=1, a=0.0, b=1.0,
                  smoother=SMOOTHER_GSRB, verbose=False, use_graphs=True, build_operator=True, library=None,
-                 bc=BC_DIRICHLET, vectors=None):
+                 bc=BC_DIRICHLET, vectors=None, bottom_solver=BOTTOM_BICGSTAB):
         self.L = library or lib()
         self.a, self.b = float(a), float(b)
         self.box_dim, self.boxes_in_i = problem_size(log2_box_dim, target_boxes_per_rank, num_ranks)
@@ -189,6 +192,7 @@ class Hierarchy:
         if library is None:
             self.L.hpgmg_b200_set_verbose(1 if verbose else 0)
             self.L.hpgmg_b200_set_smoother(smoother)
+            self.L.hpgmg_b200_set_bottom_solver(bottom_solver)
             self.L.hpgmg_b200_use_graphs(1 if use_graphs else 0)
         self._level_buf = level_type()
         self.level_h = C.pointer(self._level_buf)

@@ -1,5 +1,6 @@
 /*
- * bicgstab.cu -- the bottom solver as ONE single-thread-block kernel.
+ * bicgstab.cu -- the bottom solver as ONE single-thread-block kernel: BiCGStab (bicgstab_kernel) or, when
+ * HPGMG_BOTTOM_CG is selected, D^-1-preconditioned CG (cg_kernel, the restatement of solvers.c:cg_host_driven).
  *
  * Restates solvers/bicgstab.c:14-97 (diagonally right-preconditioned BiCGStab, <=200 iterations,
  * stop when ||s||inf or ||r||inf < rtol*||r0||inf, exact-zero breakdown tests).  In the reference
@@ -20,10 +21,17 @@ __global__ void __launch_bounds__(BOTTOM_THREADS) bicgstab_kernel(const BottomAr
   __shared__ double red[36];
   bicgstab_solve(A, prod, red);
 }
+__global__ void __launch_bounds__(BOTTOM_THREADS) cg_kernel(const BottomArgs A)
+{
+  PDL_WAIT();
+  __shared__ double prod[BOTTOM_MAX_CELLS];
+  __shared__ double red[36];
+  cg_solve(A, prod, red);
+}
 
-/* Returns 1 if the solve was enqueued on the device, 0 if the level is not eligible (more than one
- * box on this rank, other ranks involved, a periodic problem that needs mean subtraction, or a box
- * larger than the kernel's shared-memory staging) and the caller must use the host-driven loop. */
+/* Returns 1 if the solve (of the selected bottom solver) was enqueued on the device, 0 if the level is not eligible (more
+ * than one box on this rank, other ranks involved, a periodic problem that needs mean subtraction, or a box larger than the
+ * kernel's shared-memory staging) and the caller must use the host-driven loop.  Eligibility does not depend on the solver. */
 /* side-effect free: would hpgmg_bicgstab_device() take this level?  (mg.c uses it to decide whether a solve can be
  * recorded into a CUDA graph: the host-driven fallback synchronises on every dot / norm) */
 extern "C" int hpgmg_bicgstab_device_eligible(const level_type *level)
@@ -56,7 +64,8 @@ extern "C" int hpgmg_bicgstab_device(level_type *level, int x_id, int R_id, doub
   A.h2inv = 1.0 / (level->h * level->h);
   A.rtol = rtol;
   A.iters = hpgmg_rt_scalar_slots() + HPGMG_SLOT_KRYLOV;
-  LAUNCH(bicgstab_kernel, 1, BOTTOM_THREADS, 0, A);
+  if (hpgmg_rt_bottom_solver() == HPGMG_BOTTOM_CG) LAUNCH(cg_kernel, 1, BOTTOM_THREADS, 0, A);
+  else                                             LAUNCH(bicgstab_kernel, 1, BOTTOM_THREADS, 0, A);
   return 1;
 }
 

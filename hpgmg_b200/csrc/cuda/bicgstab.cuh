@@ -1,6 +1,6 @@
 /*
- * bicgstab.cuh -- device body of the single-thread-block BiCGStab (see bicgstab.cu), shared with the
- * coarse-grid cycle kernel (coarse.cu).
+ * bicgstab.cuh -- device bodies of the single-thread-block bottom solvers, BiCGStab and CG (see bicgstab.cu), shared with
+ * the coarse-grid cycle kernel (coarse.cu).
  */
 #ifndef HPGMG_B200_BICGSTAB_CUH
 #define HPGMG_B200_BICGSTAB_CUH
@@ -262,6 +262,125 @@ __device__ static void bicgstab_solve(const BottomArgs &A, double *prod, double 
     if (isinf(beta)) { failed = true; break; }
     b_add_chain(C, TEMP, 1.0, p, -omega, Ap, p, 1.0, r, beta);      /* TEMP = p - omega Ap; p = r + beta TEMP */
     r_dot_r0 = r_dot_r0_new;
+  }
+  if (threadIdx.x == 0) atomicAdd(A.iters, (double)j);
+}
+
+/* ---- CG (solvers/cg.c) ------------------------------------------------------------------------------------------------ */
+/* the sum of C.prod[0..cells) by ONE thread in linear cell order, after the barrier that publishes the products (b_dot's order) */
+__device__ static double b_sum_staged(BottomCtx &C)
+{
+  __syncthreads();
+  const int slot = 32 + 2 * C.flip;
+  if (threadIdx.x == 0) {
+    double s = 0.0;
+    for (int q = 0; q < C.cells; q++) s += C.prod[q];
+    C.red[slot] = s;
+  }
+  __syncthreads();
+  C.flip ^= 1;
+  return C.red[slot];
+}
+/* c = sa*a + sb*b */
+__device__ static void b_add(const BottomCtx &C, const int c_id, const double sa, const int a_id, const double sb, const int b_id)
+{
+  const DLevel &L = C.A.L;
+  double *c = L.vec(0, c_id);
+  const double *a = L.vec(0, a_id), *b = L.vec(0, b_id);
+  for (int q = threadIdx.x; q < C.cells; q += blockDim.x) {
+    const int ijk = C.cell_offset(q);
+    c[ijk] = sa * a[ijk] + sb * b[ijk];
+  }
+  __syncthreads();
+}
+/* out = A in, returns dot(out, in): the products are staged in the pass that produces out */
+__device__ static double b_apply_dot(BottomCtx &C, const int out_id, const int in_id)
+{
+  b_fill_ghosts(C, in_id);
+  const DLevel &L = C.A.L;
+  const double *x = L.vec(0, in_id), *bi = L.vec(0, C.A.ids.beta_i), *bj = L.vec(0, C.A.ids.beta_j), *bk = L.vec(0, C.A.ids.beta_k);
+  double *out = L.vec(0, out_id);
+  for (int c = threadIdx.x; c < C.cells; c += blockDim.x) {
+    const int ijk = C.cell_offset(c);
+    const double Ax = fv4_apply_op(x + ijk, bi + ijk, bj + ijk, bk + ijk, C.jS, C.kS, C.A.b, C.A.h2inv);
+    out[ijk] = Ax;
+    C.prod[c] = Ax * x[ijk];
+  }
+  return b_sum_staged(C);
+}
+/* z = s*d*r, returns dot(r, z): the products are staged in the pass that writes z */
+__device__ static double b_mul_dot(BottomCtx &C, const int z_id, const double s, const int d_id, const int r_id)
+{
+  const DLevel &L = C.A.L;
+  double *z = L.vec(0, z_id);
+  const double *d = L.vec(0, d_id), *r = L.vec(0, r_id);
+  for (int q = threadIdx.x; q < C.cells; q += blockDim.x) {
+    const int ijk = C.cell_offset(q);
+    const double v = s * d[ijk] * r[ijk];
+    z[ijk] = v;
+    C.prod[q] = r[ijk] * v;
+  }
+  return b_sum_staged(C);
+}
+/* the start of CG in one pass: r = 1.0*r0; z = 1.0*d*r; p = 1.0*z; returns dot(r, z) and, in *norm_r, max |r| */
+__device__ static double b_cg_start(BottomCtx &C, const int r_id, const int z_id, const int p_id, const int r0_id, const int d_id, double *norm_r)
+{
+  const DLevel &L = C.A.L;
+  double *r = L.vec(0, r_id), *z = L.vec(0, z_id), *p = L.vec(0, p_id);
+  const double *r0 = L.vec(0, r0_id), *d = L.vec(0, d_id);
+  double m = 0.0;
+  for (int q = threadIdx.x; q < C.cells; q += blockDim.x) {
+    const int ijk = C.cell_offset(q);
+    const double rv = 1.0 * r0[ijk];
+    const double zv = 1.0 * d[ijk] * rv;
+    r[ijk] = rv;
+    z[ijk] = zv;
+    p[ijk] = 1.0 * zv;
+    C.prod[q] = rv * zv;
+    const double f = fabs(rv);
+    if (f > m) m = f;
+  }
+  const double r_dot_z = b_sum_staged(C);
+  *norm_r = b_max(C, m);
+  return r_dot_z;
+}
+
+/* D^-1-preconditioned CG, the restatement of solvers.c:cg_host_driven, executed cooperatively by all threads of the calling
+ * thread block; prod: BOTTOM_MAX_CELLS doubles of shared memory, red: 36 doubles of shared memory.
+ * Vectors: r0, r, p of BottomIds play themselves, q plays Ap and s plays z (the ids of cg.c, VECTORS_RESERVED+0..4).
+ * Block barriers per iteration: 8 (ghost fill of p 1, Ap with the Ap.p sum 2, x/r update with max|r| 2, z with the r.z sum 2,
+ * p update 1). */
+__device__ static void cg_solve(const BottomArgs &A, double *prod, double *red)
+{
+  BottomCtx C = { A, prod, red, A.L.dim, A.L.dim * A.L.dim * A.L.dim, A.L.jStride, A.L.kStride, 0 };
+
+  const int r0 = A.ids.r0, r = A.ids.r, p = A.ids.p, Ap = A.ids.q, z = A.ids.s;
+  const int DINV = A.ids.dinv;
+  const int x_id = A.x_id;
+  const int jMax = 200;
+  int j = 0;
+  bool failed = false, converged = false;
+
+  b_apply(C, r0, x_id, A.R_id, 1);                        /* r0 = R - A x */
+  double norm_of_r0;
+  double r_dot_z = b_cg_start(C, r, z, p, r0, DINV, &norm_of_r0);     /* r = r0; z = D^-1 r; p = z */
+  if (r_dot_z == 0.0) converged = true;
+  if (norm_of_r0 == 0.0) converged = true;
+  while ((j < jMax) && !failed && !converged) {
+    j++;
+    const double Ap_dot_p = b_apply_dot(C, Ap, p);       /* Ap = A p */
+    if (Ap_dot_p == 0.0) { failed = true; break; }
+    const double alpha = r_dot_z / Ap_dot_p;
+    if (isinf(alpha)) { failed = true; break; }
+    const double norm_of_r = b_add2_norm(C, x_id, 1.0, x_id, alpha, p, r, 1.0, r, -alpha, Ap);      /* x += alpha p; r -= alpha Ap */
+    if (norm_of_r == 0.0) { converged = true; break; }
+    if (norm_of_r < A.rtol * norm_of_r0) { converged = true; break; }
+    const double r_dot_z_new = b_mul_dot(C, z, 1.0, DINV, r);   /* z = D^-1 r */
+    if (r_dot_z_new == 0.0) { failed = true; break; }
+    const double beta = r_dot_z_new / r_dot_z;
+    if (isinf(beta)) { failed = true; break; }
+    b_add(C, p, 1.0, z, beta, p);                         /* p = z + beta p */
+    r_dot_z = r_dot_z_new;
   }
   if (threadIdx.x == 0) atomicAdd(A.iters, (double)j);
 }

@@ -13,7 +13,7 @@
  * with __syncthreads() where the stream version has kernel boundaries.
  *
  * Residency.  A single-box level keeps the vectors the cycle touches (TEMP, e, R, Dinv, beta_i/j/k; on the
- * bottom level also the 8 Krylov vectors; under L1-Jacobi the level's L1 row inverse, which is not in the slab)
+ * bottom level also the 8 Krylov vectors of BiCGStab, of which CG uses 5; under L1-Jacobi the level's L1 row inverse, which is not in the slab)
  * in shared memory for the duration of the kernel: 160 KB for 8^3 + 4^3 + 2^3.  They arrive and leave as bulk
  * asynchronous copies (cp.async.bulk, one per vector, issued by one thread and counted by an mbarrier).  The phase program addresses vectors by SLOT, so the same
  * operator bodies run on a level that stays in global memory (slot == vector id there).
@@ -24,7 +24,8 @@
  * immediate offset (~190 instead of ~600 instructions per stencil) -- and a ghost fill that derives its
  * boundary-condition columns from the thread index instead of walking tables in global memory.  Every
  * other level (other sizes, several boxes, not resident) runs the generic bodies over the same tables as
- * the level-wide kernels.  All of them evaluate the same expressions (stencil.cuh, bc.cuh, bicgstab.cuh),
+ * the level-wide kernels.  The bottom solve is the selected solver's body (bicgstab_solve or cg_solve, bicgstab.cuh).
+ * All of them evaluate the same expressions (stencil.cuh, bc.cuh, bicgstab.cuh),
  * so the bits are those of the multi-launch path
  * (tests/test_gpu_parity.py::test_coarse_kernel_equals_multilaunch_path).
  */
@@ -83,6 +84,7 @@ struct Phase { unsigned char op, lv, a, b, c, d, e, f; };
 struct CoarseArgs {
   int nlevels, mode, smoother, profile, nphases;
   int e_slot_bottom, R_slot_bottom;
+  int bottom_solver;                              /* HPGMG_BOTTOM_BICGSTAB | HPGMG_BOTTOM_CG */
   BottomIds bottom_ids;
   double a, b, rtol;
   double *krylov;
@@ -348,14 +350,17 @@ __device__ static void c_stencil_fast(const CoarseLevel &V, double *base, const 
   }
 }
 
-__device__ static void c_bottom_solve(const CoarseArgs &A, double *prod, double *red)
+/* not inlined: with either solver body inside the phase loop the kernel spilled under its 128-register cap; as a call of its
+ * own it spills nothing (-Xptxas -v), and it runs once per cycle */
+__device__ static __noinline__ void c_bottom_solve(const CoarseArgs &A, double *prod, double *red)
 {
   const CoarseLevel &V = A.lv[A.nlevels - 1];
   BottomArgs B;
   B.L = V.L;  B.bc = V.bc[0];  B.nbc = V.n_bc[0];
   B.x_id = A.e_slot_bottom;  B.R_id = A.R_slot_bottom;  B.ids = A.bottom_ids;
   B.a = A.a;  B.b = A.b;  B.h2inv = V.h2inv;  B.rtol = A.rtol;  B.iters = A.krylov;
-  bicgstab_solve(B, prod, red);
+  if (A.bottom_solver == HPGMG_BOTTOM_CG) cg_solve(B, prod, red);
+  else                                    bicgstab_solve(B, prod, red);
 }
 
 /* ---- bulk asynchronous copies between the global slabs and the resident copies ---------------------- */
@@ -528,7 +533,7 @@ static int level_is_coarse_eligible(const level_type *level, int is_top, int is_
 }
 
 /* Can levels `from`..bottom of this hierarchy run in the single-block kernel?  (all of them small,
- * entirely local to this rank, Dirichlet, and a single-box bottom the BiCGStab body can solve) */
+ * entirely local to this rank, Dirichlet, and a single-box bottom the single-block solver bodies can solve) */
 extern "C" int hpgmg_coarse_chain_eligible(mg_type *MG, int from)
 {
   if (g_coarse_enabled < 0) {
@@ -604,6 +609,7 @@ extern "C" void hpgmg_coarse_cycle(mg_type *MG, int from, int mode_ftail, int ze
   A.nlevels = bottom - from + 1;
   A.mode = mode_ftail ? MODE_FTAIL : MODE_VCYCLE;
   A.smoother = hpgmg_rt_smoother();
+  A.bottom_solver = hpgmg_rt_bottom_solver();
   A.profile = g_coarse_profile;
   A.a = a;  A.b = b;  A.rtol = MG_DEFAULT_BOTTOM_NORM;
   A.krylov = hpgmg_rt_scalar_slots() + HPGMG_SLOT_KRYLOV;
@@ -645,7 +651,8 @@ extern "C" void hpgmg_coarse_cycle(mg_type *MG, int from, int mode_ftail, int ze
     const int s_temp = add(VECTOR_TEMP, 3), s_e = add(e_id, 3), s_R = add(R_id, 3);
     const int s_dinv = add(VECTOR_DINV, 1), s_bi = add(VECTOR_BETA_I, 1), s_bj = add(VECTOR_BETA_J, 1), s_bk = add(VECTOR_BETA_K, 1);
     int kry[8] = { 0 };
-    if (l == bottom) for (int q = 0; q < 8; q++) kry[q] = add(VECTORS_RESERVED + q, 0);     /* scratch of the solver: every one is written before it is read */
+    if (l == bottom) for (int q = 0; q < 8; q++) kry[q] = add(VECTORS_RESERVED + q, 0);     /* scratch of the solver: every one is written before it is read
+                                                                                            (CG uses the first five; the plan is the same for both solvers) */
     const size_t doubles = (size_t)(n + (l1jacobi ? 1 : 0)) * V.L.volume;     /* + the resident copy of the L1 row inverse */
     const box_type *box0 = &level->my_boxes[0];
     const bool single = V.L.nboxes == 1 && box0->low.i == 0 && box0->low.j == 0 && box0->low.k == 0;

@@ -30,6 +30,7 @@ static int g_initialised = 0;
 static int g_device = -1;
 static int g_verbose = 1;
 static int g_smoother = HPGMG_SMOOTHER_GSRB;
+static int g_bottom_solver = HPGMG_BOTTOM_BICGSTAB;
 static int g_use_graphs = 1;
 static int g_profile = 0;
 static double *g_scalars = NULL;            /* device, HPGMG_NUM_SCALARS doubles */
@@ -137,12 +138,22 @@ extern "C" void hpgmg_b200_set_smoother(int which)
   g_smoother = which;
 }
 extern "C" int  hpgmg_b200_get_smoother(void) { return g_smoother; }
+extern "C" void hpgmg_b200_set_bottom_solver(int which)
+{
+  if (which != HPGMG_BOTTOM_BICGSTAB && which != HPGMG_BOTTOM_CG) {
+    fprintf(stderr, "hpgmg_b200_set_bottom_solver: %d is not a bottom solver (0 BiCGStab, 1 CG); keeping %d\n", which, g_bottom_solver);
+    return;
+  }
+  g_bottom_solver = which;
+}
+extern "C" int  hpgmg_b200_get_bottom_solver(void) { return g_bottom_solver; }
 extern "C" void hpgmg_b200_set_verbose(int on) { g_verbose = on; }
 extern "C" void hpgmg_b200_use_graphs(int on) { g_use_graphs = on; }
 extern "C" void hpgmg_b200_profile_operators(int on) { g_profile = on; }
 
 extern "C" int hpgmg_rt_verbose(void) { return g_verbose; }
 extern "C" int hpgmg_rt_smoother(void) { return g_smoother; }
+extern "C" int hpgmg_rt_bottom_solver(void) { return g_bottom_solver; }
 extern "C" int hpgmg_rt_use_graphs(void) { return g_use_graphs; }
 extern "C" int hpgmg_rt_profile(void) { return g_profile; }
 extern "C" int hpgmg_rt_sm_count(void)

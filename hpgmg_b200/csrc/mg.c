@@ -601,6 +601,7 @@ static long long solve_key(int kind, int onLevel, int u_id, int F_id, double a, 
 {
   long long k = kind;
   k = k * 131 + onLevel;  k = k * 131 + u_id;  k = k * 131 + F_id;  k = k * 131 + hpgmg_rt_smoother();
+  k = k * 7 + hpgmg_rt_bottom_solver();                        /* a graph recorded under one bottom solver never replays under another */
   unsigned long long ua, ub;
   memcpy(&ua, &a, 8);  memcpy(&ub, &b, 8);
   k ^= (long long)(ua * 0x9E3779B97F4A7C15ull) ^ (long long)(ub * 0xC2B2AE3D27D4EB4Full);

@@ -25,6 +25,7 @@ extern "C" {
 /* process-wide settings (runtime.cu) */
 int  hpgmg_rt_verbose(void);          /* print reference-style progress lines?            */
 int  hpgmg_rt_smoother(void);
+int  hpgmg_rt_bottom_solver(void);    /* HPGMG_BOTTOM_BICGSTAB | HPGMG_BOTTOM_CG              */
 int  hpgmg_rt_use_graphs(void);
 int  hpgmg_rt_profile(void);
 int  hpgmg_rt_sm_count(void);         /* multiprocessors of the current device            */

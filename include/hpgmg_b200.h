@@ -41,6 +41,13 @@ const char *hpgmg_b200_backend(void);            /* "cuda-sm_100a": there is no 
 #define HPGMG_SMOOTHER_L1JACOBI 3                /* 6 L1-Jacobi sweeps, w = 1, 1/(Aii + sum|Aij|/2) (operators/jacobi.c) */
 void hpgmg_b200_set_smoother(int which);
 int  hpgmg_b200_get_smoother(void);
+/* The bottom solver, likewise: the reference picks it at compile time (-DUSE_BICGSTAB, the default, | -DUSE_CG; solvers.c).
+ * Any other value is refused (a message on stderr; the current selection stays).  It is read when a bottom solve is
+ * enqueued, so it may change on a built hierarchy; recorded graphs are kept per selection. */
+#define HPGMG_BOTTOM_BICGSTAB   0                /* D^-1-preconditioned BiCGStab (solvers/bicgstab.c) */
+#define HPGMG_BOTTOM_CG         1                /* D^-1-preconditioned CG       (solvers/cg.c)       */
+void hpgmg_b200_set_bottom_solver(int which);
+int  hpgmg_b200_get_bottom_solver(void);
 
 /* 0: silent; 1: the reference's progress lines on stdout (default, rank 0 only). */
 void hpgmg_b200_set_verbose(int on);
