@@ -128,13 +128,13 @@ __device__ static void c_fill_ghosts(const CoarseLevel &V, const int slot, const
   }
 }
 
-/* one sweep / residual over every cell of every box.  mode: 0 GSRB sweep s, 1 Chebyshev sweep s, 2 residual, 3 Jacobi sweep.
+/* one sweep / residual over every cell of every box.  op: OP_GSRB sweep s, OP_CHEBY sweep s, OP_RESIDUAL, OP_JACOBI sweep.
  * GSRB on even boxes: a thread owns an i-pair (exactly one active cell per pair, so no lane idles). */
-__device__ static void c_stencil(const CoarseLevel &V, const int mode, const int src, const int dst, const int rhs_slot, const int s, const double b)
+__device__ static void c_stencil(const CoarseLevel &V, const int op, const int src, const int dst, const int rhs_slot, const int s, const double b)
 {
   const DLevel &L = V.L;
   const int n = L.dim, jS = L.jStride, kS = L.kStride;
-  if (mode == 0 && (n & 1) == 0) {
+  if (op == OP_GSRB && (n & 1) == 0) {
     const int hn = n >> 1, per_box = hn * n * n, total = per_box * L.nboxes;
     for (int q = threadIdx.x; q < total; q += blockDim.x) {
       const int box = q / per_box, c = q - box * per_box;
@@ -143,10 +143,9 @@ __device__ static void c_stencil(const CoarseLevel &V, const int mode, const int
       const double *x = L.vec(box, src) + ijk;
       const double *rhs = L.vec(box, rhs_slot) + ijk;
       double *out = L.vec(box, dst) + ijk;
-      const int color000 = (V.low[3 * box] ^ V.low[3 * box + 1] ^ V.low[3 * box + 2] ^ s) & 1;
-      const int a = (j ^ k ^ color000) & 1;
+      const int a = (j ^ k ^ gsrb_box_parity(V.low, box, s)) & 1;
       const double Ax = fv4_apply_op(x + a, L.vec(box, V.s_bi) + ijk + a, L.vec(box, V.s_bj) + ijk + a, L.vec(box, V.s_bk) + ijk + a, jS, kS, b, V.h2inv);
-      const double xnew = x[a] + L.vec(box, V.s_dinv)[ijk + a] * (rhs[a] - Ax);
+      const double xnew = gsrb_update(x[a], L.vec(box, V.s_dinv)[ijk + a], rhs[a], Ax);
       out[1 - a] = x[1 - a];
       out[a] = xnew;
     }
@@ -159,21 +158,21 @@ __device__ static void c_stencil(const CoarseLevel &V, const int mode, const int
     const int ijk = i + j * jS + k * kS;
     const double *x = L.vec(box, src) + ijk;
     double *out = L.vec(box, dst) + ijk;
-    if (mode == 0) {
-      const int color000 = (V.low[3 * box] ^ V.low[3 * box + 1] ^ V.low[3 * box + 2] ^ s) & 1;
+    if (op == OP_GSRB) {
+      const int color000 = gsrb_box_parity(V.low, box, s);
       if ((i ^ j ^ k ^ color000) & 1) { out[0] = x[0]; continue; }
     }
     const double Ax = fv4_apply_op(x, L.vec(box, V.s_bi) + ijk, L.vec(box, V.s_bj) + ijk, L.vec(box, V.s_bk) + ijk, jS, kS, b, V.h2inv);
     const double rhs = L.vec(box, rhs_slot)[ijk];
-    if (mode == 2) { out[0] = rhs - Ax; continue; }
-    if (mode == 3) {                                                /* jacobi.c: x_n + weight*lambda*(rhs - Ax_n) */
+    if (op == OP_RESIDUAL) { out[0] = rhs - Ax; continue; }
+    if (op == OP_JACOBI) {
       const double lam = V.s_lam >= 0 ? L.vec(box, V.s_lam)[ijk] : V.l1[(size_t)box * L.volume + L.origin + ijk];
-      out[0] = x[0] + (V.jw * lam) * (rhs - Ax);
+      out[0] = jacobi_update(x[0], V.jw, lam, rhs, Ax);
       continue;
     }
     const double dinv = L.vec(box, V.s_dinv)[ijk];
-    if (mode == 0) out[0] = x[0] + dinv * (rhs - Ax);
-    else { const double xn = x[0]; out[0] = xn + V.c1[s] * (xn - out[0]) + V.c2[s] * dinv * (rhs - Ax); }
+    if (op == OP_GSRB) out[0] = gsrb_update(x[0], dinv, rhs, Ax);
+    else out[0] = chebyshev_update(x[0], out[0], V.c1[s], V.c2[s], dinv, rhs, Ax);
   }
 }
 
@@ -308,7 +307,7 @@ __device__ static void c_fill_fast(double *v, const bool box_shape, const bool f
  * strides Geo<N>.  GSRB: one thread per i-pair = per updated cell; Chebyshev / Jacobi / residual: one thread per cell.
  * Resident levels only: lambda of a Jacobi sweep is always in a slot there. */
 template <int N>
-__device__ static void c_stencil_fast(const CoarseLevel &V, double *base, const int mode, const int src, const int dst, const int rhs_slot, const int s, const double b)
+__device__ static void c_stencil_fast(const CoarseLevel &V, double *base, const int op, const int src, const int dst, const int rhs_slot, const int s, const double b)
 {
   typedef Geo<N> G;
   constexpr int LG = N == 8 ? 3 : (N == 4 ? 2 : 1);
@@ -316,10 +315,10 @@ __device__ static void c_stencil_fast(const CoarseLevel &V, double *base, const 
   const double *rhs = base + rhs_slot * G::VOL, *dinv = base + V.s_dinv * G::VOL, *lam = base + V.s_lam * G::VOL;
   double *out = base + dst * G::VOL;
   const double h2inv = V.h2inv;
-  const int work = mode == 0 ? N * N * N / 2 : N * N * N;
+  const int work = op == OP_GSRB ? N * N * N / 2 : N * N * N;
   for (int q = threadIdx.x; q < work; q += blockDim.x) {
     int i, j, k;
-    if (mode == 0) {
+    if (op == OP_GSRB) {
       int p;
       if (N == 8) {
         /* a warp = 4 pairs x 4 rows x 2 planes: with jStride 12 and kStride 144 the 16 lanes of a plane fall into 16 distinct
@@ -335,17 +334,16 @@ __device__ static void c_stencil_fast(const CoarseLevel &V, double *base, const 
     const int ijk = i + j * G::jS + k * G::kS;
     const FixedLoader<G::jS, G::kS> X = { x + ijk }, BI = { bi + ijk }, BJ = { bj + ijk }, BK = { bk + ijk };
     const double Ax = fv4_apply_op_at(X, BI, BJ, BK, b, h2inv);
-    if (mode == 0) {
-      const double xnew = x[ijk] + dinv[ijk] * (rhs[ijk] - Ax);
+    if (op == OP_GSRB) {
+      const double xnew = gsrb_update(x[ijk], dinv[ijk], rhs[ijk], Ax);
       out[ijk ^ 1] = x[ijk ^ 1];                                    /* the pair's other cell is copied (gsrb.c:65-71); strides are even */
       out[ijk] = xnew;
-    } else if (mode == 2) {
+    } else if (op == OP_RESIDUAL) {
       out[ijk] = rhs[ijk] - Ax;
-    } else if (mode == 3) {
-      out[ijk] = x[ijk] + (V.jw * lam[ijk]) * (rhs[ijk] - Ax);     /* jacobi.c */
+    } else if (op == OP_JACOBI) {
+      out[ijk] = jacobi_update(x[ijk], V.jw, lam[ijk], rhs[ijk], Ax);
     } else {
-      const double xn = x[ijk];
-      out[ijk] = xn + V.c1[s] * (xn - out[ijk]) + V.c2[s] * dinv[ijk] * (rhs[ijk] - Ax);     /* x_{n-1} aliases x_{n+1} (chebyshev.c:75-80) */
+      out[ijk] = chebyshev_update(x[ijk], out[ijk], V.c1[s], V.c2[s], dinv[ijk], rhs[ijk], Ax);     /* x_{n-1} aliases x_{n+1} (chebyshev.c:75-80) */
     }
   }
 }
@@ -568,11 +566,11 @@ static void p_add(CoarseArgs &A, int op, int lv, int a = 0, int b = 0, int c = 0
 }
 static void p_smooth(CoarseArgs &A, const Slots *S, int l)                  /* smooth(): gsrb.c:24-132 / chebyshev.c:8-100 / jacobi.c */
 {
-  const int mode = A.smoother == HPGMG_SMOOTHER_CHEBY ? 1 : (A.smoother == HPGMG_SMOOTHER_JACOBI || A.smoother == HPGMG_SMOOTHER_L1JACOBI) ? 3 : 0;
+  const int op = smoother_op(A.smoother);
   for (int s = 0; s < 6; s++) {
     const int src = (s & 1) ? S[l].temp : S[l].e, dst = (s & 1) ? S[l].e : S[l].temp;
     p_add(A, PH_FILL, l, src, 0, 0);
-    p_add(A, PH_STENCIL, l, mode, src, dst, S[l].R, s);
+    p_add(A, PH_STENCIL, l, op, src, dst, S[l].R, s);
   }
 }
 static void p_vcycle(CoarseArgs &A, const Slots *S, int c)                  /* MGVCycle: mg.c:1135-1164 */
@@ -581,7 +579,7 @@ static void p_vcycle(CoarseArgs &A, const Slots *S, int c)                  /* M
   for (int l = c; l < bottom; l++) {
     p_smooth(A, S, l);
     p_add(A, PH_FILL, l, S[l].e, 0, 0);                                    /* residual(): exchange + BC on x */
-    p_add(A, PH_STENCIL, l, 2, S[l].e, S[l].temp, S[l].R, 0);
+    p_add(A, PH_STENCIL, l, OP_RESIDUAL, S[l].e, S[l].temp, S[l].R, 0);
     p_add(A, PH_RESTRICT_ZERO, l, S[l + 1].R, S[l].temp, S[l + 1].e);      /* restriction(l+1,R <- l,TEMP); zero_vector(l+1,e) */
   }
   p_add(A, PH_BOTTOM, bottom);
@@ -636,13 +634,9 @@ extern "C" void hpgmg_coarse_cycle(mg_type *MG, int from, int mode_ftail, int ze
     for (int e = 0; e < Cr->num_blocks[1]; e++) { const int c = Cr->blocks[1][e].dim.i * Cr->blocks[1][e].dim.j * Cr->blocks[1][e].dim.k; if (c > V.restr_cells) V.restr_cells = c; }
     for (int e = 0; e < Ci->num_blocks[1]; e++) { const int c = Ci->blocks[1][e].dim.i * Ci->blocks[1][e].dim.j * Ci->blocks[1][e].dim.k; if (c > V.interp_cells) V.interp_cells = c; }
     V.h2inv = 1.0 / (level->h * level->h);
-    /* Chebyshev coefficients exactly as chebyshev.c:22-40 */
-    double beta = 1.000 * level->dominant_eigenvalue_of_DinvA, alpha = 0.125000 * beta;
-    double theta = 0.5 * (beta + alpha), delta = 0.5 * (beta - alpha), sigma = theta / delta, rho_n = 1 / sigma;
-    V.c1[0] = 0.0;  V.c2[0] = 1 / theta;
-    for (int s = 1; s < 6; s++) { double rho_nm1 = rho_n; rho_n = 1.0 / (2.0 * sigma - rho_nm1); V.c1[s] = rho_n * rho_nm1; V.c2[s] = rho_n * 2.0 / delta; }
+    chebyshev_coefficients(level->dominant_eigenvalue_of_DinvA, V.c1, V.c2);
+    V.jw = jacobi_weight(A.smoother);
     const bool l1jacobi = A.smoother == HPGMG_SMOOTHER_L1JACOBI;
-    V.jw = l1jacobi ? 1.0 : 2.0 / 3.0;                               /* jacobi.c */
     V.l1 = l1jacobi ? hpgmg_l1inv_array(level) : NULL;
 
     /* slots: the vectors a cycle touches; identity (slot == vector id) when the level stays in global memory */

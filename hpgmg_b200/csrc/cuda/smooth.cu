@@ -14,10 +14,6 @@
 #include "common.cuh"
 #include "stencil.cuh"
 
-enum { OP_APPLY = 0, OP_RESIDUAL = 1, OP_GSRB = 2, OP_CHEBY = 3, OP_REBUILD = 4,
-       OP_RESRES = 5,     /* residual fused with the cell restriction that follows it in MGVCycle (k-marching kernel only) */
-       OP_JACOBI = 6 };   /* one Jacobi sweep: x + (weight*lambda)*(rhs - A x) */
-
 /* The Helmholtz build (-DUSE_HELMHOLTZ, as in the reference: operators.fv4.c:56-85): A x = a*alpha*x - b*h2inv*(...).  The
  * reference subtracts (b*h2inv)*(...) from a*alpha*x; fv4_apply_op returns (-b*h2inv)*(...), the exact negation, and
  * p - q == p + (-q) in IEEE arithmetic, so the sum below has the reference's bits.  In that build every operator goes
@@ -74,12 +70,12 @@ __global__ void __launch_bounds__(256) stencil_generic_kernel(const StencilArgs 
 
   if (OP == OP_GSRB) {
     double *__restrict__ out = L.vec(box, A.out_id) + ijk;
-    const int color000 = (A.low[3 * box] ^ A.low[3 * box + 1] ^ A.low[3 * box + 2] ^ A.sweep) & 1;
+    const int color000 = gsrb_box_parity(A.low, box, A.sweep);
     if (((i ^ j ^ k ^ color000) & 1) == 0) {
       const double Ax = HELMHOLTZ_TERM(A.a, L.vec(box, VECTOR_ALPHA_OR_0)[ijk], x[0]) fv4_apply_op(x, bi, bj, bk, jS, kS, A.b, A.h2inv);
       const double dinv = L.vec(box, VECTOR_DINV)[ijk];
       const double rhs = L.vec(box, A.rhs_id)[ijk];
-      out[0] = x[0] + dinv * (rhs - Ax);
+      out[0] = gsrb_update(x[0], dinv, rhs, Ax);
     } else {
       out[0] = x[0];
     }
@@ -95,11 +91,11 @@ __global__ void __launch_bounds__(256) stencil_generic_kernel(const StencilArgs 
     const double xm1 = L.vec(box, A.xm1_id)[ijk];
     const double dinv = L.vec(box, VECTOR_DINV)[ijk];
     const double rhs = L.vec(box, A.rhs_id)[ijk];
-    L.vec(box, A.out_id)[ijk] = xn + A.c1 * (xn - xm1) + A.c2 * dinv * (rhs - Ax);
-  } else if (OP == OP_JACOBI) {                          /* jacobi.c: x_n + weight*lambda*(rhs - Ax_n), left to right */
+    L.vec(box, A.out_id)[ijk] = chebyshev_update(xn, xm1, A.c1, A.c2, dinv, rhs, Ax);
+  } else if (OP == OP_JACOBI) {
     const double lam = A.lam[(size_t)box * A.lam_bstride + ijk];
     const double rhs = L.vec(box, A.rhs_id)[ijk];
-    L.vec(box, A.out_id)[ijk] = x[0] + (A.weight * lam) * (rhs - Ax);
+    L.vec(box, A.out_id)[ijk] = jacobi_update(x[0], A.weight, lam, rhs, Ax);
   } else if (OP == OP_REBUILD) {
     /* rebuild.c:127-133: x is a 0/1 colouring; Aii += x*Ax, sumAbsAij += |(1-x)*Ax| */
     double *Aii = L.vec(box, A.out_id) + ijk;
@@ -237,12 +233,11 @@ __global__ void __launch_bounds__(256) stencil_pair_kernel(const StencilArgs A)
   const double *__restrict__ bk = L.vec(box, VECTOR_BETA_K) + ijk;
   double2 *out = reinterpret_cast<double2 *>(L.vec(box, A.out_id) + ijk);
   if (OP == OP_GSRB) {
-    const int color000 = (A.low[3 * box] ^ A.low[3 * box + 1] ^ A.low[3 * box + 2] ^ A.sweep) & 1;
-    const int a = (j ^ k ^ color000) & 1;                     /* the active cell of the pair */
+    const int a = (j ^ k ^ gsrb_box_parity(A.low, box, A.sweep)) & 1;     /* the active cell of the pair */
     const double2 rhs2 = *reinterpret_cast<const double2 *>(L.vec(box, A.rhs_id) + ijk);
     const double2 dinv2 = *reinterpret_cast<const double2 *>(L.vec(box, VECTOR_DINV) + ijk);
     const double Ax = HELMHOLTZ_TERM(A.a, L.vec(box, VECTOR_ALPHA_OR_0)[ijk + a], x[a]) fv4_apply_op(x + a, bi + a, bj + a, bk + a, jS, kS, A.b, A.h2inv);
-    const double xnew = x[a] + (a ? dinv2.y : dinv2.x) * ((a ? rhs2.y : rhs2.x) - Ax);
+    const double xnew = gsrb_update(x[a], a ? dinv2.y : dinv2.x, a ? rhs2.y : rhs2.x, Ax);
     const double xo = x[1 - a];
     *out = a ? make_double2(xo, xnew) : make_double2(xnew, xo);
     return;
@@ -254,13 +249,13 @@ __global__ void __launch_bounds__(256) stencil_pair_kernel(const StencilArgs A)
   if (OP == OP_RESIDUAL) { *out = make_double2(rhs2.x - Ax0, rhs2.y - Ax1); return; }
   if (OP == OP_JACOBI) {
     const double2 lam2 = *reinterpret_cast<const double2 *>(A.lam + (size_t)box * A.lam_bstride + ijk);
-    *out = make_double2(x[0] + (A.weight * lam2.x) * (rhs2.x - Ax0), x[1] + (A.weight * lam2.y) * (rhs2.y - Ax1));
+    *out = make_double2(jacobi_update(x[0], A.weight, lam2.x, rhs2.x, Ax0), jacobi_update(x[1], A.weight, lam2.y, rhs2.y, Ax1));
     return;
   }
   const double2 dinv2 = *reinterpret_cast<const double2 *>(L.vec(box, VECTOR_DINV) + ijk);   /* OP_CHEBY */
   const double2 xm = *reinterpret_cast<const double2 *>(L.vec(box, A.xm1_id) + ijk);
-  *out = make_double2(x[0] + A.c1 * (x[0] - xm.x) + A.c2 * dinv2.x * (rhs2.x - Ax0),
-                      x[1] + A.c1 * (x[1] - xm.y) + A.c2 * dinv2.y * (rhs2.y - Ax1));
+  *out = make_double2(chebyshev_update(x[0], xm.x, A.c1, A.c2, dinv2.x, rhs2.x, Ax0),
+                      chebyshev_update(x[1], xm.y, A.c1, A.c2, dinv2.y, rhs2.y, Ax1));
 }
 
 template <int OP>
@@ -460,66 +455,6 @@ extern "C" void hpgmg_residual_norm_async(level_type *level, int res_id, int x_i
   else hpgmg_norm_async(level, res_id, slot);
 }
 
-static void smooth_gsrb(level_type *level, int x_id, int rhs_id, double a, double b)
-{
-  for (int s = 0; s < 6; s++) {                      /* NUM_SMOOTHS=3 -> RBRBRB (operators.fv4.c:177-180) */
-    const int src = (s & 1) == 0 ? x_id : VECTOR_TEMP;
-    const int dst = (s & 1) == 0 ? VECTOR_TEMP : x_id;
-    StencilArgs A = {};
-    A.x_id = src;  A.rhs_id = rhs_id;  A.out_id = dst;  A.a = a;  A.b = b;  A.sweep = s;
-    A.reverse = g_zigzag ? (s & 1) : 0;
-    fill_and_stencil<OP_GSRB>(level, A, 0);
-  }
-}
-
-/* one GSRB sweep kernel alone (no ghost fill) */
-extern "C" void hpgmg_b200_gsrb_sweep(level_type *level, int src_id, int dst_id, int rhs_id, double a, double b, int s)
-{
-  StencilArgs A = {};
-  A.x_id = src_id;  A.rhs_id = rhs_id;  A.out_id = dst_id;  A.a = a;  A.b = b;  A.sweep = s;
-  launch_stencil<OP_GSRB>(level, A);
-}
-
-/* Chebyshev coefficients exactly as chebyshev.c:22-40 (degree 6, operators.fv4.c:184) */
-static void chebyshev_coefficients(const level_type *level, double c1[6], double c2[6])
-{
-  double beta = 1.000 * level->dominant_eigenvalue_of_DinvA;
-  double alpha = 0.125000 * beta;
-  double theta = 0.5 * (beta + alpha);
-  double delta = 0.5 * (beta - alpha);
-  double sigma = theta / delta;
-  double rho_n = 1 / sigma;
-  c1[0] = 0.0;
-  c2[0] = 1 / theta;
-  for (int s = 1; s < 6; s++) {
-    double rho_nm1 = rho_n;
-    rho_n = 1.0 / (2.0 * sigma - rho_nm1);
-    c1[s] = rho_n * rho_nm1;
-    c2[s] = rho_n * 2.0 / delta;
-  }
-}
-
-static void chebyshev_sweep(level_type *level, int src, int dst, int rhs_id, double a, double b, const double c1, const double c2, const int with_fill)
-{
-  StencilArgs A = {};
-  A.x_id = src;  A.xm1_id = dst;  A.rhs_id = rhs_id;  A.out_id = dst;  A.a = a;  A.b = b;     /* x_{n-1} aliases x_{n+1} (chebyshev.c:75-80) */
-  A.c1 = c1;  A.c2 = c2;
-  if (with_fill) fill_and_stencil<OP_CHEBY>(level, A, 0);
-  else launch_stencil<OP_CHEBY>(level, A);
-}
-
-static void smooth_chebyshev(level_type *level, int x_id, int rhs_id, double a, double b)
-{
-  if (level->dominant_eigenvalue_of_DinvA <= 0.0 && level->my_rank == 0) fprintf(stderr, "dominant_eigenvalue_of_DinvA <= 0.0 !\n");
-  double c1[6], c2[6];
-  chebyshev_coefficients(level, c1, c2);
-  for (int s = 0; s < 6; s++) {
-    const int src = (s & 1) == 0 ? x_id : VECTOR_TEMP;
-    const int dst = (s & 1) == 0 ? VECTOR_TEMP : x_id;
-    chebyshev_sweep(level, src, dst, rhs_id, a, b, c1[s], c2[s], 1);
-  }
-}
-
 /* The L1 row inverse of a level in the default build (rebuild_operator_blackbox stores it only while L1-Jacobi is selected).
  * The reference fixes its smoother at compile time, so it always has the vector; here a level built for another smoother
  * cannot be smoothed with L1-Jacobi: recomputing the array here would overwrite VECTOR_TEMP and VECTOR_E, which hold live
@@ -547,60 +482,68 @@ extern "C" void hpgmg_download_l1inv(level_type *level, int box, double *host)
 #endif
 }
 
-/* weight and lambda of the selected Jacobi variant (jacobi.c): USE_JACOBI 2/3 and Dinv, USE_L1JACOBI 1 and the L1 row inverse */
-static void jacobi_operands(level_type *level, StencilArgs &A)
+/* the arguments of sweep s (the GSRB colour, the Chebyshev step) of the smoother whose operator is op, src -> dst */
+static StencilArgs sweep_args(level_type *level, const int op, const int src, const int dst, const int rhs_id, const double a, const double b, const int s)
 {
-  const DLevel &L = dl_of(level);
-  if (hpgmg_rt_smoother() == HPGMG_SMOOTHER_L1JACOBI) {
-    A.weight = 1.0;
-#ifdef VECTOR_L1INV
-    A.lam = L.vec(0, VECTOR_L1INV);  A.lam_bstride = (size_t)L.nvec * L.volume;
-#else
-    A.lam = hpgmg_l1inv_array(level) + L.origin;  A.lam_bstride = (size_t)L.volume;
-#endif
-  } else {
-    A.weight = 2.0 / 3.0;
+  StencilArgs A = {};
+  A.x_id = src;  A.rhs_id = rhs_id;  A.out_id = dst;  A.a = a;  A.b = b;  A.sweep = s;
+  if (op == OP_CHEBY) {
+    double c1[6], c2[6];
+    chebyshev_coefficients(level->dominant_eigenvalue_of_DinvA, c1, c2);
+    A.xm1_id = dst;  A.c1 = c1[s % 6];  A.c2 = c2[s % 6];            /* x_{n-1} aliases x_{n+1} (chebyshev.c:75-80) */
+  } else if (op == OP_JACOBI) {                                          /* lambda: Dinv, or the L1 row inverse */
+    const DLevel &L = dl_of(level);
+    A.weight = jacobi_weight(hpgmg_rt_smoother());
     A.lam = L.vec(0, VECTOR_DINV);  A.lam_bstride = (size_t)L.nvec * L.volume;
+    if (hpgmg_rt_smoother() == HPGMG_SMOOTHER_L1JACOBI) {
+#ifdef VECTOR_L1INV
+      A.lam = L.vec(0, VECTOR_L1INV);
+#else
+      A.lam = hpgmg_l1inv_array(level) + L.origin;  A.lam_bstride = (size_t)L.volume;
+#endif
+    }
   }
+  return A;
 }
 
-static void smooth_jacobi(level_type *level, int x_id, int rhs_id, double a, double b)
+/* one GSRB sweep kernel alone (no ghost fill) */
+extern "C" void hpgmg_b200_gsrb_sweep(level_type *level, int src_id, int dst_id, int rhs_id, double a, double b, int s)
 {
-  StencilArgs J = {};
-  jacobi_operands(level, J);
-  for (int s = 0; s < 6; s++) {                      /* NUM_SMOOTHS=6 (operators.fv4.c:176-195); x -> TEMP -> x like GSRB */
-    StencilArgs A = J;
-    A.x_id = (s & 1) == 0 ? x_id : VECTOR_TEMP;
-    A.out_id = (s & 1) == 0 ? VECTOR_TEMP : x_id;
-    A.rhs_id = rhs_id;  A.a = a;  A.b = b;
-    fill_and_stencil<OP_JACOBI>(level, A, 0);
-  }
+  StencilArgs A = sweep_args(level, OP_GSRB, src_id, dst_id, rhs_id, a, b, s);
+  launch_stencil<OP_GSRB>(level, A);
 }
-
-static int is_jacobi(const int smoother) { return smoother == HPGMG_SMOOTHER_JACOBI || smoother == HPGMG_SMOOTHER_L1JACOBI; }
 
 /* one sweep kernel of the current smoother alone (no ghost fill): what bench.py times for the roofline line */
 extern "C" void hpgmg_b200_smoother_sweep(level_type *level, int src_id, int dst_id, int rhs_id, double a, double b, int s)
 {
-  if (hpgmg_rt_smoother() == HPGMG_SMOOTHER_CHEBY) {
-    double c1[6], c2[6];
-    chebyshev_coefficients(level, c1, c2);
-    chebyshev_sweep(level, src_id, dst_id, rhs_id, a, b, c1[s % 6], c2[s % 6], 0);
-  } else if (is_jacobi(hpgmg_rt_smoother())) {
-    StencilArgs A = {};
-    jacobi_operands(level, A);
-    A.x_id = src_id;  A.rhs_id = rhs_id;  A.out_id = dst_id;  A.a = a;  A.b = b;
-    launch_stencil<OP_JACOBI>(level, A);
-  } else hpgmg_b200_gsrb_sweep(level, src_id, dst_id, rhs_id, a, b, s);
+  const int op = smoother_op(hpgmg_rt_smoother());
+  StencilArgs A = sweep_args(level, op, src_id, dst_id, rhs_id, a, b, s);
+  switch (op) {
+    case OP_CHEBY:  launch_stencil<OP_CHEBY>(level, A);  break;
+    case OP_JACOBI: launch_stencil<OP_JACOBI>(level, A); break;
+    default:        launch_stencil<OP_GSRB>(level, A);   break;
+  }
 }
 
+/* GSRB: NUM_SMOOTHS=3 -> RBRBRB (operators.fv4.c:177-180); Chebyshev: degree 6 (:184); Jacobi: NUM_SMOOTHS=6 (:176-195).
+ * Each is 6 sweeps x -> TEMP -> x, every one after a ghost fill of its source. */
 extern "C" void smooth(level_type *level, int x_id, int rhs_id, double a, double b)
 {
   ProfileScope prof_(&level->timers.smooth);
   hpgmg_note_vector_written(level, x_id);
-  if (hpgmg_rt_smoother() == HPGMG_SMOOTHER_CHEBY) smooth_chebyshev(level, x_id, rhs_id, a, b);
-  else if (is_jacobi(hpgmg_rt_smoother())) smooth_jacobi(level, x_id, rhs_id, a, b);
-  else smooth_gsrb(level, x_id, rhs_id, a, b);
+  const int op = smoother_op(hpgmg_rt_smoother());
+  if (op == OP_CHEBY && level->dominant_eigenvalue_of_DinvA <= 0.0 && level->my_rank == 0) fprintf(stderr, "dominant_eigenvalue_of_DinvA <= 0.0 !\n");
+  for (int s = 0; s < 6; s++) {
+    const int src = (s & 1) == 0 ? x_id : VECTOR_TEMP;
+    const int dst = (s & 1) == 0 ? VECTOR_TEMP : x_id;
+    StencilArgs A = sweep_args(level, op, src, dst, rhs_id, a, b, s);
+    A.reverse = g_zigzag ? (s & 1) : 0;                                  /* GSRB only (launch_tma): alternate sweeps march k downwards */
+    switch (op) {
+      case OP_CHEBY:  fill_and_stencil<OP_CHEBY>(level, A, 0);  break;
+      case OP_JACOBI: fill_and_stencil<OP_JACOBI>(level, A, 0); break;
+      default:        fill_and_stencil<OP_GSRB>(level, A, 0);   break;
+    }
+  }
 }
 
 /* ------------------------------------------------------------------------------------------ */

@@ -15,9 +15,19 @@
  * The arithmetic is written ONCE, over four "loaders" X, BI, BJ, BK that return the value at an
  * offset (di,dj,dk) from the cell: the global-memory kernels pass pointer loaders, the tiled kernels
  * pass shared-memory loaders; both therefore produce identical bits.
+ *
+ * The smoothers' cell updates, the GSRB colouring and the smoothers' per-level coefficients live here too, so
+ * that every kernel family (smooth.cu, stencil_tma.cuh, stencil_box.cuh, coarse.cu) evaluates the same expressions.
  */
 #ifndef HPGMG_B200_STENCIL_CUH
 #define HPGMG_B200_STENCIL_CUH
+
+#include "hpgmg_b200.h"
+
+/* what an operator kernel computes; kernel symbols are named by these values (stencil_tma_kernel<2,...> is the GSRB sweep) */
+enum { OP_APPLY = 0, OP_RESIDUAL = 1, OP_GSRB = 2, OP_CHEBY = 3, OP_REBUILD = 4,
+       OP_RESRES = 5,     /* residual fused with the cell restriction that follows it in MGVCycle (k-marching kernel only) */
+       OP_JACOBI = 6 };   /* one Jacobi sweep: x + (weight*lambda)*(rhs - A x) */
 
 #define STENCIL_TWELFTH (0.0833333333333333333)
 
@@ -85,6 +95,67 @@ __device__ __forceinline__ double fv4_apply_op(const double *__restrict__ x,
 {
   const GlobalLoader X = { x, jS, kS }, BI = { bi, jS, kS }, BJ = { bj, jS, kS }, BK = { bk, jS, kS };
   return fv4_apply_op_at(X, BI, BJ, BK, b, h2inv);
+}
+
+/* ---- the smoothers at one cell: x the cell's value before the sweep, Ax = (A x) there; the reference's association order ---- */
+/* gsrb.c:41-129: x + Dinv*(rhs - Ax) */
+__device__ __forceinline__ double gsrb_update(const double x, const double dinv, const double rhs, const double Ax)
+{
+  return x + dinv * (rhs - Ax);
+}
+
+/* chebyshev.c:90: x_n + c1*(x_n - x_{n-1}) + c2*Dinv*(rhs - Ax_n) */
+__device__ __forceinline__ double chebyshev_update(const double x, const double xm1, const double c1, const double c2, const double dinv, const double rhs, const double Ax)
+{
+  return x + c1 * (x - xm1) + c2 * dinv * (rhs - Ax);
+}
+
+/* jacobi.c: x_n + weight*lambda*(rhs - Ax_n), left to right */
+__device__ __forceinline__ double jacobi_update(const double x, const double weight, const double lam, const double rhs, const double Ax)
+{
+  return x + (weight * lam) * (rhs - Ax);
+}
+
+/* GSRB colouring (gsrb.c:55,100): cell (i,j,k) of box `box`, whose low corner is low[3 box .. 3 box + 2], is updated
+ * on sweep s iff ((i ^ j ^ k ^ gsrb_box_parity(low, box, s)) & 1) == 0.  sweep is taken by reference so that, like the
+ * corner, it is a load here: taken by value, the compiler orders the xors differently (same value, other instructions). */
+__device__ __forceinline__ int gsrb_box_parity(const int *low, const int box, const int &sweep)
+{
+  return (low[3 * box] ^ low[3 * box + 1] ^ low[3 * box + 2] ^ sweep) & 1;
+}
+
+/* ---- the smoothers' per-level coefficients and operator codes (host) ---- */
+/* Chebyshev coefficients of the 6 steps, exactly as chebyshev.c:22-40 (degree 6, operators.fv4.c:184) */
+static inline void chebyshev_coefficients(const double dominant_eigenvalue_of_DinvA, double c1[6], double c2[6])
+{
+  double beta = 1.000 * dominant_eigenvalue_of_DinvA;
+  double alpha = 0.125000 * beta;
+  double theta = 0.5 * (beta + alpha);
+  double delta = 0.5 * (beta - alpha);
+  double sigma = theta / delta;
+  double rho_n = 1 / sigma;
+  c1[0] = 0.0;
+  c2[0] = 1 / theta;
+  for (int s = 1; s < 6; s++) {
+    double rho_nm1 = rho_n;
+    rho_n = 1.0 / (2.0 * sigma - rho_nm1);
+    c1[s] = rho_n * rho_nm1;
+    c2[s] = rho_n * 2.0 / delta;
+  }
+}
+
+/* jacobi.c: weight 2/3 with lambda = Dinv (USE_JACOBI), 1 with lambda = the L1 row inverse (USE_L1JACOBI) */
+static inline double jacobi_weight(const int smoother)
+{
+  return smoother == HPGMG_SMOOTHER_L1JACOBI ? 1.0 : 2.0 / 3.0;
+}
+
+/* the sweep operator of a smoother (HPGMG_SMOOTHER_*) */
+static inline int smoother_op(const int smoother)
+{
+  if (smoother == HPGMG_SMOOTHER_CHEBY) return OP_CHEBY;
+  if (smoother == HPGMG_SMOOTHER_JACOBI || smoother == HPGMG_SMOOTHER_L1JACOBI) return OP_JACOBI;
+  return OP_GSRB;
 }
 
 #endif

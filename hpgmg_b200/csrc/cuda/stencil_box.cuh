@@ -13,7 +13,8 @@
  * The values are those the separate fill would have left in the ghost cells (same expressions, same operands), so
  * the result is bit-identical; the ghost cells in HBM are simply not needed any more (residual / apply_op still
  * write them, because callers of the reference API may look at them: residual.c:15-16 fills x in place).
- * gsrb.c:41-129, chebyshev.c:51-97, jacobi.c, residual.c:18-49, apply_op.c:18-47; arithmetic = fv4_apply_op_at (stencil.cuh).
+ * gsrb.c:41-129, chebyshev.c:51-97, jacobi.c, residual.c:18-49, apply_op.c:18-47; arithmetic = fv4_apply_op_at and the
+ * smoothers' cell updates (stencil.cuh).
  *
  * Face coefficients, rhs and Dinv are read straight from global memory at compile-time strides (the box size is a
  * template parameter), i.e. as loads at immediate offsets through L1.  Rows of the staged tile are stored as they are
@@ -123,14 +124,13 @@ __global__ void __launch_bounds__((TI / 2) * TJ * TK) stencil_box_kernel(const B
   const double *bi = L.vec(box, VECTOR_BETA_I) + cell, *bj = L.vec(box, VECTOR_BETA_J) + cell, *bk = L.vec(box, VECTOR_BETA_K) + cell;
   double2 *out = reinterpret_cast<double2 *>(L.vec(box, A.out_id) + cell);
   if constexpr (OP == OP_GSRB) {
-    const int color000 = (A.low[3 * box] ^ A.low[3 * box + 1] ^ A.low[3 * box + 2] ^ A.sweep) & 1;
-    const int a = (j ^ k ^ color000) & 1;                          /* the pair's active cell (gsrb.c:55,100) */
+    const int a = (j ^ k ^ gsrb_box_parity(A.low, box, A.sweep)) & 1;     /* the pair's active cell */
     const double2 rhs2 = *reinterpret_cast<const double2 *>(L.vec(box, A.rhs_id) + cell);
     const double2 dinv2 = *reinterpret_cast<const double2 *>(L.vec(box, VECTOR_DINV) + cell);
     const TileLoader<C::SW, C::SH> X = { ts + a };
     const BoxLoader<C::jS, C::kS> BI = { bi + a }, BJ = { bj + a }, BK = { bk + a };
     const double Ax = fv4_apply_op_at(X, BI, BJ, BK, A.b, A.h2inv);
-    const double xnew = ts[a] + (a ? dinv2.y : dinv2.x) * ((a ? rhs2.y : rhs2.x) - Ax);
+    const double xnew = gsrb_update(ts[a], a ? dinv2.y : dinv2.x, a ? rhs2.y : rhs2.x, Ax);
     const double xo = ts[1 - a];                                   /* the other cell is copied (gsrb.c:65-71) */
     *out = a ? make_double2(xo, xnew) : make_double2(xnew, xo);
   } else {
@@ -147,14 +147,14 @@ __global__ void __launch_bounds__((TI / 2) * TJ * TK) stencil_box_kernel(const B
       const double2 rhs2 = *reinterpret_cast<const double2 *>(L.vec(box, A.rhs_id) + cell);
       if constexpr (OP == OP_RESIDUAL) {
         *out = make_double2(rhs2.x - Ax[0], rhs2.y - Ax[1]);
-      } else if constexpr (OP == OP_JACOBI) {                        /* jacobi.c: x_n + weight*lambda*(rhs - Ax_n), left to right */
+      } else if constexpr (OP == OP_JACOBI) {
         const double2 lam2 = *reinterpret_cast<const double2 *>(A.lam + (size_t)box * A.lam_bstride + cell);
-        *out = make_double2(ts[0] + (A.weight * lam2.x) * (rhs2.x - Ax[0]), ts[1] + (A.weight * lam2.y) * (rhs2.y - Ax[1]));
-      } else {                                                       /* OP_CHEBY (chebyshev.c:90) */
+        *out = make_double2(jacobi_update(ts[0], A.weight, lam2.x, rhs2.x, Ax[0]), jacobi_update(ts[1], A.weight, lam2.y, rhs2.y, Ax[1]));
+      } else {                                                       /* OP_CHEBY */
         const double2 dinv2 = *reinterpret_cast<const double2 *>(L.vec(box, VECTOR_DINV) + cell);
         const double2 xm = *out;                                     /* x_{n-1} aliases x_{n+1} (chebyshev.c:75-80) */
-        *out = make_double2(ts[0] + A.c1 * (ts[0] - xm.x) + A.c2 * dinv2.x * (rhs2.x - Ax[0]),
-                            ts[1] + A.c1 * (ts[1] - xm.y) + A.c2 * dinv2.y * (rhs2.y - Ax[1]));
+        *out = make_double2(chebyshev_update(ts[0], xm.x, A.c1, A.c2, dinv2.x, rhs2.x, Ax[0]),
+                            chebyshev_update(ts[1], xm.y, A.c1, A.c2, dinv2.y, rhs2.y, Ax[1]));
       }
     }
   }

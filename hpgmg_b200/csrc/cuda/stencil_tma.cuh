@@ -4,7 +4,8 @@
  *
  * GSRB / Chebyshev / Jacobi / residual / apply_op on a TI x TJ column of cells marching along k (gsrb.c:41-129,
  * chebyshev.c:51-97, jacobi.c, residual.c:18-49, apply_op.c:18-47 with the macro of operators.fv4.c:87-114); the
- * arithmetic is fv4_apply_op_at, shared with every other kernel, hence the same bits.  Around the arithmetic:
+ * arithmetic is fv4_apply_op_at and the smoothers' cell updates (stencil.cuh), shared with every other kernel, hence
+ * the same bits.  Around the arithmetic:
  *
  *  - staging: one elected thread issues cp.async.bulk.tensor (TMA) copies of whole (TI+4) x rows tiles
  *    of x, beta_i, beta_j, beta_k PF steps ahead into ring buffers; completion is counted by mbarriers
@@ -213,7 +214,7 @@ stencil_tma_kernel(const StencilArgs A, const __grid_constant__ CUtensorMap map_
     /* which cell of the pair is updated on plane k0 of this sweep (gsrb.c:55,100); flips every plane.
      * For the uncoloured operators it only fixes the ORDER in which the lane evaluates its two cells
      * (odd lanes start with the odd cell, so that a half-warp still covers all banks). */
-    int s = (OP == OP_GSRB) ? ((j ^ kf ^ A.low[3 * box] ^ A.low[3 * box + 1] ^ A.low[3 * box + 2] ^ A.sweep) & 1) : (lane & 1);
+    int s = (OP == OP_GSRB) ? ((j ^ kf ^ gsrb_box_parity(A.low, box, A.sweep)) & 1) : (lane & 1);
 
     /* Dinv from memory only where a cell of the tile is within 2 cells of the domain boundary (its stencil then
      * reaches boundary-condition ghost cells and the stored diagonal carries their contribution); elsewhere it is
@@ -290,7 +291,7 @@ stencil_tma_kernel(const StencilArgs A, const __grid_constant__ CUtensorMap map_
         const double xc = X(0, 0, 0);
         const double xo = lds_f64(ax[2] + (unsigned)(8 * (1 - s)));    /* the pair's other cell: copied (gsrb.c:65-71) */
         const double dinv = PLANE_NEEDS_DINV(k) ? (s ? dinv2.y : dinv2.x) : 1.0 / aii;
-        const double xnew = xc + dinv * ((s ? rhs2.y : rhs2.x) - Ax);
+        const double xnew = gsrb_update(xc, dinv, s ? rhs2.y : rhs2.x, Ax);
         out2 = s ? make_double2(xo, xnew) : make_double2(xnew, xo);
         s ^= 1;
       } else {
@@ -315,14 +316,8 @@ stencil_tma_kernel(const StencilArgs A, const __grid_constant__ CUtensorMap map_
           if (OP == OP_APPLY) v = Ax;
           else if (OP == OP_RESIDUAL) { v = (c ? rhs2.y : rhs2.x) - Ax; const double f = fabs(v); if (f > vmax) vmax = f; }
           else if (OP == OP_RESRES) v = (c ? rhs2.y : rhs2.x) - Ax;
-          else if (OP == OP_JACOBI) {                                /* jacobi.c: x_n + weight*lambda*(rhs - Ax_n), left to right */
-            const double xn = PX(0, 0, 0);
-            v = xn + (A.weight * (c ? dinv2.y : dinv2.x)) * ((c ? rhs2.y : rhs2.x) - Ax);
-          }
-          else {                                                     /* OP_CHEBY, chebyshev.c:90 */
-            const double xn = PX(0, 0, 0);
-            v = xn + A.c1 * (xn - (c ? xm2.y : xm2.x)) + A.c2 * (c ? dinv2.y : dinv2.x) * ((c ? rhs2.y : rhs2.x) - Ax);
-          }
+          else if (OP == OP_JACOBI) v = jacobi_update(PX(0, 0, 0), A.weight, c ? dinv2.y : dinv2.x, c ? rhs2.y : rhs2.x, Ax);
+          else v = chebyshev_update(PX(0, 0, 0), c ? xm2.y : xm2.x, A.c1, A.c2, c ? dinv2.y : dinv2.x, c ? rhs2.y : rhs2.x, Ax);     /* OP_CHEBY */
           res[c] = v;
         }
         out2 = make_double2(res[0], res[1]);
