@@ -18,6 +18,9 @@ from ._structs import (blockCopy_type, box_type, communicator_type, level_type, 
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libhpgmg_b200.so")
+# the 2nd-order operator (the reference linked with operators.fv2.c): one ghost layer, bind with bind(ctypes.CDLL(FV2_LIB_PATH))
+# and pass it as Hierarchy(..., library=...)
+FV2_LIB_PATH = os.path.join(_HERE, "lib", "libhpgmg_b200_fv2.so")
 
 # defines.h:28-38
 VECTOR_TEMP, VECTOR_U, VECTOR_F, VECTOR_E, VECTOR_R, VECTOR_DINV, VECTOR_BETA_I, VECTOR_BETA_J, VECTOR_BETA_K = range(9)
@@ -76,6 +79,7 @@ SIGNATURES = {
     "restriction": (_V, [_LP, _I, _LP, _I, _I]),
     "interpolation_vcycle": (_V, [_LP, _I, _D, _LP, _I]), "interpolation_fcycle": (_V, [_LP, _I, _D, _LP, _I]),
     "interpolation_v2": (_V, [_LP, _I, _D, _LP, _I]), "interpolation_v4": (_V, [_LP, _I, _D, _LP, _I]),
+    "interpolation_p0": (_V, [_LP, _I, _D, _LP, _I]),
     "exchange_boundary": (_V, [_LP, _I, _I]),
     "apply_BCs": (_V, [_LP, _I, _I]), "apply_BCs_v1": (_V, [_LP, _I, _I]),
     "apply_BCs_v2": (_V, [_LP, _I, _I]), "apply_BCs_v4": (_V, [_LP, _I, _I]),

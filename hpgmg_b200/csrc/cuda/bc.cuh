@@ -117,6 +117,17 @@ __device__ __forceinline__ void bc_v2_col_zero_rest(const double *r, double *w, 
   w[0] = v;
 }
 
+/* the v2 column of a ghost fill: fv4 levels have 2 ghost layers and zero the deeper one (above); fv2 levels (-DHPGMG_FV2) have
+ * one, and there is nothing deeper to zero */
+__device__ __forceinline__ void bc_v2_fill_col(const double *r, double *w, const int m, const int d0, const int d1, const int d2)
+{
+#ifdef HPGMG_FV2
+  bc_v2_col(r, w, m, d0, d1, d2);
+#else
+  bc_v2_col_zero_rest(r, w, m, d0, d1, d2);
+#endif
+}
+
 /* the normal axes of a domain normal `subtype` (0..26 = 13+di+3dj+9dk): their count and inward strides */
 struct BCNormal {
   int m, d[3];

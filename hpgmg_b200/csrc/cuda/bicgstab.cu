@@ -43,11 +43,11 @@ extern "C" int hpgmg_bicgstab_device_eligible(const level_type *level)
   if (level->boundary_condition.type != BC_DIRICHLET) return 0;
   if (level->num_my_boxes != 1) return 0;
   if (level->boxes_in.i != 1 || level->boxes_in.j != 1 || level->boxes_in.k != 1) return 0;
-  if (level->box_dim > BOTTOM_MAX_DIM || level->box_dim < 2) return 0;
-  if (level->box_ghosts != 2) return 0;
+  if (level->box_dim > BOTTOM_MAX_DIM || level->box_dim < STENCIL_RADIUS) return 0;      /* fv4: 2^3 and up; fv2: 1^3 and up */
+  if (level->box_ghosts != STENCIL_RADIUS) return 0;
   const hpgmg_device_level *D = HPGMG_DEV(level);
   /* the fill tables are rebuilt for the new vector count when IterativeSolver grows the level (create_vectors) */
-  if (D->fill_nvec == 0 || D->fill[STENCIL_SHAPE_NO_CORNERS].nlate > 0) return 0;
+  if (D->fill_nvec == 0 || D->fill[STENCIL_SHAPE].nlate > 0) return 0;
   return 1;
 }
 
@@ -58,7 +58,7 @@ extern "C" int hpgmg_bicgstab_device(level_type *level, int x_id, int R_id, doub
   BottomArgs A;
   A.L = D->L;
   if (D->fill_nvec != level->numVectors) return 0;
-  A.bc = D->fill[STENCIL_SHAPE_NO_CORNERS].bc;  A.nbc = D->fill[STENCIL_SHAPE_NO_CORNERS].nbc;
+  A.bc = D->fill[STENCIL_SHAPE].bc;  A.nbc = D->fill[STENCIL_SHAPE].nbc;
   A.x_id = x_id;  A.R_id = R_id;  A.a = a;  A.b = b;
   A.ids = bottom_ids_identity();
   A.h2inv = 1.0 / (level->h * level->h);

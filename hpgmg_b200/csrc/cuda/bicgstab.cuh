@@ -28,7 +28,7 @@ __host__ __device__ __forceinline__ BottomIds bottom_ids_identity()
 
 struct BottomArgs {
   DLevel L;
-  const FillBC *bc;             /* NO_CORNERS BC columns of the (single) box: flat table (device_level.cu); offsets are relative to a vector's start */
+  const FillBC *bc;             /* BC columns of the flavour's stencil shape (NO_CORNERS; fv2: STAR) of the (single) box: flat table (device_level.cu); offsets are relative to a vector's start */
   int nbc;
   int x_id, R_id;
   BottomIds ids;
@@ -47,9 +47,20 @@ struct BottomCtx {
 
 __device__ static void b_fill_ghosts(const BottomCtx &C, const int id)
 {
-  /* exchange_boundary is empty for a single box with Dirichlet BCs; apply_BCs = v4 (v2 if dim<4) */
   const DLevel &L = C.A.L;
   double *v = L.base + (size_t)id * (size_t)L.volume;
+#ifdef HPGMG_FV2
+  /* fv2: apply_BCs_v2 on the STAR shape, one ghost layer (nothing deeper to zero); v1 on a 1^3 box (boundary_fv.c:6-90: a face
+   * ghost cell is minus the cell behind it) */
+  const bool v1 = C.n < 2;
+  for (int e = threadIdx.x; e < C.A.nbc; e += blockDim.x) {
+    const FillBC it = C.A.bc[e];
+    const BCNormal N = bc_normal(it.subtype, L.jStride, L.kStride);
+    if (v1) v[it.dst] = -1.0 * v[it.src + N.d[0]];
+    else    bc_v2_col(v + it.src, v + it.dst, N.m, N.d[0], N.d[1], N.d[2]);
+  }
+#else
+  /* exchange_boundary is empty for a single box with Dirichlet BCs; apply_BCs = v4 (v2 if dim<4) */
   const bool v2 = C.n < 4;
   for (int e = threadIdx.x; e < C.A.nbc; e += blockDim.x) {
     const FillBC it = C.A.bc[e];
@@ -57,6 +68,7 @@ __device__ static void b_fill_ghosts(const BottomCtx &C, const int id)
     if (v2) bc_v2_col_zero_rest(v + it.src, v + it.dst, N.m, N.d[0], N.d[1], N.d[2]);
     else    bc_v4_column(v + it.src, v + it.dst, N);
   }
+#endif
   __syncthreads();
 }
 
@@ -70,7 +82,7 @@ __device__ static void b_apply(const BottomCtx &C, const int out_id, const int i
   const double *rhs = L.vec(0, rhs_id);
   for (int c = threadIdx.x; c < C.cells; c += blockDim.x) {
     const int ijk = C.cell_offset(c);
-    const double Ax = fv4_apply_op(x + ijk, bi + ijk, bj + ijk, bk + ijk, C.jS, C.kS, C.A.b, C.A.h2inv);
+    const double Ax = op_apply(x + ijk, bi + ijk, bj + ijk, bk + ijk, C.jS, C.kS, C.A.b, C.A.h2inv);
     out[ijk] = mode ? rhs[ijk] - Ax : Ax;
   }
   __syncthreads();
@@ -302,7 +314,7 @@ __device__ static double b_apply_dot(BottomCtx &C, const int out_id, const int i
   double *out = L.vec(0, out_id);
   for (int c = threadIdx.x; c < C.cells; c += blockDim.x) {
     const int ijk = C.cell_offset(c);
-    const double Ax = fv4_apply_op(x + ijk, bi + ijk, bj + ijk, bk + ijk, C.jS, C.kS, C.A.b, C.A.h2inv);
+    const double Ax = op_apply(x + ijk, bi + ijk, bj + ijk, bk + ijk, C.jS, C.kS, C.A.b, C.A.h2inv);
     out[ijk] = Ax;
     C.prod[c] = Ax * x[ijk];
   }

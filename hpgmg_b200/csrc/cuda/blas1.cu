@@ -91,8 +91,14 @@ static void launch_blas1(level_type *level, BlasArgs &A)
   LAUNCH(blas1_kernel<OP>, dim3(bx, L.nboxes), 256, 0, A);
 }
 
+/* The 16-byte pairs of B_ZERO start at ghost cell -g of a row; create_vectors aligns cell 0, so with an odd number of ghost
+ * layers (fv2) they are misaligned: there the whole box is zeroed as init_vector(0.0) does it, one double at a time. */
 extern "C" void zero_vector(level_type *level, int id_a)
-{ BlasArgs A = {}; ProfileScope prof_(&level->timers.blas1); A.c = id_a; launch_blas1<B_ZERO>(level, A); }
+{
+  BlasArgs A = {}; ProfileScope prof_(&level->timers.blas1); A.c = id_a;
+  if (level->box_ghosts & 1) launch_blas1<B_INIT>(level, A);
+  else                       launch_blas1<B_ZERO>(level, A);
+}
 extern "C" void init_vector(level_type *level, int id_a, double scalar)
 { BlasArgs A = {}; ProfileScope prof_(&level->timers.blas1); A.c = id_a; A.sa = scalar; launch_blas1<B_INIT>(level, A); }
 extern "C" void scale_vector(level_type *level, int id_c, double scale_a, int id_a)

@@ -546,6 +546,9 @@ extern "C" int hpgmg_coarse_chain_eligible(mg_type *MG, int from)
 #ifdef VECTOR_ALPHA
   return 0;                                        /* Helmholtz build: the global-memory kernels carry the a*alpha*x term */
 #endif
+#ifdef HPGMG_FV2
+  return 0;                                        /* fv2 build: the coarse kernel's phases are written for the fv4 operator and 2 ghost layers */
+#endif
   const int bottom = MG->num_levels - 1;
   if (from > bottom || bottom - from + 1 > COARSE_MAX_LEVELS) return 0;
   if (coarse_program_length(bottom - from + 1, 1) > COARSE_MAX_PHASES) return 0;
@@ -634,7 +637,7 @@ extern "C" void hpgmg_coarse_cycle(mg_type *MG, int from, int mode_ftail, int ze
     for (int e = 0; e < Cr->num_blocks[1]; e++) { const int c = Cr->blocks[1][e].dim.i * Cr->blocks[1][e].dim.j * Cr->blocks[1][e].dim.k; if (c > V.restr_cells) V.restr_cells = c; }
     for (int e = 0; e < Ci->num_blocks[1]; e++) { const int c = Ci->blocks[1][e].dim.i * Ci->blocks[1][e].dim.j * Ci->blocks[1][e].dim.k; if (c > V.interp_cells) V.interp_cells = c; }
     V.h2inv = 1.0 / (level->h * level->h);
-    chebyshev_coefficients(level->dominant_eigenvalue_of_DinvA, V.c1, V.c2);
+    chebyshev_coefficients(level->dominant_eigenvalue_of_DinvA, CHEBYSHEV_DEGREE, V.c1, V.c2);
     V.jw = jacobi_weight(A.smoother);
     const bool l1jacobi = A.smoother == HPGMG_SMOOTHER_L1JACOBI;
     V.l1 = l1jacobi ? hpgmg_l1inv_array(level) : NULL;

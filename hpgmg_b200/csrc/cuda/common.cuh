@@ -177,6 +177,7 @@ struct hpgmg_device_level {
   int    restrict_map_state;                    /* 0 not looked at yet, 1 available, -1 the level's restriction is not box-to-box on this GPU */
   double *l1inv;                                /* default build, L1-Jacobi only: the L1 row inverse, [box][k][j][i] with the geometry of one
                                                    slab vector (the vector map has no room for it); written by rebuild_operator_blackbox */
+  double *l1inv_alloc;                          /* the allocation l1inv lies in */
   double *tile_partials;                        /* scratch for dot/mean: one double per compute tile */
   blockCopy_type *tiles;                        /* device copy of level->my_blocks                  */
   int     ntiles;

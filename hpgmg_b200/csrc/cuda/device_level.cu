@@ -7,6 +7,7 @@
 #include <vector>
 #include <algorithm>
 #include "common.cuh"
+#include "stencil.cuh"
 
 static void upload_list(DList *dst, const blockCopy_type *src, int n)
 {
@@ -129,7 +130,7 @@ static void build_fill_tables(level_type *level, hpgmg_device_level *D)
 {
   free_fill_tables(D);
   D->fill_nvec = level->numVectors;
-  if (level->num_my_boxes == 0 || level->box_ghosts != 2) return;
+  if (level->num_my_boxes == 0 || level->box_ghosts != STENCIL_RADIUS) return;      /* 2 ghost layers (fv4) or 1 (fv2) */
   const int jS = level->box_jStride, kS = level->box_kStride, n = level->box_dim, g = level->box_ghosts;
   const long per_box = (long)level->numVectors * level->box_volume;
   const long origin = (long)g * (1 + jS + kS);
@@ -200,11 +201,13 @@ static void build_fill_tables(level_type *level, hpgmg_device_level *D)
       build_tile_table(level, D, copies, now);
     FillTable &T = D->fill[s];
     {
-      /* pairs for the fill kernel (FillTable, common.cuh).  Offsets count doubles from a 16-byte aligned base and strides are
-       * even, so an even offset is a 16-byte aligned address. */
+      /* pairs for the fill kernel (FillTable, common.cuh).  Offsets count doubles from the start of a box vector; create_vectors
+       * aligns cell 0 (offset `origin`) to 16 bytes and strides are even, so an offset of origin's parity is a 16-byte aligned
+       * address (any even offset with 2 ghost layers, any odd one with 1). */
+      const int odd = (int)(origin & 1);
       std::vector<FillCopy> c2, c1;
       for (size_t e = 0; e < copies.size(); e++) {
-        if (e + 1 < copies.size() && (copies[e].src & 1) == 0 && (copies[e].dst & 1) == 0 && copies[e + 1].src == copies[e].src + 1 && copies[e + 1].dst == copies[e].dst + 1) {
+        if (e + 1 < copies.size() && ((copies[e].src ^ odd) & 1) == 0 && ((copies[e].dst ^ odd) & 1) == 0 && copies[e + 1].src == copies[e].src + 1 && copies[e + 1].dst == copies[e].dst + 1) {
           c2.push_back(copies[e]);
           e++;
         } else c1.push_back(copies[e]);
@@ -212,7 +215,7 @@ static void build_fill_tables(level_type *level, hpgmg_device_level *D)
       std::vector<FillBC> b2, b1;
       for (size_t e = 0; e < now.size(); e++) {
         const bool i_tangential = (now[e].subtype % 3) == 1;                    /* the domain normal has no i component */
-        if (i_tangential && e + 1 < now.size() && (now[e].src & 1) == 0 && (now[e].dst & 1) == 0 && now[e + 1].subtype == now[e].subtype &&
+        if (i_tangential && e + 1 < now.size() && ((now[e].src ^ odd) & 1) == 0 && ((now[e].dst ^ odd) & 1) == 0 && now[e + 1].subtype == now[e].subtype &&
             now[e + 1].src == now[e].src + 1 && now[e + 1].dst == now[e].dst + 1) {
           b2.push_back(now[e]);
           e++;
@@ -310,7 +313,7 @@ extern "C" void hpgmg_device_level_destroy(level_type *level)
   free_fill_tables(D);
   if (D->low) CUDA_CHECK(cudaFree(D->low));
   if (D->restrict_map) CUDA_CHECK(cudaFree(D->restrict_map));
-  if (D->l1inv) hpgmg_rt_free(D->l1inv);
+  if (D->l1inv_alloc) hpgmg_rt_free(D->l1inv_alloc);
   if (D->tiles) CUDA_CHECK(cudaFree(D->tiles));
   if (D->tile_partials) CUDA_CHECK(cudaFree(D->tile_partials));
   free(D);

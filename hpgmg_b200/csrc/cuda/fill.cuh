@@ -19,7 +19,7 @@ __device__ __forceinline__ void fill_items(const DLevel &L, const int id, const 
     const FillBC it = bc[t - ncopies];
     const BCNormal N = bc_normal(it.subtype, L.jStride, L.kStride);
     if (version == 4) bc_v4_column(v + it.src, v + it.dst, N);
-    else              bc_v2_col_zero_rest(v + it.src, v + it.dst, N.m, N.d[0], N.d[1], N.d[2]);
+    else              bc_v2_fill_col(v + it.src, v + it.dst, N.m, N.d[0], N.d[1], N.d[2]);
   }
 }
 

@@ -4,7 +4,7 @@
  * averages) and the extrapolation of the face coefficients.
  *
  *   exchange_boundary   operators/exchange_boundary.c:12-117 + CopyBlock operators/blockCopy.c:6-105
- *   apply_BCs_v1/v2/v4  operators/boundary_fv.c:6-90 / 101-250 / 262-569 (apply_BCs = v4, operators.fv4.c:51)
+ *   apply_BCs_v1/v2/v4  operators/boundary_fv.c:6-90 / 101-250 / 262-569 (apply_BCs = v4, operators.fv4.c:51; v2 in the fv2 build)
  *   extrapolate_betas   operators/boundary_fv.c:573-681
  *
  * The kernels walk the device copies of the SAME block lists the reference walks (level.c:367-465,
@@ -16,6 +16,7 @@
  */
 #include <string.h>
 #include "common.cuh"
+#include "stencil.cuh"
 #include "p2p.cuh"
 
 /* ---- copy lists ------------------------------------------------------------------------------ */
@@ -57,7 +58,7 @@ extern "C" void exchange_boundary(level_type *level, int id, int shape)
     const blockCopy_type *pack, *unpack;
     int npack, nunpack;
     P2PPlan *plan;
-    if (D->fill_nvec == level->numVectors && level->box_ghosts == 2 && hpgmg_comm_p2p_lookup(level, shape, &pack, &npack, &unpack, &nunpack, &plan)) {
+    if (D->fill_nvec == level->numVectors && level->box_ghosts == STENCIL_RADIUS && hpgmg_comm_p2p_lookup(level, shape, &pack, &npack, &unpack, &nunpack, &plan)) {
       hpgmg_fill_ghosts(level, id, shape, 0);                              /* peer stores over NVLink, no BCs */
       return;
     }
@@ -92,7 +93,7 @@ __global__ void __launch_bounds__(128) bc_v2_kernel(const DLevel L, const int id
  * normal (boundary_fv.c:6-90).  With two ghost layers a deeper ghost reads a shallower one, possibly
  * of ANOTHER block, so the result depends on the order: the whole list is walked by one thread in
  * list order with k,j,i ascending inside a block -- the reference run on one thread.  The path only
- * exists for box_dim<2, which the radius-2 fv4 stencil never produces; kept for API completeness. */
+ * runs for box_dim<2: the 1^3 bottom of an fv2 hierarchy (the radius-2 fv4 stencil never produces one). */
 __global__ void bc_v1_kernel(const DLevel L, const int id, const blockCopy_type *__restrict__ blocks, const int nblocks)
 {
   PDL_WAIT();
@@ -127,7 +128,8 @@ __global__ void bc_v1_kernel(const DLevel L, const int id, const blockCopy_type 
  *   [.., +late blocks)         the BC columns that read those ghost cells: they wait on an in-kernel
  *                              counter until every unpack block has finished.              [multi-GPU]
  * Blocks are dispatched in index order, so a waiting block never keeps the block it waits for off the
- * machine.  version: 4 quartic, 2 quadratic (also zeroes the deeper ghost layer, like the reference). */
+ * machine.  version: 4 quartic, 2 quadratic (also zeroes the deeper ghost layer of a 2-layer level, like the reference).
+ * The tables exist for levels of STENCIL_RADIUS ghost layers: 2 (fv4) or 1 (fv2). */
 #include "fill.cuh"
 
 struct FillArgs {
@@ -215,8 +217,8 @@ __device__ __forceinline__ void fill_block(const FillArgs &A, int fb)
         if (N.m == 1) bc_v4_col1_x2(v + it.src, v + it.dst, N.d[0]);
         else          bc_v4_col2_x2(v + it.src, v + it.dst, N.d[0], N.d[1]);
       } else {
-        bc_v2_col_zero_rest(v + it.src, v + it.dst, N.m, N.d[0], N.d[1], N.d[2]);
-        bc_v2_col_zero_rest(v + it.src + 1, v + it.dst + 1, N.m, N.d[0], N.d[1], N.d[2]);
+        bc_v2_fill_col(v + it.src, v + it.dst, N.m, N.d[0], N.d[1], N.d[2]);
+        bc_v2_fill_col(v + it.src + 1, v + it.dst + 1, N.m, N.d[0], N.d[1], N.d[2]);
       }
     }
   } else {                                                           /* ---- single BC columns ---- */
@@ -296,7 +298,9 @@ void hpgmg_fill_ghosts(level_type *level, int id, int shape, int bc_version)
   if (version == 4 && level->box_dim < 4) version = 2;
   communicator_type *C = &level->exchange_ghosts[shape];
   const bool remote = level->num_ranks > 1 && (C->num_sends > 0 || C->num_recvs > 0);
-  const bool have_tables = D->fill_nvec == level->numVectors && level->box_ghosts == 2 && !(version == 2 && level->box_dim < 2);
+  /* v4 needs 2 ghost layers: on a 1-layer level the list path's apply_BCs_v4 refuses it as the reference does */
+  const bool have_tables = D->fill_nvec == level->numVectors && level->box_ghosts == STENCIL_RADIUS && !(version == 2 && level->box_dim < 2) &&
+                           !(version == 4 && level->box_ghosts < 2);
   const blockCopy_type *pack = NULL, *unpack = NULL;
   int npack = 0, nunpack = 0;
   P2PPlan *plan = NULL;
@@ -357,7 +361,11 @@ extern "C" void apply_BCs_v4(level_type *level, int x_id, int shape)
   if (list.n > 0) LAUNCH(bc_v4_kernel, list.n, 128, 0, dl_of(level), x_id, list.blocks);
 }
 
+#ifdef HPGMG_FV2
+extern "C" void apply_BCs(level_type *level, int x_id, int shape) { apply_BCs_v2(level, x_id, shape); }
+#else
 extern "C" void apply_BCs(level_type *level, int x_id, int shape) { apply_BCs_v4(level, x_id, shape); }
+#endif
 
 /* ---- face coefficients beyond the domain ------------------------------------------------------- */
 /* boundary_fv.c:573-681.  Uses the BOX-shape BC list only to know which ghost regions lie outside

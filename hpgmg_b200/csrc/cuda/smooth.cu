@@ -72,7 +72,7 @@ __global__ void __launch_bounds__(256) stencil_generic_kernel(const StencilArgs 
     double *__restrict__ out = L.vec(box, A.out_id) + ijk;
     const int color000 = gsrb_box_parity(A.low, box, A.sweep);
     if (((i ^ j ^ k ^ color000) & 1) == 0) {
-      const double Ax = HELMHOLTZ_TERM(A.a, L.vec(box, VECTOR_ALPHA_OR_0)[ijk], x[0]) fv4_apply_op(x, bi, bj, bk, jS, kS, A.b, A.h2inv);
+      const double Ax = HELMHOLTZ_TERM(A.a, L.vec(box, VECTOR_ALPHA_OR_0)[ijk], x[0]) op_apply(x, bi, bj, bk, jS, kS, A.b, A.h2inv);
       const double dinv = L.vec(box, VECTOR_DINV)[ijk];
       const double rhs = L.vec(box, A.rhs_id)[ijk];
       out[0] = gsrb_update(x[0], dinv, rhs, Ax);
@@ -81,7 +81,7 @@ __global__ void __launch_bounds__(256) stencil_generic_kernel(const StencilArgs 
     }
     return;
   }
-  const double Ax = HELMHOLTZ_TERM(A.a, L.vec(box, VECTOR_ALPHA_OR_0)[ijk], x[0]) fv4_apply_op(x, bi, bj, bk, jS, kS, A.b, A.h2inv);
+  const double Ax = HELMHOLTZ_TERM(A.a, L.vec(box, VECTOR_ALPHA_OR_0)[ijk], x[0]) op_apply(x, bi, bj, bk, jS, kS, A.b, A.h2inv);
   if (OP == OP_APPLY) {
     L.vec(box, A.out_id)[ijk] = Ax;
   } else if (OP == OP_RESIDUAL) {
@@ -236,14 +236,14 @@ __global__ void __launch_bounds__(256) stencil_pair_kernel(const StencilArgs A)
     const int a = (j ^ k ^ gsrb_box_parity(A.low, box, A.sweep)) & 1;     /* the active cell of the pair */
     const double2 rhs2 = *reinterpret_cast<const double2 *>(L.vec(box, A.rhs_id) + ijk);
     const double2 dinv2 = *reinterpret_cast<const double2 *>(L.vec(box, VECTOR_DINV) + ijk);
-    const double Ax = HELMHOLTZ_TERM(A.a, L.vec(box, VECTOR_ALPHA_OR_0)[ijk + a], x[a]) fv4_apply_op(x + a, bi + a, bj + a, bk + a, jS, kS, A.b, A.h2inv);
+    const double Ax = HELMHOLTZ_TERM(A.a, L.vec(box, VECTOR_ALPHA_OR_0)[ijk + a], x[a]) op_apply(x + a, bi + a, bj + a, bk + a, jS, kS, A.b, A.h2inv);
     const double xnew = gsrb_update(x[a], a ? dinv2.y : dinv2.x, a ? rhs2.y : rhs2.x, Ax);
     const double xo = x[1 - a];
     *out = a ? make_double2(xo, xnew) : make_double2(xnew, xo);
     return;
   }
-  const double Ax0 = HELMHOLTZ_TERM(A.a, L.vec(box, VECTOR_ALPHA_OR_0)[ijk], x[0]) fv4_apply_op(x, bi, bj, bk, jS, kS, A.b, A.h2inv);
-  const double Ax1 = HELMHOLTZ_TERM(A.a, L.vec(box, VECTOR_ALPHA_OR_0)[ijk + 1], x[1]) fv4_apply_op(x + 1, bi + 1, bj + 1, bk + 1, jS, kS, A.b, A.h2inv);
+  const double Ax0 = HELMHOLTZ_TERM(A.a, L.vec(box, VECTOR_ALPHA_OR_0)[ijk], x[0]) op_apply(x, bi, bj, bk, jS, kS, A.b, A.h2inv);
+  const double Ax1 = HELMHOLTZ_TERM(A.a, L.vec(box, VECTOR_ALPHA_OR_0)[ijk + 1], x[1]) op_apply(x + 1, bi + 1, bj + 1, bk + 1, jS, kS, A.b, A.h2inv);
   if (OP == OP_APPLY) { *out = make_double2(Ax0, Ax1); return; }
   const double2 rhs2 = *reinterpret_cast<const double2 *>(L.vec(box, A.rhs_id) + ijk);
   if (OP == OP_RESIDUAL) { *out = make_double2(rhs2.x - Ax0, rhs2.y - Ax1); return; }
@@ -257,6 +257,10 @@ __global__ void __launch_bounds__(256) stencil_pair_kernel(const StencilArgs A)
   *out = make_double2(chebyshev_update(x[0], xm.x, A.c1, A.c2, dinv2.x, rhs2.x, Ax0),
                       chebyshev_update(x[1], xm.y, A.c1, A.c2, dinv2.y, rhs2.y, Ax1));
 }
+
+#ifdef HPGMG_FV2
+#include "stencil_fv2.cuh"
+#endif
 
 template <int OP>
 static void launch_stencil(level_type *level, StencilArgs &A)
@@ -278,7 +282,11 @@ static void launch_stencil(level_type *level, StencilArgs &A)
   A.diag = 0;                                                                     /* the diagonal carries a*alpha */
 #endif
   if (OP != OP_REBUILD && !g_force_generic) {
-#ifndef VECTOR_ALPHA
+#if defined(HPGMG_FV2)
+    A.diag = 0;                                                                   /* the shortcut is written for the fv4 TMA kernel */
+    if constexpr (OP != OP_REBUILD)
+      if (n % 32 == 0 && g_tma) { launch_fv2_march<OP>(A); return; }             /* boxes of 32^3 .. 256^3: the 7-point k-marching kernel */
+#elif !defined(VECTOR_ALPHA)
     if (n % 32 == 0 && g_tma) { launch_tma<OP, 32, 8, 1, 4>(A); return; }       /* boxes of 32^3 .. 256^3 */
 #endif
     if ((n & 1) == 0 && n >= 4 && g_pair_kernel) {
@@ -301,7 +309,7 @@ static void launch_stencil(level_type *level, StencilArgs &A)
 void hpgmg_fill_ghosts(level_type *level, int id, int shape, int bc_version);   /* ghost.cu */
 static void fill_ghosts(level_type *level, int id)
 {
-  hpgmg_fill_ghosts(level, id, STENCIL_SHAPE_NO_CORNERS, 4);    /* exchange_boundary + apply_BCs, fused */
+  hpgmg_fill_ghosts(level, id, STENCIL_SHAPE, SMOOTH_BC_VERSION);    /* exchange_boundary + apply_BCs, fused */
 }
 
 /* ---- ghost fill + operator in one launch (stencil_box.cuh) where the level allows it ---------------- */
@@ -331,6 +339,9 @@ static int try_launch_box(level_type *level, const StencilArgs &S, const int wri
 #ifdef VECTOR_ALPHA
   return 0;
 #endif
+#ifdef HPGMG_FV2
+  return 0;                                       /* the fill-fused box kernels stage the fv4 stencil with 2-cell halos */
+#endif
   if (g_force_generic || n > g_box_fused_max || T.ntiles == 0 || level->num_my_boxes == 0) return 0;
   if (D->fill_nvec != level->numVectors || level->box_ghosts != 2 || level->box_jStride != ((n + 4 + 3) / 4) * 4) return 0;
   if (hpgmg_ablate(n < 64 ? 8 : 64)) return 1;
@@ -352,8 +363,8 @@ static void fill_and_stencil(level_type *level, StencilArgs &A, const int write_
   launch_stencil<OP>(level, A);
 }
 
-extern "C" int stencil_get_radius(void) { return 2; }
-extern "C" int stencil_get_shape(void) { return STENCIL_SHAPE_NO_CORNERS; }
+extern "C" int stencil_get_radius(void) { return STENCIL_RADIUS; }
+extern "C" int stencil_get_shape(void) { return STENCIL_SHAPE; }
 
 extern "C" void apply_op(level_type *level, int Ax_id, int x_id, double a, double b)
 {
@@ -417,7 +428,7 @@ extern "C" void hpgmg_residual_then_restriction(level_type *level_c, int rc_id, 
   stencil_env();
   const int n = level->box_dim;
   const int *rmap = NULL;
-#ifndef VECTOR_ALPHA
+#if !defined(VECTOR_ALPHA) && !defined(HPGMG_FV2)          /* OP_RESRES exists in the fv4 TMA kernel only */
   if (fuse && !hpgmg_rt_profile() && !g_force_generic && g_tma && n % 32 == 0 && level->num_my_boxes > 0 && level_c->num_my_boxes > 0 && !hpgmg_ablate(32))
     rmap = restriction_map(level, level_c);
   /* the fused kernel pairs planes 2m, 2m+1 inside a block: k-chunks must be even (and not split by HPGMG_B200_TMA_BLOCKS) */
@@ -444,6 +455,9 @@ extern "C" void hpgmg_residual_norm_async(level_type *level, int res_id, int x_i
 {
   static int fuse = -1;
   if (fuse < 0) { const char *e = getenv("HPGMG_B200_FUSE_NORM"); fuse = e ? atoi(e) : 1; }
+#ifdef HPGMG_FV2
+  fuse = 0;                                            /* the norm is fused into the fv4 TMA residual kernel only */
+#endif
   if (!fuse || hpgmg_rt_profile()) { residual(level, res_id, x_id, rhs_id, a, b); hpgmg_norm_async(level, res_id, slot); return; }
   double *s = hpgmg_rt_scalar_slots() + slot;
   CUDA_CHECK(cudaMemsetAsync(s, 0, sizeof(double), g_stream));
@@ -482,15 +496,17 @@ extern "C" void hpgmg_download_l1inv(level_type *level, int box, double *host)
 #endif
 }
 
-/* the arguments of sweep s (the GSRB colour, the Chebyshev step) of the smoother whose operator is op, src -> dst */
-static StencilArgs sweep_args(level_type *level, const int op, const int src, const int dst, const int rhs_id, const double a, const double b, const int s)
+/* the arguments of sweep s (the GSRB colour, the Chebyshev step) of the smoother whose operator is op, src -> dst; the Chebyshev
+ * polynomial has `degree` steps */
+static StencilArgs sweep_args(level_type *level, const int op, const int src, const int dst, const int rhs_id, const double a, const double b, const int s,
+                              const int degree)
 {
   StencilArgs A = {};
   A.x_id = src;  A.rhs_id = rhs_id;  A.out_id = dst;  A.a = a;  A.b = b;  A.sweep = s;
   if (op == OP_CHEBY) {
-    double c1[6], c2[6];
-    chebyshev_coefficients(level->dominant_eigenvalue_of_DinvA, c1, c2);
-    A.xm1_id = dst;  A.c1 = c1[s % 6];  A.c2 = c2[s % 6];            /* x_{n-1} aliases x_{n+1} (chebyshev.c:75-80) */
+    double c1[CHEBYSHEV_MAX_DEGREE], c2[CHEBYSHEV_MAX_DEGREE];
+    chebyshev_coefficients(level->dominant_eigenvalue_of_DinvA, degree, c1, c2);
+    A.xm1_id = dst;  A.c1 = c1[s % degree];  A.c2 = c2[s % degree];  /* x_{n-1} aliases x_{n+1} (chebyshev.c:75-80) */
   } else if (op == OP_JACOBI) {                                          /* lambda: Dinv, or the L1 row inverse */
     const DLevel &L = dl_of(level);
     A.weight = jacobi_weight(hpgmg_rt_smoother());
@@ -509,7 +525,7 @@ static StencilArgs sweep_args(level_type *level, const int op, const int src, co
 /* one GSRB sweep kernel alone (no ghost fill) */
 extern "C" void hpgmg_b200_gsrb_sweep(level_type *level, int src_id, int dst_id, int rhs_id, double a, double b, int s)
 {
-  StencilArgs A = sweep_args(level, OP_GSRB, src_id, dst_id, rhs_id, a, b, s);
+  StencilArgs A = sweep_args(level, OP_GSRB, src_id, dst_id, rhs_id, a, b, s, CHEBYSHEV_DEGREE);
   launch_stencil<OP_GSRB>(level, A);
 }
 
@@ -517,7 +533,7 @@ extern "C" void hpgmg_b200_gsrb_sweep(level_type *level, int src_id, int dst_id,
 extern "C" void hpgmg_b200_smoother_sweep(level_type *level, int src_id, int dst_id, int rhs_id, double a, double b, int s)
 {
   const int op = smoother_op(hpgmg_rt_smoother());
-  StencilArgs A = sweep_args(level, op, src_id, dst_id, rhs_id, a, b, s);
+  StencilArgs A = sweep_args(level, op, src_id, dst_id, rhs_id, a, b, s, CHEBYSHEV_DEGREE);
   switch (op) {
     case OP_CHEBY:  launch_stencil<OP_CHEBY>(level, A);  break;
     case OP_JACOBI: launch_stencil<OP_JACOBI>(level, A); break;
@@ -525,18 +541,16 @@ extern "C" void hpgmg_b200_smoother_sweep(level_type *level, int src_id, int dst
   }
 }
 
-/* GSRB: NUM_SMOOTHS=3 -> RBRBRB (operators.fv4.c:177-180); Chebyshev: degree 6 (:184); Jacobi: NUM_SMOOTHS=6 (:176-195).
- * Each is 6 sweeps x -> TEMP -> x, every one after a ghost fill of its source. */
-extern "C" void smooth(level_type *level, int x_id, int rhs_id, double a, double b)
+/* `sweeps` sweeps x -> TEMP -> x (an even number), every one after a ghost fill of its source; Chebyshev steps cycle through
+ * a polynomial of `degree` */
+static void smooth_sweeps(level_type *level, int x_id, int rhs_id, double a, double b, const int sweeps, const int degree)
 {
-  ProfileScope prof_(&level->timers.smooth);
-  hpgmg_note_vector_written(level, x_id);
   const int op = smoother_op(hpgmg_rt_smoother());
   if (op == OP_CHEBY && level->dominant_eigenvalue_of_DinvA <= 0.0 && level->my_rank == 0) fprintf(stderr, "dominant_eigenvalue_of_DinvA <= 0.0 !\n");
-  for (int s = 0; s < 6; s++) {
+  for (int s = 0; s < sweeps; s++) {
     const int src = (s & 1) == 0 ? x_id : VECTOR_TEMP;
     const int dst = (s & 1) == 0 ? VECTOR_TEMP : x_id;
-    StencilArgs A = sweep_args(level, op, src, dst, rhs_id, a, b, s);
+    StencilArgs A = sweep_args(level, op, src, dst, rhs_id, a, b, s, degree);
     A.reverse = g_zigzag ? (s & 1) : 0;                                  /* GSRB only (launch_tma): alternate sweeps march k downwards */
     switch (op) {
       case OP_CHEBY:  fill_and_stencil<OP_CHEBY>(level, A, 0);  break;
@@ -544,6 +558,15 @@ extern "C" void smooth(level_type *level, int x_id, int rhs_id, double a, double
       default:        fill_and_stencil<OP_GSRB>(level, A, 0);   break;
     }
   }
+}
+
+/* fv4: GSRB NUM_SMOOTHS=3 -> RBRBRB (operators.fv4.c:177-180); Chebyshev: degree 6 (:184); Jacobi: NUM_SMOOTHS=6 (:176-195).
+ * fv2: 4 sweeps of every smoother, Chebyshev degree 4 (stencil.cuh). */
+extern "C" void smooth(level_type *level, int x_id, int rhs_id, double a, double b)
+{
+  ProfileScope prof_(&level->timers.smooth);
+  hpgmg_note_vector_written(level, x_id);
+  smooth_sweeps(level, x_id, rhs_id, a, b, SMOOTH_SWEEPS, CHEBYSHEV_DEGREE);
 }
 
 /* ------------------------------------------------------------------------------------------ */
@@ -609,8 +632,12 @@ extern "C" void rebuild_operator_blackbox(level_type *level, double a, double b,
   /* the default vector map has no room for the L1 row inverse: an array of the level, made when L1-Jacobi is selected
    * and refreshed by every later rebuild */
   hpgmg_device_level *D = HPGMG_DEV(level);
-  if (!D->l1inv && L.nboxes > 0 && hpgmg_rt_smoother() == HPGMG_SMOOTHER_L1JACOBI)
-    D->l1inv = (double *)hpgmg_rt_alloc_zero((size_t)L.nboxes * L.volume * sizeof(double));
+  if (!D->l1inv && L.nboxes > 0 && hpgmg_rt_smoother() == HPGMG_SMOOTHER_L1JACOBI) {
+    /* cell 0 of every box 16-byte aligned, as in the slab (the pair kernel reads lambda in pairs): with an odd origin (one
+     * ghost layer) the array starts one double into its allocation */
+    D->l1inv_alloc = (double *)hpgmg_rt_alloc_zero(((size_t)L.nboxes * L.volume + 1) * sizeof(double));
+    D->l1inv = D->l1inv_alloc + (L.origin & 1);
+  }
   l1inv = D->l1inv;
 #endif
   if (L.nboxes > 0) {
@@ -639,13 +666,15 @@ extern "C" void rebuild_operator(level_type *level, level_type *fromLevel, doubl
     restriction(level, VECTOR_BETA_J, fromLevel, VECTOR_BETA_J, RESTRICT_FACE_J);
     restriction(level, VECTOR_BETA_K, fromLevel, VECTOR_BETA_K, RESTRICT_FACE_K);
   }
-  extrapolate_betas(level);
+#ifndef HPGMG_FV2
+  extrapolate_betas(level);                            /* fv2: the star stencil never reads a beta it would extrapolate */
+#endif
 #ifdef VECTOR_ALPHA
   exchange_boundary(level, VECTOR_ALPHA, STENCIL_SHAPE_BOX);
 #endif
   exchange_boundary(level, VECTOR_BETA_I, STENCIL_SHAPE_BOX);
   exchange_boundary(level, VECTOR_BETA_J, STENCIL_SHAPE_BOX);
   exchange_boundary(level, VECTOR_BETA_K, STENCIL_SHAPE_BOX);
-  rebuild_operator_blackbox(level, a, b, 4);
+  rebuild_operator_blackbox(level, a, b, BLACKBOX_COLORS);
   exchange_boundary(level, VECTOR_DINV, STENCIL_SHAPE_BOX);
 }

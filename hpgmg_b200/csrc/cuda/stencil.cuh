@@ -78,6 +78,56 @@ __device__ __forceinline__ double fv4_apply_op_at(const XL &X, const BIL &BI, co
   return -b * h2inv * (STENCIL_TWELFTH * axial + 0.25 * STENCIL_TWELFTH * mixed);
 }
 
+/* The 2nd-order variable-coefficient finite-volume operator (operators.fv2.c), the 7-point star over the same loaders:
+ *   A x = -b h^-2 ( beta_i[i+1]*(x[i+1]-x) + beta_i[i]*(x[i-1]-x) + the same in j and k ),  summed left to right in that order.
+ * aii (optional): the same expression on the unit vector at this cell, as rebuild_operator_blackbox accumulates it where the
+ * stencil does not reach a boundary-condition ghost cell. */
+template <class XL, class BIL, class BJL, class BKL>
+__device__ __forceinline__ double fv2_apply_op_at(const XL &X, const BIL &BI, const BJL &BJ, const BKL &BK, const double b, const double h2inv, double *aii = nullptr)
+{
+  const double xc = X(0, 0, 0);
+  const double bi0 = BI(0, 0, 0), bi1 = BI(1, 0, 0), bj0 = BJ(0, 0, 0), bj1 = BJ(0, 1, 0), bk0 = BK(0, 0, 0), bk1 = BK(0, 0, 1);
+  if (aii) *aii = -b * h2inv * (bi1 * (0.0 - 1.0) + bi0 * (0.0 - 1.0) + bj1 * (0.0 - 1.0) + bj0 * (0.0 - 1.0) + bk1 * (0.0 - 1.0) + bk0 * (0.0 - 1.0));
+  return -b * h2inv * (bi1 * (X(1, 0, 0) - xc) + bi0 * (X(-1, 0, 0) - xc)
+                     + bj1 * (X(0, 1, 0) - xc) + bj0 * (X(0, -1, 0) - xc)
+                     + bk1 * (X(0, 0, 1) - xc) + bk0 * (X(0, 0, -1) - xc));
+}
+
+/* ---- the flavour: which operator the library is built for (-DHPGMG_FV2: operators.fv2.c, otherwise operators.fv4.c) ----
+ * STENCIL_RADIUS is stencil_get_radius(), i.e. the ghost depth of every level MGBuild makes, and the only depth the flat
+ * fill tables and the fast kernels are built for; levels of another depth take the list-walking kernels.
+ * Values that could not be checked against operators.fv2.c are marked (unverified); each is defined here only. */
+#if defined(HPGMG_FV2) && defined(USE_HELMHOLTZ)
+#error "the fv2 flavour is built with the default vector map only"
+#endif
+#ifdef HPGMG_FV2
+#define STENCIL_RADIUS      1
+#define STENCIL_SHAPE       STENCIL_SHAPE_STAR
+#define SMOOTH_SWEEPS       4      /* (unverified) GSRB NUM_SMOOTHS 2 (RBRB), Jacobi / L1-Jacobi 4 sweeps, Chebyshev = its degree */
+#define CHEBYSHEV_DEGREE    4      /* (unverified) */
+#define BLACKBOX_COLORS     2      /* rebuild_operator_blackbox(level, a, b, 2): no two cells of a colour in one radius-1 star */
+#define SMOOTH_BC_VERSION   2      /* (unverified) apply_BCs = apply_BCs_v2 (v1 below 2^3) */
+#else
+#define STENCIL_RADIUS      2
+#define STENCIL_SHAPE       STENCIL_SHAPE_NO_CORNERS
+#define SMOOTH_SWEEPS       6      /* GSRB NUM_SMOOTHS 3 (RBRBRB), Jacobi NUM_SMOOTHS 6, Chebyshev degree 6 (operators.fv4.c:176-195) */
+#define CHEBYSHEV_DEGREE    6
+#define BLACKBOX_COLORS     4      /* operators.fv4.c:145-173 */
+#define SMOOTH_BC_VERSION   4      /* apply_BCs = apply_BCs_v4 (v2 below 4^3) */
+#endif
+#define CHEBYSHEV_MAX_DEGREE 6
+
+/* the operator of this flavour at one cell */
+template <class XL, class BIL, class BJL, class BKL>
+__device__ __forceinline__ double op_apply_at(const XL &X, const BIL &BI, const BJL &BJ, const BKL &BK, const double b, const double h2inv, double *aii = nullptr)
+{
+#ifdef HPGMG_FV2
+  return fv2_apply_op_at(X, BI, BJ, BK, b, h2inv, aii);
+#else
+  return fv4_apply_op_at(X, BI, BJ, BK, b, h2inv, aii);
+#endif
+}
+
 /* loader over a global-memory array: p points at cell ijk */
 struct GlobalLoader {
   const double *__restrict__ p;
@@ -95,6 +145,14 @@ __device__ __forceinline__ double fv4_apply_op(const double *__restrict__ x,
 {
   const GlobalLoader X = { x, jS, kS }, BI = { bi, jS, kS }, BJ = { bj, jS, kS }, BK = { bk, jS, kS };
   return fv4_apply_op_at(X, BI, BJ, BK, b, h2inv);
+}
+
+/* the same for the operator of this flavour */
+__device__ __forceinline__ double op_apply(const double *__restrict__ x, const double *__restrict__ bi, const double *__restrict__ bj, const double *__restrict__ bk,
+                                           const int jS, const int kS, const double b, const double h2inv)
+{
+  const GlobalLoader X = { x, jS, kS }, BI = { bi, jS, kS }, BJ = { bj, jS, kS }, BK = { bk, jS, kS };
+  return op_apply_at(X, BI, BJ, BK, b, h2inv);
 }
 
 /* ---- the smoothers at one cell: x the cell's value before the sweep, Ax = (A x) there; the reference's association order ---- */
@@ -125,8 +183,8 @@ __device__ __forceinline__ int gsrb_box_parity(const int *low, const int box, co
 }
 
 /* ---- the smoothers' per-level coefficients and operator codes (host) ---- */
-/* Chebyshev coefficients of the 6 steps, exactly as chebyshev.c:22-40 (degree 6, operators.fv4.c:184) */
-static inline void chebyshev_coefficients(const double dominant_eigenvalue_of_DinvA, double c1[6], double c2[6])
+/* Chebyshev coefficients of the `degree` steps (<= CHEBYSHEV_MAX_DEGREE), exactly as chebyshev.c:22-40 */
+static inline void chebyshev_coefficients(const double dominant_eigenvalue_of_DinvA, const int degree, double c1[], double c2[])
 {
   double beta = 1.000 * dominant_eigenvalue_of_DinvA;
   double alpha = 0.125000 * beta;
@@ -136,7 +194,7 @@ static inline void chebyshev_coefficients(const double dominant_eigenvalue_of_Di
   double rho_n = 1 / sigma;
   c1[0] = 0.0;
   c2[0] = 1 / theta;
-  for (int s = 1; s < 6; s++) {
+  for (int s = 1; s < degree; s++) {
     double rho_nm1 = rho_n;
     rho_n = 1.0 / (2.0 * sigma - rho_nm1);
     c1[s] = rho_n * rho_nm1;

@@ -121,7 +121,7 @@ extern "C" void restriction(level_type *level_c, int id_c, level_type *level_f, 
   }
 }
 
-/* ---- interpolation ---------------------------------------------------------------------------- */
+/* ---- interpolation (every kernel reads at most W/2 coarse ghost layers: v2 runs on 1- and 2-layer levels, v4 needs 2) ---------------------------------------------------------------------------- */
 /* 1-D volume-averaged prolongation of one coarse cell into its two children.
  * quadratic (v2): lo = c0 + 1/8 (c- - c+),  hi = c0 - 1/8 (c- - c+)
  * quartic  (v4): lo = c0 + 22/128 (c-1 - c+1) + -3/128 (c-2 - c+2),  hi = c0 - ... - ...            */
@@ -349,6 +349,52 @@ __global__ void __launch_bounds__(256) interpolation_march_kernel(const DLevel L
   }
 }
 
+/* ---- piecewise-constant prolongation (interpolation_p0): every fine cell = prescale*fine + its coarse parent; no ghost cells ---- */
+/* box -> box entries: one thread per fine i-pair (both cells share the parent), 16-byte accesses where the pair is aligned
+ * (create_vectors aligns cell 0, so: where the entry starts on an even fine cell) */
+__global__ void __launch_bounds__(256) interpolation_p0_kernel(const DLevel Lf, const int id_f, const double prescale,
+                                                               const DLevel Lc, const int id_c, const blockCopy_type *__restrict__ blocks)
+{
+  PDL_WAIT();
+  const blockCopy_type B = blocks[blockIdx.x];
+  const int di = B.dim.i, fj = 2 * B.dim.j, fk = 2 * B.dim.k;     /* coarse i (= fine pairs), fine j, fine k */
+  const int t = blockIdx.y * blockDim.x + threadIdx.x;
+  if (t >= di * fj * fk) return;
+  const int ii = t % di, j = (t / di) % fj, k = t / (di * fj);
+  const double c = Lc.vec(B.read.box, id_c)[(B.read.i + ii) + (B.read.j + (j >> 1)) * Lc.jStride + (B.read.k + (k >> 1)) * Lc.kStride];
+  double *w = Lf.vec(B.write.box, id_f) + (B.write.i + 2 * ii) + (B.write.j + j) * Lf.jStride + (B.write.k + k) * Lf.kStride;
+  if ((B.write.i & 1) == 0) {
+    double2 o = *reinterpret_cast<double2 *>(w);
+    o.x = prescale * o.x + c;  o.y = prescale * o.y + c;
+    *reinterpret_cast<double2 *>(w) = o;
+  } else {
+    w[0] = prescale * w[0] + c;  w[1] = prescale * w[1] + c;
+  }
+}
+
+/* box -> MESSAGE entries: the sender interpolates into the message with prescale 0.0, i.e. 0.0*old + value; `old` is read from
+ * the rank's own send buffer when the message goes straight into the receiver's memory (see interpolation_pack_kernel) */
+__global__ void __launch_bounds__(128) interpolation_p0_pack_kernel(const DLevel Lc, const int id_c, const blockCopy_type *__restrict__ blocks,
+                                                                    const blockCopy_type *__restrict__ mirror_blocks)
+{
+  PDL_WAIT();
+  const blockCopy_type B = blocks[blockIdx.x];
+  const int rj = Lc.jStride, rk = Lc.kStride, wj = B.write.jStride, wk = B.write.kStride;
+  const double *__restrict__ rd = Lc.vec(B.read.box, id_c) + B.read.i + B.read.j * rj + B.read.k * rk;
+  const int w0 = B.write.i + B.write.j * wj + B.write.k * wk;
+  double *__restrict__ wr = B.write.ptr + w0;
+  double *__restrict__ mr = (mirror_blocks ? mirror_blocks[blockIdx.x].write.ptr : B.write.ptr) + w0;
+  const bool twice = mirror_blocks != nullptr;
+  const int fi = 2 * B.dim.i, fj = 2 * B.dim.j, cells = fi * fj * 2 * B.dim.k;
+  for (int c = threadIdx.x; c < cells; c += blockDim.x) {
+    const int i = c % fi, j = (c / fi) % fj, k = c / (fi * fj);
+    const int o = i + j * wj + k * wk;
+    const double v = 0.0 * mr[o] + rd[(i >> 1) + (j >> 1) * rj + (k >> 1) * rk];
+    wr[o] = v;
+    if (twice) mr[o] = v;
+  }
+}
+
 /* fine-level unpack of prolonged data received from another rank: write = prescale*write + recv
  * (IncrementBlock, blockCopy.c:108-156) */
 __global__ void __launch_bounds__(128) increment_blocks_kernel(const DLevel L, const int id, const double prescale, const blockCopy_type *__restrict__ blocks)
@@ -372,6 +418,15 @@ __global__ void __launch_bounds__(128) increment_blocks_kernel(const DLevel L, c
   }
 }
 
+/* the kernels of prolongation W: 1 piecewise constant (p0), 3 quadratic (v2), 5 quartic (v4) */
+template <int W>
+static void launch_interpolation_pack(const DLevel &Lc, const int id_c, const DList &list, const blockCopy_type *mirror)
+{
+  if (list.n <= 0) return;
+  if constexpr (W == 1) LAUNCH(interpolation_p0_pack_kernel, list.n, 128, 0, Lc, id_c, list.blocks, mirror);
+  else                  LAUNCH(interpolation_pack_kernel<W>, list.n, 128, 0, Lc, id_c, list.blocks, mirror);
+}
+
 template <int W>
 static void interpolation_driver(level_type *level_f, int id_f, double prescale_f, level_type *level_c, int id_c)
 {
@@ -388,16 +443,23 @@ static void interpolation_driver(level_type *level_f, int id_f, double prescale_
   if (remote && p2p) {
     if (p2p_send) {                                                  /* interpolate straight into the fine boxes' owners (comm.cu) */
       hpgmg_comm_xfer_pre(Cc);
-      if (peer_pack.n > 0) LAUNCH(interpolation_pack_kernel<W>, peer_pack.n, 128, 0, Dc->L, id_c, peer_pack.blocks, Dc->interpolation[0].blocks);
+      launch_interpolation_pack<W>(Dc->L, id_c, peer_pack, Dc->interpolation[0].blocks);
       hpgmg_comm_xfer_post(Cc);
     }
   } else if (remote) {
     const DList &pack = Dc->interpolation[0];
-    if (pack.n > 0) LAUNCH(interpolation_pack_kernel<W>, pack.n, 128, 0, Dc->L, id_c, pack.blocks, (const blockCopy_type *)NULL);
+    launch_interpolation_pack<W>(Dc->L, id_c, pack, (const blockCopy_type *)NULL);
     hpgmg_comm_transfer(level_c, Cc, level_f, Cf, 0x7);
   }
   const DList &local = Dc->interpolation[1];
-  if (local.n > 0) {
+  if constexpr (W == 1) {
+    if (local.n > 0) {
+      /* local entries are box -> box tiles of at most 10000 x 8 x 8 coarse cells (mg.c:274-277) */
+      const int half = level_f->box_dim / 2;
+      const int pairs = half * 2 * (half < BLOCKCOPY_TILE_J ? half : BLOCKCOPY_TILE_J) * 2 * (half < BLOCKCOPY_TILE_K ? half : BLOCKCOPY_TILE_K);
+      LAUNCH(interpolation_p0_kernel, dim3(local.n, (pairs + 255) / 256), dim3(256), 0, Df->L, id_f, prescale_f, Dc->L, id_c, local.blocks);
+    }
+  } else if (local.n > 0) {
     /* local entries are box -> box tiles of at most 10000 x 8 x 8 coarse cells (mg.c:274-277) */
     const int half = level_f->box_dim / 2;
     const int di = half, dj = half < BLOCKCOPY_TILE_J ? half : BLOCKCOPY_TILE_J, dk = half < BLOCKCOPY_TILE_K ? half : BLOCKCOPY_TILE_K;
@@ -430,11 +492,26 @@ extern "C" void interpolation_v4(level_type *level_f, int id_f, double prescale_
   interpolation_driver<5>(level_f, id_f, prescale_f, level_c, id_c);
 }
 
+/* interpolation_p0.c: reads only the coarse parents, so no ghost fill */
+extern "C" void interpolation_p0(level_type *level_f, int id_f, double prescale_f, level_type *level_c, int id_c)
+{
+  interpolation_driver<1>(level_f, id_f, prescale_f, level_c, id_c);
+}
+
+/* operators.fv4.c:204-205: v2 / v4; operators.fv2.c: p0 / v2 */
 extern "C" void interpolation_vcycle(level_type *level_f, int id_f, double prescale_f, level_type *level_c, int id_c)
 {
+#ifdef HPGMG_FV2
+  interpolation_p0(level_f, id_f, prescale_f, level_c, id_c);
+#else
   interpolation_v2(level_f, id_f, prescale_f, level_c, id_c);
+#endif
 }
 extern "C" void interpolation_fcycle(level_type *level_f, int id_f, double prescale_f, level_type *level_c, int id_c)
 {
+#ifdef HPGMG_FV2
+  interpolation_v2(level_f, id_f, prescale_f, level_c, id_c);
+#else
   interpolation_v4(level_f, id_f, prescale_f, level_c, id_c);
+#endif
 }

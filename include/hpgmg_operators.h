@@ -27,8 +27,8 @@ extern "C" {
 #define RESTRICT_FACE_J 2
 #define RESTRICT_FACE_K 3
 
-int stencil_get_radius(void);   /* 2                         operators.fv4.c:138 */
-int stencil_get_shape(void);    /* STENCIL_SHAPE_NO_CORNERS  operators.fv4.c:139 */
+int stencil_get_radius(void);   /* 2                         operators.fv4.c:138   (fv2 flavour: 1) */
+int stencil_get_shape(void);    /* STENCIL_SHAPE_NO_CORNERS  operators.fv4.c:139   (fv2 flavour: STENCIL_SHAPE_STAR) */
 
 /* operators/apply_op.c:9, residual.c:9, gsrb.c:24 | chebyshev.c:8, operators.fv4.c:145, rebuild.c:47 */
 void apply_op(level_type *level, int Ax_id, int x_id, double a, double b);
@@ -37,12 +37,14 @@ void smooth(level_type *level, int phi_id, int rhs_id, double a, double b);
 void rebuild_operator(level_type *level, level_type *fromLevel, double a, double b);
 void rebuild_operator_blackbox(level_type *level, double a, double b, int colors_in_each_dim);
 
-/* operators/restriction.c:104, interpolation_v2.c:210, interpolation_v4.c:276, operators.fv4.c:204-205 */
+/* operators/restriction.c:104, interpolation_v2.c:210, interpolation_v4.c:276, interpolation_p0.c, operators.fv4.c:204-205
+ * (vcycle = v2, fcycle = v4; in the fv2 flavour, operators.fv2.c: vcycle = p0, fcycle = v2).  v4 needs 2 ghost layers. */
 void restriction(level_type *level_c, int id_c, level_type *level_f, int id_f, int restrictionType);
 void interpolation_vcycle(level_type *level_f, int id_f, double prescale_f, level_type *level_c, int id_c);
 void interpolation_fcycle(level_type *level_f, int id_f, double prescale_f, level_type *level_c, int id_c);
 void interpolation_v2(level_type *level_f, int id_f, double prescale_f, level_type *level_c, int id_c);
 void interpolation_v4(level_type *level_f, int id_f, double prescale_f, level_type *level_c, int id_c);
+void interpolation_p0(level_type *level_f, int id_f, double prescale_f, level_type *level_c, int id_c);   /* fine = prescale*fine + coarse parent */
 
 /* operators/exchange_boundary.c:12, operators.fv4.c:51, boundary_fv.c:6,101,262,573 */
 void exchange_boundary(level_type *level, int id_a, int shape);
