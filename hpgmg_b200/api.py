@@ -21,6 +21,9 @@ LIB_PATH = os.path.join(_HERE, "lib", "libhpgmg_b200.so")
 # the 2nd-order operator (the reference linked with operators.fv2.c): one ghost layer, bind with bind(ctypes.CDLL(FV2_LIB_PATH))
 # and pass it as Hierarchy(..., library=...)
 FV2_LIB_PATH = os.path.join(_HERE, "lib", "libhpgmg_b200_fv2.so")
+# the same with -DUSE_HELMHOLTZ (the reference's operators.fv2.c with -DUSE_HELMHOLTZ): a*alpha*u - b*div(beta grad u), the
+# Helmholtz vector map (VECTOR_ALPHA 9, VECTOR_L1INV 10, VECTORS_RESERVED 11: pass vectors=11 to Hierarchy)
+FV2_HELMHOLTZ_LIB_PATH = os.path.join(_HERE, "lib", "libhpgmg_b200_fv2_helmholtz.so")
 
 # defines.h:28-38
 VECTOR_TEMP, VECTOR_U, VECTOR_F, VECTOR_E, VECTOR_R, VECTOR_DINV, VECTOR_BETA_I, VECTOR_BETA_J, VECTOR_BETA_K = range(9)

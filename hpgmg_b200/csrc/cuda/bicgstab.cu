@@ -36,8 +36,8 @@ __global__ void __launch_bounds__(BOTTOM_THREADS) cg_kernel(const BottomArgs A)
  * recorded into a CUDA graph: the host-driven fallback synchronises on every dot / norm) */
 extern "C" int hpgmg_bicgstab_device_eligible(const level_type *level)
 {
-#ifdef VECTOR_ALPHA
-  return 0;                                        /* Helmholtz build: host-driven BiCGStab over the public operators (solvers.c) */
+#if defined(VECTOR_ALPHA) && !defined(HPGMG_FV2)
+  return 0;                                        /* fv4 Helmholtz build: host-driven solvers over the public operators (solvers.c) */
 #endif
   if (level->must_subtract_mean == 1) return 0;
   if (level->boundary_condition.type != BC_DIRICHLET) return 0;

@@ -14,15 +14,23 @@
 #define BOTTOM_THREADS   256   /* the stand-alone kernel; the body works for any 1-D block that is a multiple of 32 (<=1024) */
 
 /* which vector of L plays which role: the identity (vector ids of the reference, bicgstab.c:17-24, defines.h:28-38) for the
- * stand-alone kernel; the coarse-cycle kernel keeps only the vectors a cycle touches in shared memory and passes their slots */
+ * stand-alone kernel; the coarse-cycle kernel keeps only the vectors a cycle touches in shared memory and passes their slots.
+ * alpha (Helmholtz builds) is set by the identity only: the coarse-cycle kernel does not run in those builds. */
 struct BottomIds {
   int r0, r, p, q, s, t, Ap, As;
   int dinv, temp, beta_i, beta_j, beta_k;
+#ifdef VECTOR_ALPHA
+  int alpha;
+#endif
 };
 __host__ __device__ __forceinline__ BottomIds bottom_ids_identity()
 {
   BottomIds I = { VECTORS_RESERVED + 0, VECTORS_RESERVED + 1, VECTORS_RESERVED + 2, VECTORS_RESERVED + 3, VECTORS_RESERVED + 4, VECTORS_RESERVED + 5,
-                  VECTORS_RESERVED + 6, VECTORS_RESERVED + 7, VECTOR_DINV, VECTOR_TEMP, VECTOR_BETA_I, VECTOR_BETA_J, VECTOR_BETA_K };
+                  VECTORS_RESERVED + 6, VECTORS_RESERVED + 7, VECTOR_DINV, VECTOR_TEMP, VECTOR_BETA_I, VECTOR_BETA_J, VECTOR_BETA_K,
+#ifdef VECTOR_ALPHA
+                  VECTOR_ALPHA
+#endif
+                };
   return I;
 }
 
@@ -72,7 +80,7 @@ __device__ static void b_fill_ghosts(const BottomCtx &C, const int id)
   __syncthreads();
 }
 
-/* out = A in   (mode 0)   or   out = rhs - A in   (mode 1) */
+/* out = A in   (mode 0)   or   out = rhs - A in   (mode 1); A carries a*alpha in the Helmholtz builds */
 __device__ static void b_apply(const BottomCtx &C, const int out_id, const int in_id, const int rhs_id, const int mode)
 {
   b_fill_ghosts(C, in_id);
@@ -80,9 +88,12 @@ __device__ static void b_apply(const BottomCtx &C, const int out_id, const int i
   const double *x = L.vec(0, in_id), *bi = L.vec(0, C.A.ids.beta_i), *bj = L.vec(0, C.A.ids.beta_j), *bk = L.vec(0, C.A.ids.beta_k);
   double *out = L.vec(0, out_id);
   const double *rhs = L.vec(0, rhs_id);
+#ifdef VECTOR_ALPHA
+  const double *alpha = L.vec(0, C.A.ids.alpha);
+#endif
   for (int c = threadIdx.x; c < C.cells; c += blockDim.x) {
     const int ijk = C.cell_offset(c);
-    const double Ax = op_apply(x + ijk, bi + ijk, bj + ijk, bk + ijk, C.jS, C.kS, C.A.b, C.A.h2inv);
+    const double Ax = HELMHOLTZ_TERM(C.A.a, alpha[ijk], x[ijk]) op_apply(x + ijk, bi + ijk, bj + ijk, bk + ijk, C.jS, C.kS, C.A.b, C.A.h2inv);
     out[ijk] = mode ? rhs[ijk] - Ax : Ax;
   }
   __syncthreads();
@@ -312,9 +323,12 @@ __device__ static double b_apply_dot(BottomCtx &C, const int out_id, const int i
   const DLevel &L = C.A.L;
   const double *x = L.vec(0, in_id), *bi = L.vec(0, C.A.ids.beta_i), *bj = L.vec(0, C.A.ids.beta_j), *bk = L.vec(0, C.A.ids.beta_k);
   double *out = L.vec(0, out_id);
+#ifdef VECTOR_ALPHA
+  const double *alpha = L.vec(0, C.A.ids.alpha);
+#endif
   for (int c = threadIdx.x; c < C.cells; c += blockDim.x) {
     const int ijk = C.cell_offset(c);
-    const double Ax = op_apply(x + ijk, bi + ijk, bj + ijk, bk + ijk, C.jS, C.kS, C.A.b, C.A.h2inv);
+    const double Ax = HELMHOLTZ_TERM(C.A.a, alpha[ijk], x[ijk]) op_apply(x + ijk, bi + ijk, bj + ijk, bk + ijk, C.jS, C.kS, C.A.b, C.A.h2inv);
     out[ijk] = Ax;
     C.prod[c] = Ax * x[ijk];
   }

@@ -14,17 +14,9 @@
 #include "common.cuh"
 #include "stencil.cuh"
 
-/* The Helmholtz build (-DUSE_HELMHOLTZ, as in the reference: operators.fv4.c:56-85): A x = a*alpha*x - b*h2inv*(...).  The
- * reference subtracts (b*h2inv)*(...) from a*alpha*x; fv4_apply_op returns (-b*h2inv)*(...), the exact negation, and
- * p - q == p + (-q) in IEEE arithmetic, so the sum below has the reference's bits.  In that build every operator goes
- * through the two global-memory kernels of this file (no TMA / fused-box / single-block paths). */
-#ifdef VECTOR_ALPHA
-#define HELMHOLTZ_TERM(a, alpha, x) (a) * (alpha) * (x) +
-#define VECTOR_ALPHA_OR_0 VECTOR_ALPHA
-#else
-#define HELMHOLTZ_TERM(a, alpha, x)
-#define VECTOR_ALPHA_OR_0 0
-#endif
+/* The Helmholtz builds carry a*alpha*x in every operator through HELMHOLTZ_TERM (stencil.cuh).  The fv4 Helmholtz build runs
+ * every operator through the two global-memory kernels of this file (no TMA / fused-box / single-block paths); the fv2
+ * Helmholtz build also runs the k-marching kernel of stencil_fv2.cuh and the single-block bottom solvers. */
 
 struct StencilArgs {
   DLevel L;

@@ -96,10 +96,8 @@ __device__ __forceinline__ double fv2_apply_op_at(const XL &X, const BIL &BI, co
 /* ---- the flavour: which operator the library is built for (-DHPGMG_FV2: operators.fv2.c, otherwise operators.fv4.c) ----
  * STENCIL_RADIUS is stencil_get_radius(), i.e. the ghost depth of every level MGBuild makes, and the only depth the flat
  * fill tables and the fast kernels are built for; levels of another depth take the list-walking kernels.
- * Values that could not be checked against operators.fv2.c are marked (unverified); each is defined here only. */
-#if defined(HPGMG_FV2) && defined(USE_HELMHOLTZ)
-#error "the fv2 flavour is built with the default vector map only"
-#endif
+ * Values that could not be checked against operators.fv2.c are marked (unverified); each is defined here only.
+ * Either operator combines with -DUSE_HELMHOLTZ (the Helmholtz vector map of hpgmg_defines.h and HELMHOLTZ_TERM below). */
 #ifdef HPGMG_FV2
 #define STENCIL_RADIUS      1
 #define STENCIL_SHAPE       STENCIL_SHAPE_STAR
@@ -127,6 +125,19 @@ __device__ __forceinline__ double op_apply_at(const XL &X, const BIL &BI, const 
   return fv4_apply_op_at(X, BI, BJ, BK, b, h2inv, aii);
 #endif
 }
+
+/* The Helmholtz build (-DUSE_HELMHOLTZ, as in the reference: operators.fv4.c:56-85, and operators.fv2.c in its Helmholtz form):
+ * A x = a*alpha*x - b*h2inv*(...).  Written before the operator, HELMHOLTZ_TERM(a, alpha, x) op_apply_at(...) forms that sum.
+ * The reference subtracts (b*h2inv)*(...) from a*alpha*x; op_apply_at returns (-b*h2inv)*(...), the exact negation, and
+ * p - q == p + (-q) in IEEE arithmetic, so the sum has the reference's bits.  Without VECTOR_ALPHA the term is empty and
+ * VECTOR_ALPHA_OR_0 only keeps the call sites compiling. */
+#ifdef VECTOR_ALPHA
+#define HELMHOLTZ_TERM(a, alpha, x) (a) * (alpha) * (x) +
+#define VECTOR_ALPHA_OR_0 VECTOR_ALPHA
+#else
+#define HELMHOLTZ_TERM(a, alpha, x)
+#define VECTOR_ALPHA_OR_0 0
+#endif
 
 /* loader over a global-memory array: p points at cell ijk */
 struct GlobalLoader {

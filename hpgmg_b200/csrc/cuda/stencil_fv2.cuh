@@ -6,8 +6,9 @@
  * coefficient beta_k of plane k+1 (the next cell's beta_k(k)) stay in registers, so each plane costs one new x, one rhs-side
  * value and the four in-plane x neighbours and the i+1 / j+1 betas, which neighbouring lanes of the same warp or tile have just
  * loaded: those come from L1, and HBM sees each array once -- 56 B per cell for GSRB and Jacobi, 64 for Chebyshev, 48 for
- * the residual, 40 for apply_op.  Staging is by plain loads: the halo is one cell deep, which L1 serves without shared memory
- * and without the barriers a TMA pipeline would need (DESIGN.md section 4).
+ * the residual, 40 for apply_op.  The Helmholtz build (-DUSE_HELMHOLTZ) also reads alpha at the cells that evaluate the stencil,
+ * 8 B more per cell for every operator.  Staging is by plain loads: the halo is one cell deep, which L1 serves without shared
+ * memory and without the barriers a TMA pipeline would need (DESIGN.md section 4).
  *
  * The arithmetic is op_apply_at and the smoother updates of stencil.cuh over loaders that read the register window, so the
  * results are bit-identical to the generic and pair kernels.
@@ -56,6 +57,9 @@ __global__ void __launch_bounds__(FV2_TI * FV2_TJ, 4) stencil_fv2_march_kernel(c
   const double *__restrict__ dinv = L.vec(box, VECTOR_DINV) + ij;
   const double *__restrict__ xm1 = L.vec(box, A.xm1_id) + ij;
   const double *__restrict__ lam = A.lam ? A.lam + (size_t)box * A.lam_bstride + ij : nullptr;
+#ifdef VECTOR_ALPHA
+  const double *__restrict__ alpha = L.vec(box, VECTOR_ALPHA) + ij;
+#endif
   const int color = (OP == OP_GSRB) ? ((i ^ j ^ gsrb_box_parity(A.low, box, A.sweep)) & 1) : 0;
 
   Fv2WindowX X = { x + k0 * kS, jS, x[(k0 - 1) * kS], x[k0 * kS], 0.0 };
@@ -71,7 +75,7 @@ __global__ void __launch_bounds__(FV2_TI * FV2_TJ, 4) stencil_fv2_march_kernel(c
     if (OP == OP_GSRB && ((k ^ color) & 1) != 0) {
       out[o] = X.xc;                                               /* not this sweep's colour */
     } else {
-      const double Ax = op_apply_at(X, BI, BJ, BK, A.b, A.h2inv);
+      const double Ax = HELMHOLTZ_TERM(A.a, alpha[o], X.xc) op_apply_at(X, BI, BJ, BK, A.b, A.h2inv);
       if (OP == OP_APPLY)         out[o] = Ax;
       else if (OP == OP_RESIDUAL) out[o] = rhs[o] - Ax;
       else if (OP == OP_GSRB)     out[o] = gsrb_update(X.xc, dinv[o], rhs[o], Ax);

@@ -453,7 +453,8 @@ void MGBuild(mg_type *MG, level_type *fine, double a, double b, int minCoarseGri
     /* Poisson-like with periodic BCs: the solution is only defined up to a constant (mg.c:1009-1018).  Without
      * VECTOR_ALPHA "alpha is zero" always holds. */
 #ifdef VECTOR_ALPHA
-    const int alpha_is_zero = (dot(L, VECTOR_ALPHA, VECTOR_ALPHA) == 0.0);
+    /* layout-only mode has no vector data to read: alpha counts as nonzero there */
+    const int alpha_is_zero = !hpgmg_rt_layout_only() && (dot(L, VECTOR_ALPHA, VECTOR_ALPHA) == 0.0);
     L->must_subtract_mean = (L->boundary_condition.type == BC_PERIODIC && (a == 0 || alpha_is_zero)) ? 1 : 0;
 #else
     L->must_subtract_mean = (L->boundary_condition.type == BC_PERIODIC) ? 1 : 0;
