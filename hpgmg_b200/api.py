@@ -47,7 +47,7 @@ _D, _I, _V = C.c_double, C.c_int, None
 SIGNATURES = {
     # hpgmg_b200.h
     "hpgmg_b200_init": (_I, [_I]), "hpgmg_b200_finalize": (_V, []), "hpgmg_b200_sync": (_V, []),
-    "hpgmg_b200_backend": (C.c_char_p, []),
+    "hpgmg_b200_backend": (C.c_char_p, []), "hpgmg_b200_device": (_I, []),
     "hpgmg_b200_set_smoother": (_V, [_I]), "hpgmg_b200_get_smoother": (_I, []),
     "hpgmg_b200_set_bottom_solver": (_V, [_I]), "hpgmg_b200_get_bottom_solver": (_I, []),
     "hpgmg_b200_set_verbose": (_V, [_I]), "hpgmg_b200_use_graphs": (_V, [_I]),
@@ -60,9 +60,11 @@ SIGNATURES = {
     "hpgmg_fmg_solve_host_bytes": (C.c_ulonglong, [_MP, _I]),
     "hpgmg_fmg_solve_host_submit": (_I, [_MP, _I, _I, _I, _D, _D, _D, C.c_void_p, C.c_void_p]),
     "hpgmg_fmg_solve_host_wait": (_D, [_MP, _I]),
+    "hpgmg_fmg_solve_device": (_D, [_MP, _I, _I, _I, _D, _D, _D, C.c_void_p, C.c_void_p, C.c_void_p]),
     "hpgmg_last_norm_of_F": (_D, [_MP]), "hpgmg_last_norm_of_residual": (_D, [_MP]),
     "hpgmg_last_richardson_error": (_D, []), "hpgmg_last_richardson_order": (_D, []),
     "hpgmg_b200_kernel_launches": (C.c_ulonglong, []), "hpgmg_b200_device_seconds_last_solve": (_D, []),
+    "hpgmg_b200_recorded_graphs": (C.c_ulonglong, []),
     "hpgmg_b200_bench_mark": (_V, [_I]), "hpgmg_b200_bench_elapsed_ms": (_D, [_I, _I]),
     "hpgmg_b200_profiler_start": (_V, []), "hpgmg_b200_profiler_stop": (_V, []),
     "hpgmg_b200_gsrb_sweep": (_V, [_LP, _I, _I, _I, _D, _D, _I]),
@@ -241,6 +243,26 @@ class Hierarchy:
         r, f = self.L.hpgmg_last_norm_of_residual(self.mg), self.L.hpgmg_last_norm_of_F(self.mg)
         return r, (r / f if f != 0 else float("nan"))
 
+    def fmg_solve_device(self, f, out=None, on_level=0, rtol=1e-10):
+        """FMG solve of A u = f with f and u as CUDA tensors of the level's whole domain (hpgmg_fmg_solve_device).
+
+        `f` and `out` are contiguous float64 tensors of shape (dim.k, dim.j, dim.i) on the library's device; element [k, j, i] is
+        cell (i, j, k).  `out` may be `f` itself (solved in place); None allocates torch.zeros_like(f).  Only the cells of this
+        rank's boxes are read and written.  The solve starts after the work already queued on the current torch stream and
+        returns after u is written.  Returns (u, (||r||, ||r||/||f||)) with the F-cycle residual max-norm, as fmg_solve does."""
+        import torch
+        lvl = self.level(on_level).contents
+        shape = (lvl.dim.k, lvl.dim.j, lvl.dim.i)
+        device = self.L.hpgmg_b200_device()
+        _check_grid_tensor("f", f, shape, device)
+        if out is None:
+            out = torch.zeros_like(f)
+        _check_grid_tensor("out", out, shape, device)
+        stream = torch.cuda.current_stream(f.device).cuda_stream
+        r = self.L.hpgmg_fmg_solve_device(self.mg, on_level, VECTOR_U, VECTOR_F, self.a, self.b, rtol, f.data_ptr(), out.data_ptr(), stream)
+        nf = self.L.hpgmg_last_norm_of_F(self.mg)
+        return out, (r, (r / nf if nf != 0 else float("nan")))
+
     def restrict_rhs_to(self, l):
         """restriction(level l, F <- level l-1, F) as the driver does before solving on level l (hpgmg-fv.c:322)."""
         self.L.restriction(self.level(l), VECTOR_F, self.level(l - 1), VECTOR_F, RESTRICT_CELL)
@@ -268,6 +290,23 @@ class Hierarchy:
 
     def __exit__(self, *exc):
         self.close()
+
+
+def _check_grid_tensor(name, t, shape, device):
+    """What hpgmg_fmg_solve_device needs of an array, as TypeError / ValueError instead of the library's exit(1)."""
+    import torch
+    if not isinstance(t, torch.Tensor):
+        raise TypeError(f"{name} must be a torch.Tensor, not {type(t).__name__}")
+    if t.dtype != torch.float64:
+        raise TypeError(f"{name} must be float64, not {t.dtype}")
+    if t.device.type != "cuda" or t.device.index != device:
+        raise ValueError(f"{name} is on {t.device}; the library runs on cuda:{device}")
+    if tuple(t.shape) != shape:
+        raise ValueError(f"{name} has shape {tuple(t.shape)}; the level's domain is (dim.k, dim.j, dim.i) = {shape}")
+    if not t.is_contiguous():
+        raise ValueError(f"{name} must be contiguous (strides {t.stride()})")
+    if t.data_ptr() % 16:
+        raise ValueError(f"{name} must start on a 16-byte boundary (data_ptr {t.data_ptr():#x})")
 
 
 # ------------------------------------------------------------------------------------------------

@@ -187,25 +187,41 @@ __global__ void __launch_bounds__(256) copy_norm_kernel(const DLevel L, const in
   }
 }
 
-/* ---- dense <-> padded: the cells of every box as one contiguous [box][k][j][i] array (the end-to-end solve's staging buffers) ---- */
+/* ---- dense <-> padded: the cells of every box in a contiguous array without ghosts, in one of two layouts ---- */
+/* Where the cells of box `box` lie in the dense array, in 16-byte i-pairs: box_start() is the pair of cell (0,0,0) of the box,
+ * pair() the offset of pair p of row j of plane k from there (q: the same pair counted inside the box, p fastest). */
+struct BoxMajorDense {               /* [box][k][j][i], box after box: the end-to-end solve's staging buffers */
+  __device__ __forceinline__ double2 *box_start(double *dense, const DLevel &L, int box) const
+  { const int n = L.dim; return reinterpret_cast<double2 *>(dense + (size_t)box * n * n * n); }
+  __device__ __forceinline__ int pair(int q, int, int, int) const { return q; }
+};
+struct GridDense {                   /* [k][j][i] over the level's whole domain: a box's cells start at its low corner */
+  const int *low;                    /* device [nboxes][3] (hpgmg_device_level::low); low.i is even since the box size is */
+  size_t hjS, hkS;                   /* row and plane strides of the domain, in pairs: dim.i / 2 and dim.i * dim.j / 2 */
+  __device__ __forceinline__ double2 *box_start(double *dense, const DLevel &, int box) const
+  { const int *lo = low + 3 * box; return reinterpret_cast<double2 *>(dense) + ((size_t)lo[2] * hkS + (size_t)lo[1] * hjS + lo[0] / 2); }
+  __device__ __forceinline__ size_t pair(int, int p, int j, int k) const { return (size_t)p + (size_t)j * hjS + (size_t)k * hkS; }
+};
+
 /* MODE 0: box vector <- dense.  MODE 1: dense <- box vector.  MODE 2: F <- dense, R <- 1.0*dense, max|dense| (the first step of
- * FMGSolve, mg.c:1259-1269, fused with the unpack of the uploaded right-hand side) */
-template <int MODE>
-__global__ void __launch_bounds__(256) dense_kernel(const DLevel L, const int id, const int id2, double *__restrict__ dense, double *__restrict__ slot)
+ * FMGSolve, mg.c:1259-1269, fused with the unpack of the right-hand side) */
+template <int MODE, class Dense>
+__global__ void __launch_bounds__(256) dense_kernel(const DLevel L, const int id, const int id2, double *__restrict__ dense, double *__restrict__ slot, const Dense lay)
 {
   PDL_WAIT();
   const int n = L.dim, box = blockIdx.y;
   const int hn = n / 2, pairs = hn * n * n;                /* even n only */
   double *__restrict__ v = L.vec(box, id);
   double *__restrict__ v2 = (MODE == 2) ? L.vec(box, id2) : nullptr;
-  double2 *__restrict__ d = reinterpret_cast<double2 *>(dense + (size_t)box * n * n * n);
+  double2 *__restrict__ d = lay.box_start(dense, L, box);
   double m = 0.0;
   for (int q = blockIdx.x * blockDim.x + threadIdx.x; q < pairs; q += gridDim.x * blockDim.x) {
     const int p = q % hn, j = (q / hn) % n, k = q / (hn * n);
     const int ijk = 2 * p + j * L.jStride + k * L.kStride;
-    if constexpr (MODE == 1) { d[q] = *reinterpret_cast<const double2 *>(v + ijk); }
+    double2 *__restrict__ dq = d + lay.pair(q, p, j, k);
+    if constexpr (MODE == 1) { *dq = *reinterpret_cast<const double2 *>(v + ijk); }
     else {
-    const double2 a = d[q];
+    const double2 a = *dq;
     *reinterpret_cast<double2 *>(v + ijk) = a;
     if constexpr (MODE == 2) {
       *reinterpret_cast<double2 *>(v2 + ijk) = make_double2(1.0 * a.x, 1.0 * a.y);
@@ -230,8 +246,8 @@ __global__ void __launch_bounds__(256) dense_kernel(const DLevel L, const int id
   }
   }
 }
-template <int MODE>
-static void launch_dense(level_type *level, int id, int id2, double *dense, double *slot)
+template <int MODE, class Dense>
+static void launch_dense(level_type *level, int id, int id2, double *dense, double *slot, const Dense &lay)
 {
   const DLevel &L = dl_of(level);
   if (L.nboxes == 0) return;
@@ -239,20 +255,34 @@ static void launch_dense(level_type *level, int id, int id2, double *dense, doub
   const int pairs = (L.dim / 2) * L.dim * L.dim;
   int bx = (pairs + 1023) / 1024;
   if (bx > 592) bx = 592;
-  LAUNCH(dense_kernel<MODE>, dim3(bx, L.nboxes), 256, 0, L, id, id2, dense, slot);
+  LAUNCH((dense_kernel<MODE, Dense>), dim3(bx, L.nboxes), 256, 0, L, id, id2, dense, slot, lay);
 }
-extern "C" void hpgmg_unpack_async(level_type *level, int id, const double *dense)
-{ hpgmg_note_vector_written(level, id); launch_dense<0>(level, id, id, const_cast<double *>(dense), NULL); }
-extern "C" void hpgmg_pack_async(level_type *level, int id, double *dense) { launch_dense<1>(level, id, id, dense, NULL); }
-extern "C" void hpgmg_unpack_copy_norm_async(level_type *level, int id_f, int id_r, const double *dense, int slot)
+static GridDense grid_of(const level_type *level)
+{
+  GridDense g;
+  g.low = HPGMG_DEV(level)->low;
+  g.hjS = (size_t)level->dim.i / 2;
+  g.hkS = (size_t)level->dim.i * level->dim.j / 2;
+  return g;
+}
+template <class Dense>
+static void unpack_copy_norm(level_type *level, int id_f, int id_r, const double *dense, int slot, const Dense &lay)
 {
   hpgmg_note_vector_written(level, id_f);  hpgmg_note_vector_written(level, id_r);
   double *s = hpgmg_rt_scalar_slots() + slot;
   CUDA_CHECK(cudaMemsetAsync(s, 0, sizeof(double), g_stream));
   g_launches++;
-  launch_dense<2>(level, id_f, id_r, const_cast<double *>(dense), s);
+  launch_dense<2>(level, id_f, id_r, const_cast<double *>(dense), s, lay);
   hpgmg_comm_allreduce_slot_max(level, slot);
 }
+extern "C" void hpgmg_unpack_async(level_type *level, int id, const double *dense)
+{ hpgmg_note_vector_written(level, id); launch_dense<0>(level, id, id, const_cast<double *>(dense), NULL, BoxMajorDense()); }
+extern "C" void hpgmg_pack_async(level_type *level, int id, double *dense) { launch_dense<1>(level, id, id, dense, NULL, BoxMajorDense()); }
+extern "C" void hpgmg_unpack_copy_norm_async(level_type *level, int id_f, int id_r, const double *dense, int slot)
+{ unpack_copy_norm(level, id_f, id_r, dense, slot, BoxMajorDense()); }
+extern "C" void hpgmg_grid_unpack_copy_norm_async(level_type *level, int id_f, int id_r, const double *grid, int slot)
+{ unpack_copy_norm(level, id_f, id_r, grid, slot, grid_of(level)); }
+extern "C" void hpgmg_grid_pack_async(level_type *level, int id, double *grid) { launch_dense<1>(level, id, id, grid, NULL, grid_of(level)); }
 
 extern "C" void hpgmg_norm_async(level_type *level, int id_a, int slot);
 /* norm(level, id_a) into `slot` and scale_vector(level, id_c, 1.0, id_a) */

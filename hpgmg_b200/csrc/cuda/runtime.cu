@@ -42,6 +42,7 @@ static void *g_staging[NSTAGING] = { NULL, NULL, NULL, NULL };
 static size_t g_staging_bytes[NSTAGING] = { 0, 0, 0, 0 };
 static cudaStream_t g_side_stream = 0, g_main_stream_saved = 0;
 static cudaEvent_t g_ev_fork = 0, g_ev_join = 0;
+static cudaEvent_t g_ev_caller = 0;                /* hpgmg_rt_wait_for_stream */
 
 /* Layout-only mode: the host-side data model (decomposition, block lists, level table) can be built
  * and inspected on a machine without a GPU.  Allocations become inaccessible address-space
@@ -119,6 +120,7 @@ extern "C" void hpgmg_b200_finalize(void)
   for (int w = 0; w < NSTAGING; w++) { if (g_staging[w]) cudaFree(g_staging[w]); g_staging[w] = NULL; g_staging_bytes[w] = 0; }
   hpgmg_rt_pipe_destroy();
   if (g_side_stream) { cudaStreamDestroy(g_side_stream); cudaEventDestroy(g_ev_fork); cudaEventDestroy(g_ev_join); g_side_stream = 0; }
+  if (g_ev_caller) { cudaEventDestroy(g_ev_caller); g_ev_caller = 0; }
   cudaEventDestroy(g_ev0);  cudaEventDestroy(g_ev1);
   cudaStreamDestroy(g_stream);
   g_stream = 0;  g_initialised = 0;
@@ -291,6 +293,8 @@ extern "C" void hpgmg_graph_end(const void *owner, long long key)
   CUDA_CHECK(cudaGraphLaunch(e.exec, g_stream));
 }
 
+extern "C" unsigned long long hpgmg_b200_recorded_graphs(void) { return (unsigned long long)g_graphs.size(); }
+
 extern "C" void hpgmg_graph_drop_all(const void *owner)
 {
   if (g_capturing) { fprintf(stderr, "hpgmg_b200: the hierarchy was modified (vectors re-allocated / operator rebuilt / kernel switches) inside a recorded solve\n"); abort(); }
@@ -373,6 +377,30 @@ extern "C" void hpgmg_rt_side_end(void)
 }
 /* the compute stream waits for the side work */
 extern "C" void hpgmg_rt_side_join(void) { CUDA_CHECK(cudaStreamWaitEvent(g_stream, g_ev_join, 0)); }
+
+/* ------------------------------------------------------------------------------------------ */
+/* The end-to-end solve with DEVICE arrays (hpgmg_fmg_solve_device, mg.c): the caller's arrays are checked before any work is
+ * enqueued, and the compute stream (non-blocking, so not ordered with the legacy default stream either) waits for the work
+ * the caller has already put on its own stream, e.g. the kernels that produced f. */
+extern "C" void hpgmg_rt_check_device_array(const char *who, const char *name, const void *p)
+{
+  require_init(who);
+  if (!p) { fprintf(stderr, "%s: %s is NULL\n", who, name); exit(1); }
+  cudaPointerAttributes attr;
+  const cudaError_t e = cudaPointerGetAttributes(&attr, p);
+  if (e != cudaSuccess) (void)cudaGetLastError();
+  if (e != cudaSuccess || attr.type != cudaMemoryTypeDevice || attr.device != g_device) {
+    fprintf(stderr, "%s: %s = %p is not device memory of device %d, the library's device\n", who, name, p, g_device);
+    exit(1);
+  }
+  if ((uintptr_t)p & 15) { fprintf(stderr, "%s: %s = %p is not 16-byte aligned\n", who, name, p); exit(1); }
+}
+extern "C" void hpgmg_rt_wait_for_stream(void *stream)
+{
+  if (!g_ev_caller) CUDA_CHECK(cudaEventCreateWithFlags(&g_ev_caller, cudaEventDisableTiming));
+  CUDA_CHECK(cudaEventRecord(g_ev_caller, (cudaStream_t)stream));
+  CUDA_CHECK(cudaStreamWaitEvent(g_stream, g_ev_caller, 0));
+}
 
 /* ------------------------------------------------------------------------------------------ */
 /* Pipelined end-to-end solves (hpgmg_fmg_solve_host_submit / _wait, mg.c): two slots, each with its own staging buffers.

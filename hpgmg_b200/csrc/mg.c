@@ -766,6 +766,45 @@ double hpgmg_fmg_solve_host(mg_type *MG, int onLevel, int u_id, int F_id, double
 }
 
 /* ------------------------------------------------------------------------------------------ */
+/* The end-to-end solve with DEVICE arrays of the whole domain (include/hpgmg_b200.h).  The caller's arrays are read and written by
+ * plain launches around the recorded solve -- unpack f into F fused with ||F|| and R = F, then [zero u, the F-cycle, the residual
+ * norm], then pack u -- so the recording is keyed by the hierarchy and the solve's parameters, not by the arrays' addresses: a
+ * program that hands in a new tensor every call replays one graph.  Same kernels and order as hpgmg_fmg_solve_host, same bits. */
+double hpgmg_fmg_solve_device(mg_type *MG, int onLevel, int u_id, int F_id, double a, double b, double rtol, const double *f_dev, double *u_dev, void *stream)
+{
+  (void)rtol;
+  level_type *L = MG->levels[onLevel];
+  if ((L->box_dim & 1) || !L->active) {
+    fprintf(stderr, "hpgmg_fmg_solve_device: needs an even box size and an active level\n");
+    exit(1);
+  }
+  hpgmg_rt_check_device_array("hpgmg_fmg_solve_device", "f_dev", f_dev);
+  hpgmg_rt_check_device_array("hpgmg_fmg_solve_device", "u_dev", u_dev);
+  MG->MGSolves_performed++;
+  const int e_id = u_id, R_id = VECTOR_R;
+  const int capturable = solve_is_capturable(MG, L);
+  const long long key = solve_key(4, onLevel, u_id, F_id, a, b);
+  hpgmg_rt_wait_for_stream(stream);                                              /* f is complete */
+  hpgmg_rt_timer_start();
+  hpgmg_grid_unpack_copy_norm_async(L, F_id, R_id, f_dev, HPGMG_SLOT_NORM_F);
+  if (!capturable || hpgmg_graph_begin(MG, key)) {
+    hpgmg_rt_zero_scalar(HPGMG_SLOT_KRYLOV);
+    zero_vector(L, u_id);                                                        /* hpgmg-fv.c:78 */
+    enqueue_fcycle_after_rhs(MG, onLevel, e_id, R_id, a, b);
+    enqueue_residual_norm(L, e_id, F_id, a, b);                                  /* periodic: removes the mean from u first */
+    if (capturable) hpgmg_graph_end(MG, key);
+  }
+  hpgmg_grid_pack_async(L, u_id, u_dev);
+  hpgmg_rt_timer_stop();
+  count_vcycle_visits(MG, onLevel);
+  double s[3];
+  hpgmg_rt_read_scalars(s, HPGMG_SLOT_NORM_F, 3);                                /* u is written */
+  MG->levels[MG->num_levels - 1]->Krylov_iterations += (int)s[2];
+  record_norms(MG, s[0], s[1]);
+  return s[1];
+}
+
+/* ------------------------------------------------------------------------------------------ */
 /* The same end-to-end solve, PIPELINED for back-to-back solves: submit() enqueues upload, solve and download of one solve
  * and returns at once; wait() blocks until that solve's u_host and norms are complete.  Two solves may be in flight: while
  * solve n computes, f of solve n+1 travels up and u of solve n-1 travels down on their own streams (PCIe is full duplex),

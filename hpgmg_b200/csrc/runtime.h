@@ -128,6 +128,12 @@ void  hpgmg_rt_pipe_destroy(void);
 void  hpgmg_unpack_copy_norm_async(level_type *level, int id_f, int id_r, const double *dense, int slot);   /* F = dense; R = 1.0*F; slot = max|F| */
 void  hpgmg_pack_async(level_type *level, int id, double *dense);
 void  hpgmg_unpack_async(level_type *level, int id, const double *dense);
+/* end-to-end solve with device arrays of the whole domain (mg.c: hpgmg_fmg_solve_device): the same moves to and from a
+ * [k][j][i] array of the level's dim.k x dim.j x dim.i cells, each box at its low corner (blas1.cu) */
+void  hpgmg_grid_unpack_copy_norm_async(level_type *level, int id_f, int id_r, const double *grid, int slot);
+void  hpgmg_grid_pack_async(level_type *level, int id, double *grid);
+void  hpgmg_rt_check_device_array(const char *who, const char *name, const void *p);  /* exit(1) unless 16-byte aligned memory of this device */
+void  hpgmg_rt_wait_for_stream(void *stream);                                         /* the compute stream waits for what `stream` holds now */
 
 /* event timing of a solve body */
 void hpgmg_rt_timer_start(void);

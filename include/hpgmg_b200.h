@@ -28,6 +28,7 @@ int  hpgmg_b200_init(int device_ordinal);
 void hpgmg_b200_finalize(void);
 void hpgmg_b200_sync(void);                      /* drain the compute stream                    */
 const char *hpgmg_b200_backend(void);            /* "cuda-sm_100a": there is no other backend    */
+int  hpgmg_b200_device(void);                    /* ordinal of the library's device; -1 before init */
 
 /* ---- variant selection ----------------------------------------------------------------------
  * The reference picks the smoother at compile time (-DUSE_GSRB | -DUSE_CHEBY | -DUSE_JACOBI | -DUSE_L1JACOBI,
@@ -115,6 +116,19 @@ unsigned long long hpgmg_fmg_solve_host_bytes(mg_type *all_grids, int onLevel);
 int    hpgmg_fmg_solve_host_submit(mg_type *all_grids, int onLevel, int u_id, int F_id, double a, double b,
                                    double rtol, const double *f_host, double *u_host);
 double hpgmg_fmg_solve_host_wait(mg_type *all_grids, int ticket);
+/* FMGSolve with DEVICE arrays of the whole domain, for a caller whose f is already on the GPU (a torch.Tensor, another
+ * library's output).  f_dev and u_dev hold dim.k x dim.j x dim.i doubles of level onLevel, [k][j][i] with i fastest: element
+ * (k*dim.j + j)*dim.i + i is global cell (i, j, k) -- a contiguous (N, N, N) tensor, NOT the box-major layout of the host call.
+ * Only the cells of this rank's boxes are read from f_dev and written to u_dev; the other cells of u_dev are left untouched,
+ * so on several ranks the ranks' results combine by summing zero-initialised u.  f_dev == u_dev solves in place (f is read
+ * before u is written); arrays that overlap only in part give undefined results.
+ * Before it reads f, the library's compute stream waits for everything enqueued on `stream` so far (a cudaStream_t of the
+ * library's device; NULL is the legacy default stream).  Returns, after u is written, the F-cycle residual max-norm, and
+ * records the norms and the bottom solver's iteration count as hpgmg_fmg_solve_host does, with the same bits for the same f.
+ * No staging buffers are allocated.  Refused with a message and exit(1): NULL, host, managed or other-device pointers,
+ * pointers not 16-byte aligned, odd box sizes and inactive levels. */
+double hpgmg_fmg_solve_device(mg_type *all_grids, int onLevel, int u_id, int F_id, double a, double b,
+                              double rtol, const double *f_dev, double *u_dev, void *stream);
 
 /* Norms of the last FMGSolve/MGSolve on this hierarchy: ||F||, ||r|| after the F-cycle (or
  * last V-cycle).  The reference only prints them (mg.c:1325-1329); tests need the values. */
@@ -124,6 +138,7 @@ double hpgmg_last_norm_of_residual(const mg_type *all_grids);
 /* ---- evidence ------------------------------------------------------------------------------ */
 unsigned long long hpgmg_b200_kernel_launches(void);  /* kernels enqueued so far (graph replays count their nodes) */
 double hpgmg_b200_device_seconds_last_solve(void);    /* CUDA-event time of the last FMGSolve/MGSolve body */
+unsigned long long hpgmg_b200_recorded_graphs(void);  /* recorded solves (CUDA graphs) the library holds now */
 
 /* event marks on the library's compute stream, for timing several calls from outside (bench.py) */
 void   hpgmg_b200_bench_mark(int idx);                /* idx 0..7 */
